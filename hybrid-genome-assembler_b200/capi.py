@@ -59,7 +59,7 @@ class Metrics(C.Structure):
                [(n, C.c_uint64) for n in ("n_bases", "n_reads", "n_hits", "n_pairs", "n_increments", "n_selected", "n_components", "table_bytes",
                                           "filter_bytes", "pair_retries", "heavy_pivots", "kernel_launches", "table_overflow_keys", "mid_pivots", "n_candidates")] + \
                [("enrich_ms", C.c_double)] + [(n, C.c_uint64) for n in ("n_cores", "n_enrich_connections", "n_final_components", "redo_pivots")] + \
-               [("enrich_phase_ms", C.c_double * 6)]
+               [("enrich_phase_ms", C.c_double * 6), ("scan_retries", C.c_uint64)]
 
     def as_dict(self):
         return {n: (list(getattr(self, n)) if n == "enrich_phase_ms" else getattr(self, n)) for n, _ in self._fields_}

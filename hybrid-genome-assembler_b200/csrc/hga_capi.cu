@@ -171,7 +171,6 @@ int hga_set_stream(hga_handle *h, void *cuda_stream) {
 int hga_scan_device(hga_handle *h, const char *d_bases, const uint64_t *d_read_off, uint64_t n_reads, uint64_t n_bases, uint32_t read_id_base) {
     if (!h) { hga_set_error("NULL handle"); return HGA_E_ARG; }
     if ((n_bases && !d_bases) || !d_read_off) { hga_set_error("hga_scan_device: NULL buffer"); return HGA_E_ARG; }
-    if (((uintptr_t) d_bases & 15) != 0) { hga_set_error("hga_scan_device: d_bases must be 16-byte aligned"); return HGA_E_ARG; }
     HGA_TRY(use_device(h));
     h->read_id_base = read_id_base;
     return hga_scan_run(h, d_bases, d_read_off, n_reads, n_bases, nullptr);

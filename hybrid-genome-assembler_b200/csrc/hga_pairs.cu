@@ -57,7 +57,7 @@ struct PairScalars {
     unsigned long long redo_count;    // rows whose partner set overflowed the first-pass accumulator of tier 1
     unsigned long long redo_ticket;
     unsigned int overflow;
-    unsigned int pad;
+    unsigned int score_carry;         // a 32-bit score accumulator wrapped (set by the checked kernel variants only)
 };
 
 namespace {
@@ -93,6 +93,16 @@ __device__ __forceinline__ bool keep_candidate(uint32_t x, uint32_t y, int mode,
 }
 
 __device__ __forceinline__ uint32_t hash_row(uint32_t y) { return y * 2654435761u; }
+
+// score accumulation. A score is at most hits(x) * hits(y), so it cannot exceed 2^32 - 1 while every row holds fewer than 65 536
+// hits; hga_pairs_run runs the CHECK = false kernels then (the plain atomic, unchanged). Otherwise the CHECK = true variants look at
+// the value the atomic returns: values only grow and every partial sum is a lower bound of a true score, so a carry out of any add
+// means a true score above 2^32 - 1, which the host reports as HGA_E_OVERFLOW.
+template<bool CHECK>
+__device__ __forceinline__ void score_add(uint32_t *v, uint32_t c, unsigned int *carry) {
+    if (CHECK) { if (atomicAdd(v, c) > 0xFFFFFFFFu - c) *carry = 1u; }
+    else atomicAdd(v, c);
+}
 
 template<int THREADS>
 __device__ __forceinline__ unsigned long long block_sum(unsigned long long v, unsigned long long *s_red) {
@@ -134,8 +144,8 @@ struct WarpAcc {
 };
 
 // ++count[y] with shared-memory atomics; most calls find y already present: one plain read, one atomic add
-template<int CMAX>
-__device__ __forceinline__ void acc_add(WarpAcc<CMAX> &A, uint32_t y, uint32_t c, uint32_t cmask, int cshift, uint32_t limit) {
+template<int CMAX, bool CHECK = false>
+__device__ __forceinline__ void acc_add(WarpAcc<CMAX> &A, uint32_t y, uint32_t c, uint32_t cmask, int cshift, uint32_t limit, unsigned int *carry) {
     uint32_t h = hash_row(y) >> cshift;
     for (;;) {
         uint32_t cur = *reinterpret_cast<volatile uint32_t *>(&A.key[h]);
@@ -143,7 +153,7 @@ __device__ __forceinline__ void acc_add(WarpAcc<CMAX> &A, uint32_t y, uint32_t c
             cur = atomicCAS(&A.key[h], PC_EMPTY, y);
             if (cur == PC_EMPTY) { if (atomicAdd(&A.distinct, 1u) >= limit) A.overflow = 1; cur = y; }
         }
-        if (cur == y) { atomicAdd(&A.val[h], c); return; }
+        if (cur == y) { score_add<CHECK>(&A.val[h], c, carry); return; }
         if (*reinterpret_cast<volatile uint32_t *>(&A.overflow)) return;
         h = (h + 1) & cmask;
     }
@@ -151,7 +161,7 @@ __device__ __forceinline__ void acc_add(WarpAcc<CMAX> &A, uint32_t y, uint32_t c
 
 // The walk of one pivot row's incidence entries [a, b) by one warp into its accumulator A.
 // TAILONLY: the mode is PAIR_MODE_TAIL at compile time (all rows are pivots: the first-pass kernel of the hot path), so the candidate test is y > x and nothing else
-template<int CMAX, int EPS = 4, bool TAILONLY = false>
+template<int CMAX, int EPS = 4, bool TAILONLY = false, bool CHECK = false>
 __device__ __forceinline__ void walk_row(WarpAcc<CMAX> &A, const PairParams &p, uint32_t x, uint64_t a, uint64_t b, bool tail_rt, uint32_t cmask, int cshift,
                                          uint32_t limit, int lane) {
     const bool tail = TAILONLY ? true : tail_rt;
@@ -224,7 +234,7 @@ __device__ __forceinline__ void walk_row(WarpAcc<CMAX> &A, const PairParams &p, 
         #pragma unroll
         for (int e = 0; e < EPS; e++) {
             const bool fast = ok[e] && kk[e] == ys[e];
-            if (fast) atomicAdd(&A.val[hh[e]], 1u);
+            if (fast) score_add<CHECK>(&A.val[hh[e]], 1u, &p.sc->score_carry);
             if (ok[e] && !fast) pend |= 1u << e;
         }
         if (__any_sync(0xFFFFFFFFu, pend != 0)) {                  // warp uniform
@@ -245,7 +255,7 @@ __device__ __forceinline__ void walk_row(WarpAcc<CMAX> &A, const PairParams &p, 
                         cur = atomicCAS(&A.key[hsl], PC_EMPTY, y);
                         if (cur == PC_EMPTY) { if (atomicAdd(&A.distinct, 1u) >= limit) A.overflow = 1; cur = y; }
                     }
-                    if (cur == y) { atomicAdd(&A.val[hsl], 1u); busy = false; }
+                    if (cur == y) { score_add<CHECK>(&A.val[hsl], 1u, &p.sc->score_carry); busy = false; }
                     else if (*reinterpret_cast<volatile uint32_t *>(&A.overflow)) { busy = false; pend = 0; }
                     else hsl = (hsl + 1) & cmask;
                 }
@@ -263,7 +273,7 @@ __device__ __forceinline__ void walk_row(WarpAcc<CMAX> &A, const PairParams &p, 
             if (go) {
                 const uint32_t y = __ldg(&p.inv_row[i]);
                 if (tail && y <= x) go = false;
-                else if (keep_candidate(x, y, mode, p.pivot_flag)) acc_add(A, y, 1u, cmask, cshift, limit);
+                else if (keep_candidate(x, y, mode, p.pivot_flag)) acc_add<CMAX, CHECK>(A, y, 1u, cmask, cshift, limit, &p.sc->score_carry);
             }
             if (!__any_sync(0xFFFFFFFFu, go)) break;
         }
@@ -308,7 +318,7 @@ __device__ __forceinline__ void flush_table(WarpAcc<CMAX> &A, const PairParams &
 // 4 / 6 CTAs per SM -> 359 / 186 / 130 / 102 / 75 ms), and the accumulator is what limits them. The first pass therefore runs with
 // a 512-entry accumulator (17 KB per CTA: 11 CTAs = 44 warps per SM); the rows whose partner set does not fit it are listed and
 // redone by a second pass with 1024 entries (6 CTAs per SM), and only what overflows that goes on to tier 2.
-template<int CMAX, bool REDO, int MINB = 1, int EPS = 4, bool TAILONLY = false>
+template<int CMAX, bool REDO, int MINB = 1, int EPS = 4, bool TAILONLY = false, bool CHECK = false>
 __global__ void __launch_bounds__(PW_THREADS, MINB) pair_count_warp_kernel(const __grid_constant__ PairParams p) {
     __shared__ WarpAcc<CMAX> s_acc[PW_WARPS];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -338,7 +348,7 @@ __global__ void __launch_bounds__(PW_THREADS, MINB) pair_count_warp_kernel(const
             if (lane == 0) { A.distinct = 0; A.overflow = 0; A.n_defer = 0; }
             __syncwarp();
 
-            walk_row<CMAX, EPS, TAILONLY>(A, p, x, a, b, tail, cmask, cshift, limit, lane);
+            walk_row<CMAX, EPS, TAILONLY, CHECK>(A, p, x, a, b, tail, cmask, cshift, limit, lane);
             if (!*reinterpret_cast<volatile uint32_t *>(&A.overflow)) {
                 flush_table<CMAX>(A, p, x, C, lane);
                 break;
@@ -359,6 +369,7 @@ __global__ void __launch_bounds__(PW_THREADS, MINB) pair_count_warp_kernel(const
 // config 4) and they are the longest rows, so one warp per row leaves the GPU waiting for the slowest of them (5.6 ms); here a
 // CTA takes a row: every warp walks a quarter of the row's incidence entries into its own 1024-entry accumulator, then warps
 // 1 .. 3 pour theirs into warp 0's, which is flushed. A row whose merged partner set still does not fit goes to tier 2.
+template<bool CHECK = false>
 __global__ void __launch_bounds__(PW_THREADS) pair_count_redo_kernel(const __grid_constant__ PairParams p) {
     __shared__ WarpAcc<PW_CMAX> s_acc[PW_WARPS];
     __shared__ unsigned long long s_ticket;
@@ -383,7 +394,7 @@ __global__ void __launch_bounds__(PW_THREADS) pair_count_redo_kernel(const __gri
         for (uint32_t i = lane; i < C; i += 32) { A.key[i] = PC_EMPTY; A.val[i] = 0; }
         if (lane == 0) { A.distinct = 0; A.overflow = 0; A.n_defer = 0; }
         __syncwarp();
-        if (a < b) walk_row<PW_CMAX>(A, p, x, a, b, tail, cmask, cshift, limit, lane);
+        if (a < b) walk_row<PW_CMAX, 4, false, CHECK>(A, p, x, a, b, tail, cmask, cshift, limit, lane);
         __syncthreads();
         bool over = false;
         #pragma unroll
@@ -391,7 +402,7 @@ __global__ void __launch_bounds__(PW_THREADS) pair_count_redo_kernel(const __gri
         if (!over && warp > 0) {
             for (uint32_t i = lane; i < C; i += 32) {
                 const uint32_t y = A.key[i];
-                if (y != PC_EMPTY) acc_add(s_acc[0], y, A.val[i], cmask, cshift, limit);
+                if (y != PC_EMPTY) acc_add<PW_CMAX, CHECK>(s_acc[0], y, A.val[i], cmask, cshift, limit, &p.sc->score_carry);
             }
         }
         __syncthreads();
@@ -406,6 +417,7 @@ __global__ void __launch_bounds__(PW_THREADS) pair_count_redo_kernel(const __gri
 }
 
 // ---- tier 2 ---------------------------------------------------------------------------------------------------
+template<bool CHECK = false>
 __global__ void __launch_bounds__(PC_THREADS) pair_count_kernel(PairParams p) {
     __shared__ uint32_t s_key[PC_CMAX];
     __shared__ uint32_t s_val[PC_CMAX];
@@ -456,7 +468,7 @@ __global__ void __launch_bounds__(PC_THREADS) pair_count_kernel(PairParams p) {
                     if (old == PC_EMPTY) {
                         if (atomicAdd(&s_distinct, 1u) + 1 > limit) s_overflow = 1;
                     }
-                    if (old == PC_EMPTY || old == y) { atomicAdd(&s_val[hsh], 1u); break; }
+                    if (old == PC_EMPTY || old == y) { score_add<CHECK>(&s_val[hsh], 1u, &p.sc->score_carry); break; }
                     if (s_overflow) break;
                     hsh = (hsh + 1) & cmask;
                 }
@@ -499,6 +511,7 @@ __global__ void __launch_bounds__(PC_THREADS) pair_count_kernel(PairParams p) {
 }
 
 // Rows whose partner set overflowed the shared-memory accumulator: same algorithm, table in HBM.
+template<bool CHECK = false>
 __global__ void __launch_bounds__(HV_THREADS) pair_count_heavy_kernel(PairParams p) {
     __shared__ uint32_t s_red[HV_THREADS / 32];
     __shared__ unsigned long long s_ticket, s_base;
@@ -528,7 +541,7 @@ __global__ void __launch_bounds__(HV_THREADS) pair_count_heavy_kernel(PairParams
                 uint32_t hsh = hash_row(y) >> (32 - cbits);
                 for (;;) {
                     const uint32_t old = atomicCAS(&tab_key[hsh], PC_EMPTY, y);
-                    if (old == PC_EMPTY || old == y) { atomicAdd(&tab_val[hsh], 1u); break; }
+                    if (old == PC_EMPTY || old == y) { score_add<CHECK>(&tab_val[hsh], 1u, &p.sc->score_carry); break; }
                     hsh = (hsh + 1) & cmask;
                 }
             }
@@ -616,6 +629,15 @@ __global__ void row_neighbor_min_kernel(const uint32_t *__restrict__ inv_off, co
     }
 }
 
+// largest hit count of a row: bounds every score by its square
+__global__ void max_row_hits_kernel(const uint64_t *__restrict__ row_off, uint64_t n_rows, unsigned long long *out) {
+    unsigned long long m = 0;
+    for (uint64_t i = blockIdx.x * (uint64_t) blockDim.x + threadIdx.x; i < n_rows; i += (uint64_t) gridDim.x * blockDim.x) m = max(m, (unsigned long long) (row_off[i + 1] - row_off[i]));
+    #pragma unroll
+    for (int d = 16; d > 0; d >>= 1) m = max(m, __shfl_xor_sync(0xFFFFFFFFu, m, d));
+    if ((threadIdx.x & 31) == 0 && m) atomicMax(out, m);
+}
+
 __global__ void flag_min_score_kernel(const uint32_t *__restrict__ score, uint64_t n, uint32_t min_score, uint8_t *flag) {
     for (uint64_t i = blockIdx.x * (uint64_t) blockDim.x + threadIdx.x; i < n; i += (uint64_t) gridDim.x * blockDim.x) flag[i] = score[i] >= min_score;
 }
@@ -640,6 +662,33 @@ int hga_pairs_run(hga_handle *h, uint32_t min_score, const uint32_t *pivots, uin
     HGA_TRY(h->d_heavy_list.ensure((n_rows + 1) * 4));
     HGA_TRY(h->d_mid_list.ensure((n_rows + 1) * 4));
     HGA_TRY(h->d_redo_list.ensure((n_rows + 1) * 4));
+
+    // Scores fit 32 bits while every read has fewer than 65 536 hits (score <= hits(x) * hits(y)); above that the checked kernel
+    // variants run and a score that does not fit is an error rather than a wrapped value. With a communicator the partial scores
+    // are summed in 32 bits by the exchange, which has no such check: such inputs are refused there.
+    uint64_t max_hits = 0;
+    {
+        HGA_CUDA(cudaMemsetAsync(&d_sc->increments, 0, 8, h->stream));
+        if (h->n_reads) {
+            max_row_hits_kernel<<<(int) std::min<uint64_t>((h->n_reads + 255) / 256, (uint64_t) h->sm_count * 8), 256, 0, h->stream>>>(
+                h->d_row_off.as<uint64_t>(), h->n_reads, &d_sc->increments);
+            h->metrics.kernel_launches++;
+            HGA_CUDA(cudaGetLastError());
+        }
+        HGA_CUDA(cudaMemcpyAsync(&max_hits, &d_sc->increments, 8, cudaMemcpyDeviceToHost, h->stream));
+        HGA_CUDA(cudaStreamSynchronize(h->stream));
+        if (multi) {
+            std::vector<uint64_t> all;
+            HGA_TRY(hga_comm_allgather_u64(h, max_hits, all));
+            for (uint64_t v : all) max_hits = std::max(max_hits, v);
+        }
+    }
+    const bool check_scores = max_hits > 65535;
+    if (check_scores && multi) {
+        hga_set_error("hga_pair_count: a read has %llu hits, so a pair score may exceed 2^32 - 1, which the multi-GPU reduction of partial "
+                      "scores cannot detect; run this input on one GPU", (unsigned long long) max_hits);
+        return HGA_E_OVERFLOW;
+    }
 
     PairParams p;
     memset(&p, 0, sizeof(p));
@@ -757,10 +806,18 @@ int hga_pairs_run(hga_handle *h, uint32_t min_score, const uint32_t *pivots, uin
     if (p.mode != PAIR_MODE_TAIL) first_pass = pair_count_warp_kernel<PW_CMAX_FIRST, false, 9, 8, false>;
     if (pair_occ == 4) first_pass = pair_count_warp_kernel<PW_CMAX_FIRST, false, 1, 4>;
     if (pair_occ == 98) first_pass = pair_count_warp_kernel<PW_CMAX_FIRST, false, 9, 8, false>;
+    pair_kernel_t single_pass_kernel = pair_count_warp_kernel<PW_CMAX, false>;
+    pair_kernel_t redo_kernel = pair_count_redo_kernel<false>, mid_kernel = pair_count_kernel<false>, heavy_kernel = pair_count_heavy_kernel<false>;
+    if (check_scores) {
+        first_pass = p.mode == PAIR_MODE_TAIL ? pair_count_warp_kernel<PW_CMAX_FIRST, false, 9, 8, true, true> : pair_count_warp_kernel<PW_CMAX_FIRST, false, 9, 8, false, true>;
+        single_pass_kernel = pair_count_warp_kernel<PW_CMAX, false, 1, 4, false, true>;
+        redo_kernel = pair_count_redo_kernel<true>; mid_kernel = pair_count_kernel<true>; heavy_kernel = pair_count_heavy_kernel<true>;
+        pad_smem = 0;
+    }
     HGA_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_w, first_pass, PW_THREADS, pad_smem));
-    HGA_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_r, pair_count_redo_kernel, PW_THREADS, 0));
+    HGA_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_r, redo_kernel, PW_THREADS, 0));
     if (occ_r < 1) occ_r = 1;
-    HGA_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_c, pair_count_kernel, PC_THREADS, 0));
+    HGA_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_c, mid_kernel, PC_THREADS, 0));
     if (occ_w < 1) occ_w = 1;
     if (occ_c < 1) occ_c = 1;
     const int grid_w = (int) std::max<uint64_t>(1, std::min<uint64_t>((uint64_t) h->sm_count * occ_w, (p.n_pivots + PW_WARPS - 1) / PW_WARPS));
@@ -777,7 +834,7 @@ int hga_pairs_run(hga_handle *h, uint32_t min_score, const uint32_t *pivots, uin
         if (p.n_pivots) {
             // multi-GPU: the index is keyed by kmer_id there, neighbouring hits of a read do not have neighbouring lists, and the
             // extra warps of the 512-entry pass only add random DRAM traffic (r3z, 2 GPUs: 50.6 ms against 45.2 ms single pass)
-            if (p.single_pass) pair_count_warp_kernel<PW_CMAX, false><<<grid_s, PW_THREADS, 0, h->stream>>>(p);
+            if (p.single_pass) single_pass_kernel<<<grid_s, PW_THREADS, 0, h->stream>>>(p);
             else first_pass<<<grid_w, PW_THREADS, pad_smem, h->stream>>>(p);
             h->metrics.kernel_launches++;
             HGA_CUDA(cudaGetLastError());
@@ -786,7 +843,7 @@ int hga_pairs_run(hga_handle *h, uint32_t min_score, const uint32_t *pivots, uin
         HGA_CUDA(cudaStreamSynchronize(h->stream));
         if (sc.redo_count) {
             const int grid_r = (int) std::max<uint64_t>(1, std::min<uint64_t>((uint64_t) h->sm_count * occ_r, sc.redo_count));
-            pair_count_redo_kernel<<<grid_r, PW_THREADS, 0, h->stream>>>(p);
+            redo_kernel<<<grid_r, PW_THREADS, 0, h->stream>>>(p);
             h->metrics.kernel_launches++;
             HGA_CUDA(cudaGetLastError());
             HGA_CUDA(cudaMemcpyAsync(&sc, d_sc, sizeof(sc), cudaMemcpyDeviceToHost, h->stream));
@@ -795,7 +852,7 @@ int hga_pairs_run(hga_handle *h, uint32_t min_score, const uint32_t *pivots, uin
         h->metrics.redo_pivots = sc.redo_count;
         if (sc.mid_count) {
             const int grid_c = (int) std::min<uint64_t>(sc.mid_count, (uint64_t) h->sm_count * occ_c);
-            pair_count_kernel<<<grid_c, PC_THREADS, 0, h->stream>>>(p);
+            mid_kernel<<<grid_c, PC_THREADS, 0, h->stream>>>(p);
             h->metrics.kernel_launches++;
             HGA_CUDA(cudaGetLastError());
             HGA_CUDA(cudaMemcpyAsync(&sc, d_sc, sizeof(sc), cudaMemcpyDeviceToHost, h->stream));
@@ -809,7 +866,7 @@ int hga_pairs_run(hga_handle *h, uint32_t min_score, const uint32_t *pivots, uin
             while (hgrid > 1 && (uint64_t) hgrid * cap * 8 > budget) hgrid--;
             HGA_TRY(h->d_heavy_tab.ensure((size_t) hgrid * cap * 8));
             p.heavy_tab = h->d_heavy_tab.as<uint32_t>(); p.heavy_cap = cap;
-            pair_count_heavy_kernel<<<hgrid, HV_THREADS, 0, h->stream>>>(p);
+            heavy_kernel<<<hgrid, HV_THREADS, 0, h->stream>>>(p);
             h->metrics.kernel_launches++;
             HGA_CUDA(cudaGetLastError());
             HGA_CUDA(cudaMemcpyAsync(&sc, d_sc, sizeof(sc), cudaMemcpyDeviceToHost, h->stream));
@@ -817,6 +874,10 @@ int hga_pairs_run(hga_handle *h, uint32_t min_score, const uint32_t *pivots, uin
         }
         h->metrics.heavy_pivots = sc.heavy_count;
         h->metrics.mid_pivots = sc.mid_count;
+        if (sc.score_carry) {
+            hga_set_error("hga_pair_count: a pair score exceeds 2^32 - 1 (a read has %llu hits; scores are counted in 32 bits)", (unsigned long long) max_hits);
+            return HGA_E_OVERFLOW;
+        }
         if (!sc.overflow) break;
         if (attempt >= 1) { hga_set_error("pair_count: output overflow after exact resize (internal error)"); return HGA_E_OVERFLOW; }
         capacity = sc.cursor;

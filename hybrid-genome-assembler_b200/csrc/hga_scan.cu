@@ -709,6 +709,7 @@ int hga_scan_run(hga_handle *h, const char *d_bases, const uint64_t *d_read_off,
     ScanScalars sc;
     memset(&sc, 0, sizeof(sc));
     uint64_t capacity = 0, E = 0;
+    h->metrics.scan_retries = 0;
     // Hit-buffer sizes. Warps reserve chunks, so the buffer holds gaps: what is left of a chunk when the next tile does not fit (less
     // than one tile's hits, <= SCAN_TILE) and every warp's last chunk. `expected` sizes the first attempt from an estimate of the hit
     // count (an overflow is detected and the scan reruns), `certain` is the bound that cannot overflow for an exact count.
@@ -788,7 +789,8 @@ int hga_scan_run(hga_handle *h, const char *d_bases, const uint64_t *d_read_off,
         cudaEventDestroy(ev_begin); cudaEventDestroy(ev_end);
         E = sc.total;
         p.tile_begin = 0; p.warp_chunks = nullptr;
-        if (!sc.overflow) done = true; else capacity = certain(E, 1, SCAN_CHUNK);     // the bases are resident now: one plain rerun with the exact count
+        if (!sc.overflow) done = true;
+        else { capacity = certain(E, 1, SCAN_CHUNK); h->metrics.scan_retries++; }     // the bases are resident now: one plain rerun with the exact count
     } else if (n_tiles > 0) {
         // capacity of the hit arrays: exact upper bound for small inputs, otherwise estimated from a strided
         // count-only sample (1 tile in 64)
@@ -826,6 +828,7 @@ int hga_scan_run(hga_handle *h, const char *d_bases, const uint64_t *d_read_off,
         if (!sc.overflow) break;
         if (attempt == 1) { hga_set_error("scan: hit buffer overflow after exact resize (internal error)"); return HGA_E_OVERFLOW; }
         capacity = certain(E, 1, SCAN_CHUNK);   // cannot overflow; rerun once
+        h->metrics.scan_retries++;
     }
 
     HGA_TRY(h->d_hit_slot.ensure((E + 1) * 4));

@@ -79,7 +79,8 @@ int hga_set_stream(hga_handle *h, void *cuda_stream);
  * bases  : the reads' sequence bytes back to back (no separators), ASCII as in the file
  * read_off[n_reads+1] : byte offset of every read in `bases`
  * Any byte other than 'A','C','G','T' follows the reference rule (code 0 on BOTH strands).
- * hga_scan copies the host buffers to the GPU inside the call; hga_scan_device takes device pointers. */
+ * hga_scan copies the host buffers to the GPU inside the call; hga_scan_device takes device pointers. d_bases may have any
+ * alignment (a read set can start anywhere inside a larger buffer): the scan loads the aligned 16-byte blocks that hold the bases. */
 int hga_scan(hga_handle *h, const char *bases, const uint64_t *read_off, uint64_t n_reads, uint32_t read_id_base);
 int hga_scan_device(hga_handle *h, const char *d_bases, const uint64_t *d_read_off, uint64_t n_reads, uint64_t n_bases,
                     uint32_t read_id_base);
@@ -107,7 +108,9 @@ int hga_get_index(hga_handle *h, hga_index *out);
 /* score(x,y) = sum_k mult_x(k) * mult_y(k) for every unordered read pair sharing a k-mer.
  * pivots == NULL: all reads (get_all_connections); else only pairs with at least one endpoint in pivots
  * (get_connections over a component list). A non-NULL pointer with n_pivots == 0 is the EMPTY subset: no pairs, as get_connections({}).
- * Pairs with score < min_score are dropped. */
+ * Pairs with score < min_score are dropped. Scores are 32-bit: a score above 2^32 - 1 (possible only when two reads have more than
+ * 65 535 hits each) fails with HGA_E_OVERFLOW. With a communicator an input with a read of more than 65 535 hits fails with it
+ * up front, since the reduction of partial scores does not check for a carry. */
 int hga_pair_count(hga_handle *h, uint32_t min_score, const uint32_t *pivots, uint64_t n_pivots);
 typedef struct {
     uint64_t n_pairs;          /* unordered pairs, x < y, ordered by (x, y) */
@@ -269,6 +272,7 @@ typedef struct {
      * [0] Merging of initial components, [1] Calculation of tail connections, [2] Spectral clustering, [3] Merging of scaffold
      * components, [4] Calculation of enrichment connections, [5] Merging into core components ([1]..[3]: 0 when the block did not run) */
     double enrich_phase_ms[6];
+    uint64_t scan_retries;     /* reruns of the last scan with the exact hit count after its estimated hit buffer overflowed */
 } hga_metrics_t;
 int hga_metrics(hga_handle *h, hga_metrics_t *out);
 

@@ -78,3 +78,17 @@ def check_enrichment(ref, e, kmers_sorted):
     fr = np.concatenate(e["final_reads"]) if len(e["final_reads"]) else np.zeros(0, np.uint32)
     assert np.array_equal(fr, ref["final_read"]), "final components differ"
     assert np.array_equal(np.cumsum([0] + [len(c) for c in e["final_reads"]]).astype(np.uint64), ref["final_off"])
+
+
+def enrichment_as_dump(e, kmers_sorted):
+    """an Oracle.enrich-style result (exact_ref.enrich, oracle_lib.enrich) in the shape of a ref_driver --enrich dump, so that
+    check_enrichment can judge another result with it"""
+    kmers_sorted = np.asarray(kmers_sorted, dtype=np.uint64)
+    cat = lambda parts, dt: np.concatenate([np.asarray(p, dtype=dt) for p in parts]) if len(parts) else np.zeros(0, dt)
+    off = lambda parts: np.cumsum([0] + [len(p) for p in parts]).astype(np.uint64)
+    ex, ey, es = e["econn"]
+    return dict(core_id=np.asarray(e["core_id"], dtype=np.uint32), core_kmer=cat([np.sort(kmers_sorted[np.asarray(c, dtype=np.int64)]) for c in e["core_kmers"]], np.uint64),
+                core_kmer_off=off(e["core_kmers"]), core_read=cat(e["core_reads"], np.uint32), purged_off=np.asarray(e["purged_off"], dtype=np.uint64),
+                purged_read=np.asarray(e["purged_read"], dtype=np.uint32), econn_x=np.asarray(ex, dtype=np.uint32), econn_y=np.asarray(ey, dtype=np.uint32),
+                econn_score=np.asarray(es, dtype=np.uint64), final_id=np.asarray(e["final_id"], dtype=np.uint32), final_read=cat(e["final_reads"], np.uint32),
+                final_off=off(e["final_reads"]))

@@ -166,3 +166,24 @@ def fuzz_case(seed):
     min_size = int(rng.choice([2, 3, 5, 10, 30]))
     enrich_min = int(rng.choice([1, 2, 5, 20, 40]))
     return [a, b], reads, k, fraction, min_size, enrich_min
+
+
+def many_loci_case(n_loci, locus_len, reads_per_haplotype, read_len, seed, k=19, divergence=0.03, error_rate=0.005, repeat_every=0):
+    """Many independent diploid loci sampled with short reads, read ids shuffled: (bases, read_off uint64, discriminative k-mers of
+    every locus, sorted). Large selections and many scaffold components from one input. With repeat_every = r, every r-th locus has a
+    tandem repeat (10 copies of a 40 bp unit) in one haplotype only: its k-mers occur several times per read, so a read with few hits
+    can still share a high score with a read inside the repeat."""
+    reads, kmers = [], []
+    for i in range(n_loci):
+        a = random_genome(locus_len, seed + 4 * i)
+        b = mutate(a, divergence, seed + 4 * i + 1)
+        if repeat_every and i % repeat_every == 0:
+            at = locus_len // 2
+            a = np.concatenate([a[:at], np.tile(random_genome(40, seed + 4 * i + 5), 10), a[at:]])
+        reads += sample_reads(a, reads_per_haplotype, read_len, seed + 4 * i + 2, error_rate=error_rate) + \
+            sample_reads(b, reads_per_haplotype, read_len, seed + 4 * i + 3, error_rate=error_rate)
+        kmers.append(discriminative_kmers([a, b], k))
+    seqs = [to_ascii(reads[i]).encode() for i in np.random.default_rng(seed).permutation(len(reads))]
+    off = np.zeros(len(seqs) + 1, dtype=np.uint64)
+    np.cumsum([len(s) for s in seqs], out=off[1:])
+    return b"".join(seqs), off, np.unique(np.concatenate(kmers))

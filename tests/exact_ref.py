@@ -13,6 +13,24 @@ loops) it scales to tens of Mbases, so it can judge the GPU in the regimes only 
               threshold mode: score > S
   components  connected components of the selected edges, label = smallest member id; a read without a selected edge is labelled
               with itself and is no listed component whatever min_size is (as union_find only sees the reads of some edge)
+
+From the selection on, what run_clustering does to its engine state (ReadClusteringEngine.cpp), in the order it does it:
+
+  scaffold list  the directed list union_find receives, built literally: fraction mode = the first n entries of the canonical order
+              (score desc, min(x, y) asc, max(x, y) asc, x asc) over both directions of every pair; sc_score mode = what
+              get_connections emits for the pivots ((pivot, other); a pair of two pivots in both directions), score > S, canonical
+  union_find  sequential over the list in order; vertices = ids some edge touches; union by size, ties to y's root; a union is
+              skipped when it would exceed max_size or join two restricted roots; a root inherits `restricted`; components of
+              >= min_size vertices with the root first, spanning-tree edges in replay order
+  merge       merge_components: element [0] survives with the sorted unique union of the members' k-mer lists and all their reads;
+              every member goes into the removal list of every k-mer once per entry of its current list (the survivor's current
+              list being the union); each inverted list of a k-mer with removals is then purged by the two-pointer walk that stops
+              when the removal list runs out (purge_walk; vectorized in purge)
+  connections get_connections on the current state: score(p, y) = sum over the entries k of p's list of the copies of y in the list
+              of k, y != p, score >= min_score; a pivot that is no survivor keeps its own list with duplicates
+  enrich      union_find(min_size, max_size) -> merge -> [second merge of caller-given clusters] -> cores = ids with >= min_size
+              reads -> connections(cores, enrich_min), canonical -> union_find(min 2, restricted = cores) -> merge -> final ids
+              with >= min_size reads
 """
 import numpy as np
 import scipy.sparse as sp
@@ -140,3 +158,240 @@ def components(n_reads, sel_x, sel_y, min_size):
     big = np.nonzero(size >= max(int(min_size), 2))[0]
     o = np.argsort(first[big])
     return dict(label=label, comp_label=(first[big][o] + 1).astype(np.uint32), comp_size=size[big][o].astype(np.uint32))
+
+
+# ---- scaffold stage, merge and enrichment (ReadClusteringEngine::run_clustering after the selection) ------------------------------
+
+def canonical(x, y, score):
+    """-> (x, y, score) of a directed list in the canonical order: score desc, min(x, y) asc, max(x, y) asc, x asc"""
+    x = np.asarray(x, dtype=np.int64); y = np.asarray(y, dtype=np.int64); score = np.asarray(score, dtype=np.int64)
+    o = np.lexsort((x, np.maximum(x, y), np.minimum(x, y), -score))
+    return x[o], y[o], score[o]
+
+
+def directed_fraction(x, y, score, n):
+    """the list union_find receives in fraction mode: the first n entries of the canonical order over both directions of every pair"""
+    x = np.asarray(x, dtype=np.int64); y = np.asarray(y, dtype=np.int64); score = np.asarray(score, dtype=np.int64)
+    cx, cy, cs = canonical(np.concatenate([x, y]), np.concatenate([y, x]), np.concatenate([score, score]))
+    return cx[:n], cy[:n], cs[:n]
+
+
+def directed_pivots(x, y, score, pivots, sc_score):
+    """the list union_find receives in sc_score mode: get_connections of every pivot emits (pivot, other), so a pair of two pivots
+    is there in both directions and a pair with one pivot only as (pivot, other); the entries with score > sc_score, canonical"""
+    x = np.asarray(x, dtype=np.int64); y = np.asarray(y, dtype=np.int64); score = np.asarray(score, dtype=np.int64)
+    pv = np.zeros(int(max(x.max(initial=0), y.max(initial=0))) + 2, dtype=bool)
+    p = np.asarray(pivots, dtype=np.int64)
+    pv[p[p < pv.shape[0]]] = True
+    fwd, bwd = pv[x], pv[y]                         # (x, y) is emitted by pivot x, (y, x) by pivot y
+    dx = np.concatenate([x[fwd], y[bwd]]); dy = np.concatenate([y[fwd], x[bwd]]); ds = np.concatenate([score[fwd], score[bwd]])
+    keep = ds > sc_score
+    return canonical(dx[keep], dy[keep], ds[keep])
+
+
+def union_find(ex, ey, min_size, max_size=-1, restricted=None):
+    """The sequential union_find over a directed edge list in its given order. Only vertices some edge touches exist. A union
+    skips when both roots are restricted or the merged size would exceed max_size; otherwise the smaller root joins the larger, ties
+    to y's root, and the new root inherits `restricted`. -> (components of >= min_size vertices ordered by smallest member, each an
+    int64 array with the root first and the other members ascending; the spanning-tree edges of each, in replay order)"""
+    limit = (1 << 31) - 1 if max_size == -1 else int(max_size)
+    ex = np.asarray(ex, dtype=np.int64).tolist(); ey = np.asarray(ey, dtype=np.int64).tolist()
+    parent, size, tree = {}, {}, {}
+    for v in ex + ey:
+        parent[v] = v; size[v] = 1
+    rest = {int(v) for v in (restricted if restricted is not None else ()) if int(v) in parent}
+
+    def find(v):
+        r = v
+        while parent[r] != r:
+            r = parent[r]
+        while parent[v] != r:
+            parent[v], v = r, parent[v]
+        return r
+
+    order = []
+    for i, (x, y) in enumerate(zip(ex, ey)):
+        px, py = find(x), find(y)
+        if px == py or (px in rest and py in rest) or size[px] + size[py] > limit:
+            continue
+        big, small = (px, py) if size[px] > size[py] else (py, px)
+        parent[small] = big
+        size[big] += size[small]
+        if small in rest:
+            rest.add(big)
+        order.append(i)
+    verts = np.array(sorted(parent), dtype=np.int64)
+    roots = np.array([find(int(v)) for v in verts], dtype=np.int64)
+    comps, trees = [], []
+    for r in np.unique(roots):
+        if size[int(r)] < min_size:
+            continue
+        mem = verts[roots == r]
+        comps.append(np.concatenate([[r], mem[mem != r]]))
+    comps.sort(key=lambda c: int(c.min()))
+    at = {int(c[0]): j for j, c in enumerate(comps)}
+    trees = [([], []) for _ in comps]
+    for i in order:
+        j = at.get(find(ex[i]))
+        if j is not None:
+            trees[j][0].append(ex[i]); trees[j][1].append(ey[i])
+    return comps, [(np.array(a, dtype=np.int64), np.array(b, dtype=np.int64)) for a, b in trees]
+
+
+class State:
+    """The engine state merge_components and get_connections work on. Ids 1..n_reads; id r starts as read r with its k-mer id list
+    (sorted, one entry per hit) and contains read r. kl_id / kl_kmer: every (id, k-mer) list entry, sorted by (id, k-mer);
+    owner[r - 1]: the id that contains read r; inv_off / inv_id: the inverted index, one ascending id list per k-mer."""
+
+    def __init__(self, row_off, kid, n_kmers):
+        self.n_reads = np.asarray(row_off).shape[0] - 1
+        self.n_kmers = int(n_kmers)
+        rows = _rows(row_off) + 1
+        kid = np.asarray(kid, dtype=np.int64)
+        o = np.lexsort((kid, rows))
+        self.kl_id, self.kl_kmer = rows[o], kid[o]
+        self.owner = np.arange(1, self.n_reads + 1, dtype=np.int64)
+        self.inv_off, ids = index(row_off, kid, n_kmers)
+        self.inv_off = self.inv_off.astype(np.int64)
+        self.inv_id = ids.astype(np.int64)
+
+    def copy(self):
+        s = object.__new__(State)
+        s.__dict__.update({k: (v.copy() if isinstance(v, np.ndarray) else v) for k, v in self.__dict__.items()})
+        return s
+
+    def kmers_of(self, i):
+        lo, hi = np.searchsorted(self.kl_id, [i, i + 1])
+        return self.kl_kmer[lo:hi]
+
+    def ids(self, min_size):
+        """ids that contain >= min_size reads, ascending"""
+        cnt = np.bincount(self.owner, minlength=self.n_reads + 1)
+        return np.nonzero(cnt >= min_size)[0].astype(np.int64)
+
+    def reads_of(self, i):
+        return np.nonzero(self.owner == i)[0].astype(np.int64) + 1
+
+    def _inv_rows(self):
+        return np.repeat(np.arange(self.n_kmers, dtype=np.int64), np.diff(self.inv_off))
+
+
+def _entries(st, ids):
+    """(id, k-mer) list entries of the given ids, duplicates included"""
+    m = np.isin(st.kl_id, ids)
+    return st.kl_id[m], st.kl_kmer[m]
+
+
+def purge_walk(lst, removal):
+    """the purge of one inverted list as the reference writes it: a two-pointer walk over the ascending list and the ascending removal
+    list that ends when either runs out, keeping only what it copied"""
+    removal = sorted(removal)
+    out, i, j = [], 0, 0
+    while i < len(removal) and j < len(lst):
+        if removal[i] < lst[j]:
+            i += 1
+        elif lst[j] < removal[i]:
+            out.append(lst[j]); j += 1
+        else:
+            i += 1; j += 1
+    return out
+
+
+def purge(inv_off, inv_id, rem_kmer, rem_id):
+    """purge_walk of every list at once: k-mers with no removal entry keep their list; the others keep the entries below their largest
+    removed id, minus the removal multiset. -> (off, id)"""
+    inv_off = np.asarray(inv_off, dtype=np.int64); inv_id = np.asarray(inv_id, dtype=np.int64)
+    n_kmers = inv_off.shape[0] - 1
+    rem_kmer = np.asarray(rem_kmer, dtype=np.int64); rem_id = np.asarray(rem_id, dtype=np.int64)
+    base = int(max(inv_id.max(initial=0), rem_id.max(initial=0))) + 1
+    rows = np.repeat(np.arange(n_kmers, dtype=np.int64), np.diff(inv_off))
+    R = np.full(n_kmers, -1, dtype=np.int64)
+    np.maximum.at(R, rem_kmer, rem_id)
+    lk, lc = np.unique(rows * base + inv_id, return_counts=True)
+    rk, rc = np.unique(rem_kmer * base + rem_id, return_counts=True)
+    at = np.searchsorted(rk, lk)
+    hit = at < rk.shape[0]
+    hit[hit] = rk[at[hit]] == lk[hit]
+    r = np.zeros(lk.shape[0], dtype=np.int64)
+    r[hit] = rc[at[hit]]
+    k, e = lk // base, lk % base
+    keep = np.where(R[k] < 0, lc, np.where(e < R[k], np.maximum(lc - r, 0), 0))
+    off = np.zeros(n_kmers + 1, dtype=np.int64)
+    np.add.at(off, k + 1, keep)
+    return np.cumsum(off), np.repeat(e, keep)
+
+
+def merge(st, comps):
+    """merge_components: element [0] of every component of >= 2 ids survives with the sorted unique union of the members' k-mer lists
+    and all their reads; every member is removed from every k-mer once per entry of its current list (the survivor's current list
+    being the union), then every inverted list is purged (purge)."""
+    comps = [np.asarray(c, dtype=np.int64) for c in comps if len(c) > 1]
+    if not comps:
+        return st
+    mem = np.concatenate(comps)
+    surv = np.concatenate([np.full(len(c), c[0], dtype=np.int64) for c in comps])
+    mi, mk = _entries(st, mem)
+    into = np.zeros(st.n_reads + 1, dtype=np.int64)
+    into[mem] = surv
+    u = np.unique(into[mi] * (st.n_kmers + 1) + mk)
+    uid, ukm = u // (st.n_kmers + 1), u % (st.n_kmers + 1)
+    is_surv = np.zeros(st.n_reads + 1, dtype=bool)
+    is_surv[[c[0] for c in comps]] = True
+    other = ~is_surv[mi]
+    st.inv_off, st.inv_id = purge(st.inv_off, st.inv_id, np.concatenate([mk[other], ukm]), np.concatenate([mi[other], uid]))
+    keep = ~is_surv[st.kl_id]
+    kl_id = np.concatenate([st.kl_id[keep], uid]); kl_kmer = np.concatenate([st.kl_kmer[keep], ukm])
+    o = np.lexsort((kl_kmer, kl_id))
+    st.kl_id, st.kl_kmer = kl_id[o], kl_kmer[o]
+    moved = into[st.owner]
+    st.owner = np.where(moved != 0, moved, st.owner)
+    return st
+
+
+def connections(st, pivots, min_score):
+    """get_connections on the current state: score(p, y) = sum over the entries k of p's k-mer list of the copies of y in the list of
+    k, for y != p with score >= min_score. -> (x = pivot, y, score) in (x, y) order"""
+    pivots = np.unique(np.asarray(pivots, dtype=np.int64))
+    if pivots.shape[0] == 0:
+        z = np.zeros(0, dtype=np.int64)
+        return z, z, z
+    pi, pk = _entries(st, pivots)
+    a = sp.csr_matrix((np.ones(pi.shape[0], dtype=np.int64), (np.searchsorted(pivots, pi), pk)), shape=(pivots.shape[0], st.n_kmers))
+    b = sp.csr_matrix((np.ones(st.inv_id.shape[0], dtype=np.int64), (st._inv_rows(), st.inv_id)), shape=(st.n_kmers, st.n_reads + 1))
+    s = (a @ b).tocoo()
+    x, y, sc = pivots[s.row], s.col.astype(np.int64), s.data.astype(np.int64)
+    keep = (y != x) & (sc >= min_score)
+    x, y, sc = x[keep], y[keep], sc[keep]
+    o = np.lexsort((y, x))
+    return x[o], y[o], sc[o]
+
+
+def enrich(row_off, kid, n_kmers, ex, ey, min_size, enrich_min, max_size=-1, clusters=None):
+    """run_clustering from the directed scaffold list (ex, ey) on: union_find(min_size, max_size), merge of the scaffold components,
+    optionally a second merge of caller-given clusters of cores (the tail / spectral block's), cores = ids with >= min_size reads,
+    connections(cores, enrich_min) in canonical order, union_find(min 2, restricted = cores), merge, final ids with >= min_size reads.
+    -> dict with what hga_get_enrichment / hga_get_purged_index / hga_get_core_kmers return (in compare.check_enrichment's shape,
+    final components ordered by smallest member, assignment[r - 1] = final id of read r or 0), plus the scaffold components, their
+    spanning trees and the state right after the first merge"""
+    scaffold, trees = union_find(ex, ey, min_size, max_size)
+    st = merge(State(row_off, kid, n_kmers), scaffold)
+    first = st.copy()
+    if clusters is not None:
+        st = merge(st, clusters)
+    cores = st.ids(min_size)
+    core_kmers = [st.kmers_of(c) for c in cores]
+    core_reads = [st.reads_of(c) for c in cores]
+    purged_off, purged_read = st.inv_off.copy(), st.inv_id.copy()
+    cx, cy, cs = canonical(*connections(st, cores, enrich_min))
+    ecomp, _ = union_find(cx, cy, 2, restricted=cores)
+    merge(st, ecomp)
+    final = st.ids(min_size)
+    final_reads = [st.reads_of(f) for f in final]
+    o = np.argsort([int(r[0]) for r in final_reads], kind="stable")
+    final, final_reads = final[o], [final_reads[i] for i in o]
+    assignment = np.zeros(st.n_reads, dtype=np.int64)
+    for f, r in zip(final, final_reads):
+        assignment[r - 1] = f
+    return dict(core_id=cores, core_kmers=core_kmers, core_reads=core_reads, purged_off=purged_off, purged_read=purged_read,
+                econn=(cx, cy, cs), final_id=final, final_reads=final_reads, assignment=assignment,
+                scaffold=scaffold, trees=trees, first_merge=first)

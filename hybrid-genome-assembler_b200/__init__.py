@@ -5,6 +5,6 @@ libhga_b200.so (capi) and a mirror of the reference's ReadClusteringEngine stage
 There is no CPU path: importing works anywhere (so that the library's exports can be checked), but every compute
 entry point raises HgaError unless a CUDA device is present.
 """
-from .capi import HgaError, Handle, library_path, load_library  # noqa: F401
+from .capi import HgaError, Handle, library_path, load_library, pack_bases  # noqa: F401
 from .engine import ReadClusteringConfig, ReadClusteringEngine, load_text_file_kmers, SequenceRecords  # noqa: F401
 from . import capi, parallel  # noqa: F401,E402

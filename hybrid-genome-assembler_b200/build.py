@@ -20,7 +20,7 @@ EXE = os.path.join(HERE, "categorization")
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "-Xcompiler", "-fPIC", "-Xptxas", "-v",
               "--expt-relaxed-constexpr", "-I", os.path.join(ROOT, "include")]
-CPP_SOURCES = ["hga_spectral.cpp", "hga_tails.cpp", "hga_sdk.cpp"]        # host-only translation units (g++)
+CPP_SOURCES = ["hga_spectral.cpp", "hga_tails.cpp", "hga_sdk.cpp", "hga_pack.cpp"]        # host-only translation units (g++)
 CU_SOURCES = ["hga_capi.cu", "hga_table.cu", "hga_scan.cu", "hga_index.cu", "hga_pairs.cu", "hga_select.cu", "hga_cc.cu", "hga_enrich.cu", "hga_comm.cu", "hga_count.cu"]
 
 
@@ -43,7 +43,7 @@ def _run(cmd, verbose):
 
 def build(force=False, verbose=False):
     os.makedirs(BUILD, exist_ok=True)
-    headers = [os.path.join(CSRC, "hga_internal.cuh"), os.path.join(ROOT, "include", "hga_b200.h")]
+    headers = [os.path.join(CSRC, "hga_internal.cuh"), os.path.join(CSRC, "hga_pack.h"), os.path.join(ROOT, "include", "hga_b200.h")]
     objs, jobs = [], []
     for src in CU_SOURCES:
         s = os.path.join(CSRC, src)

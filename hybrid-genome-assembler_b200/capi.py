@@ -67,7 +67,7 @@ class Metrics(C.Structure):
 
 # every symbol include/hga_b200.h declares (tests check the .so exports exactly these)
 EXPORTS = ["hga_last_error", "hga_version", "hga_device_count", "hga_init", "hga_host_alloc", "hga_host_free", "hga_create", "hga_destroy", "hga_set_stream",
-           "hga_scan", "hga_scan_device", "hga_get_hits", "hga_build_index", "hga_get_index", "hga_pair_count", "hga_get_pairs", "hga_select_edges",
+           "hga_scan", "hga_scan_device", "hga_host_pack_bases", "hga_scan_packed", "hga_scan_packed_device", "hga_get_hits", "hga_build_index", "hga_get_index", "hga_pair_count", "hga_get_pairs", "hga_select_edges",
            "hga_get_selection", "hga_components", "hga_get_components", "hga_enrich", "hga_enrich_ex", "hga_enrich_full", "hga_get_tail_block", "hga_count_kmers", "hga_free_kmer_counts", "hga_host_sdk_merge", "hga_host_sdk_specificity", "hga_host_sdk_select", "hga_get_enrichment", "hga_get_purged_index", "hga_get_core_kmers", "hga_spectral_clustering", "hga_host_tail_connections", "hga_host_sym_eigen",
            "hga_metrics", "hga_comm_unique_id", "hga_comm_init", "hga_comm_gather_root"]
 
@@ -92,6 +92,10 @@ def load_library():
         lib.hga_set_stream.argtypes = [C.c_void_p, C.c_void_p]
         lib.hga_scan.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint32]
         lib.hga_scan_device.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint32]
+        lib.hga_host_pack_bases.argtypes = [C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64), C.c_int]
+        lib.hga_scan_packed.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint32]
+        lib.hga_scan_packed_device.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64, C.c_uint64, C.c_void_p, C.c_void_p, C.c_uint64,
+                                               C.c_uint32]
         lib.hga_get_hits.argtypes = [C.c_void_p, C.c_int, C.POINTER(_Hits)]
         lib.hga_build_index.argtypes = [C.c_void_p]
         lib.hga_get_index.argtypes = [C.c_void_p, C.POINTER(_Index)]
@@ -128,6 +132,36 @@ def _arr(ptr, n, dtype):
     if n == 0:
         return np.zeros(0, dtype=dtype)
     return np.ctypeslib.as_array(ptr, shape=(int(n),)).astype(dtype, copy=True)
+
+
+def _host_bytes(bases):
+    """(keep-alive object, pointer, length) of host bytes given as bytes / bytearray / uint8 array"""
+    if isinstance(bases, np.ndarray):
+        b = np.ascontiguousarray(bases, dtype=np.uint8)
+        return b, b.ctypes.data_as(C.c_void_p), b.shape[0]
+    b = bytes(bases)
+    return b, C.cast(C.c_char_p(b), C.c_void_p), len(b)
+
+
+def pack_bases(bases, threads=0, capacity=64):
+    """hga_host_pack_bases: ASCII bases -> (packed uint8[(n + 3) // 4], exc_start uint64[], exc_end uint64[]), the input of Handle.scan_packed.
+    Codes A0 C1 G2 T3, four bases per byte, first base in the most significant bits; every byte other than uppercase ACGT is code 0 under
+    a maximal exception run [start, end). Starts with `capacity` runs and retries once with the exact count."""
+    lib = load_library()
+    keep, ptr, n = _host_bytes(bases)
+    packed = np.zeros((n + 3) // 4, dtype=np.uint8)
+    n_exc = C.c_uint64()
+    while True:
+        cap = max(int(capacity), 1)
+        st = np.zeros(cap, dtype=np.uint64); en = np.zeros(cap, dtype=np.uint64)
+        rc = lib.hga_host_pack_bases(ptr, n, packed.ctypes.data_as(C.c_void_p), st.ctypes.data_as(C.c_void_p), en.ctypes.data_as(C.c_void_p), cap,
+                                     C.byref(n_exc), int(threads))
+        if rc == 2 and n_exc.value > cap:
+            capacity = n_exc.value
+            continue
+        _check(rc)
+        del keep
+        return packed, st[:n_exc.value].copy(), en[:n_exc.value].copy()
 
 
 def spectral_clustering(conn_x, conn_y, conn_score, dims=16):
@@ -320,6 +354,26 @@ class Handle:
 
     def scan_device(self, d_bases_ptr, d_read_off_ptr, n_reads, n_bases, read_id_base=1):
         _check(self.lib.hga_scan_device(self._h, C.c_void_p(d_bases_ptr), C.c_void_p(d_read_off_ptr), int(n_reads), int(n_bases), int(read_id_base)))
+
+    def scan_packed(self, packed, read_off, exc_start, exc_end, first_base=0, read_id_base=1):
+        """packed: uint8 array / bytes (host), bases first_base + read_off[..] of it; exc_start / exc_end: the exception runs relative to
+        first_base (pack_bases gives them for first_base = 0)."""
+        read_off = np.ascontiguousarray(read_off, dtype=np.uint64)
+        st = np.ascontiguousarray(exc_start, dtype=np.uint64); en = np.ascontiguousarray(exc_end, dtype=np.uint64)
+        if st.shape != en.shape:
+            raise ValueError("exc_start and exc_end differ in length")
+        keep, ptr, _ = _host_bytes(packed)
+        _check(self.lib.hga_scan_packed(self._h, ptr, int(first_base), read_off.ctypes.data_as(C.c_void_p), read_off.shape[0] - 1,
+                                        st.ctypes.data_as(C.c_void_p), en.ctypes.data_as(C.c_void_p), st.shape[0], int(read_id_base)))
+        del keep
+
+    def scan_packed_host_ptr(self, packed_ptr, first_base, read_off_ptr, n_reads, exc_start_ptr, exc_end_ptr, n_exc, read_id_base=1):
+        _check(self.lib.hga_scan_packed(self._h, C.c_void_p(packed_ptr), int(first_base), C.c_void_p(read_off_ptr), int(n_reads), C.c_void_p(exc_start_ptr),
+                                        C.c_void_p(exc_end_ptr), int(n_exc), int(read_id_base)))
+
+    def scan_packed_device(self, d_packed_ptr, first_base, d_read_off_ptr, n_reads, n_bases, d_exc_start_ptr, d_exc_end_ptr, n_exc, read_id_base=1):
+        _check(self.lib.hga_scan_packed_device(self._h, C.c_void_p(d_packed_ptr), int(first_base), C.c_void_p(d_read_off_ptr), int(n_reads), int(n_bases),
+                                               C.c_void_p(d_exc_start_ptr), C.c_void_p(d_exc_end_ptr), int(n_exc), int(read_id_base)))
 
     def get_hits(self, sorted_by_kmer_id=False):
         out = _Hits()

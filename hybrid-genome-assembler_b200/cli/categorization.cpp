@@ -126,6 +126,14 @@ hga_handle *run_hot_path_multi(const hga_host::KmerSet &ks, const hga_host::Sequ
             const uint64_t lo = bound[r], hi = bound[r + 1];
             std::vector<uint64_t> off(hi - lo + 1);
             for (uint64_t i = lo; i <= hi; i++) off[i - lo] = reads.seq_off[i] - reads.seq_off[lo];
+            // the rank's slice of the packed stream is scanned in place: its exception runs, clipped to the slice and rebased
+            const uint64_t b0 = reads.seq_off[lo], b1 = reads.seq_off[hi];
+            std::vector<uint64_t> es, ee;
+            for (size_t j = (size_t) (std::upper_bound(reads.exc_end.begin(), reads.exc_end.end(), b0) - reads.exc_end.begin());
+                 j < reads.exc_start.size() && reads.exc_start[j] < b1; j++) {
+                es.push_back(std::max(reads.exc_start[j], b0) - b0);
+                ee.push_back(std::min(reads.exc_end[j], b1) - b0);
+            }
             double t = now();
             auto lap = [&](int i) { const double n2 = now(); if (r == 0) stamp[i] = n2 - t; t = n2; };
             // every stage is entered by all ranks or by none
@@ -134,7 +142,7 @@ hga_handle *run_hot_path_multi(const hga_host::KmerSet &ks, const hga_host::Sequ
             alive = !fail(hga_comm_init(hs[r], id, r, gpus, n_reads), "hga_comm_init");
             if (!meet(alive)) return;
             lap(0);
-            alive = !fail(hga_scan(hs[r], reads.bases_data + reads.seq_off[lo], off.data(), hi - lo, (uint32_t) (lo + 1)), "hga_scan");
+            alive = !fail(hga_scan_packed(hs[r], reads.packed_data, b0, off.data(), hi - lo, es.data(), ee.data(), es.size(), (uint32_t) (lo + 1)), "hga_scan_packed");
             if (!meet(alive)) return;
             lap(1);
             alive = !fail(hga_build_index(hs[r]), "hga_build_index");
@@ -256,7 +264,8 @@ int main(int argc, char **argv) {
     hga_host::KmerSet ks;
     Timer t_load("Loading of k-mers and reads");
     if (!parse_only && !kmer_path.empty()) ks = hga_host::load_text_file_kmers(kmer_path, config.threads > 1 ? config.threads : 0);
-    hga_host::SequenceRecords reads(read_paths, config.threads > 1 ? config.threads : 0);
+    // the reads are packed while they load (2-bit codes + exception runs: a quarter of the bytes to copy to the GPU)
+    hga_host::SequenceRecords reads(read_paths, config.threads > 1 ? config.threads : 0, /*packed=*/true);
     if (!parse_only) t_load.done();
     if (export_test) {   // writer self-test (no GPU): read r (1-based) goes to component 1 + r % 3, every 7th read to none
         std::vector<uint32_t> of_read(reads.n_reads());
@@ -311,7 +320,8 @@ int main(int argc, char **argv) {
         const auto w0 = std::chrono::steady_clock::now();
         check(hga_create(device, ks.k, ks.kmers.data(), ks.kmers.size(), &h), "hga_create");
         const auto w1 = std::chrono::steady_clock::now();
-        check(hga_scan(h, reads.bases_data, reads.seq_off.data(), reads.n_reads(), 1), "hga_scan");
+        check(hga_scan_packed(h, reads.packed_data, 0, reads.seq_off.data(), reads.n_reads(), reads.exc_start.data(), reads.exc_end.data(), reads.exc_start.size(), 1),
+              "hga_scan_packed");
         const auto w2 = std::chrono::steady_clock::now();
         check(hga_build_index(h), "hga_build_index");
         const auto w3 = std::chrono::steady_clock::now();

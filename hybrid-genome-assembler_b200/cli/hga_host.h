@@ -23,6 +23,8 @@
 #include <thread>
 #include <vector>
 
+#include "../csrc/hga_pack.h"
+
 #include <fcntl.h>
 #include <sys/mman.h>
 #include <sys/stat.h>
@@ -183,17 +185,20 @@ struct MetaData {
 
 // All records of the input files, loaded in ONE pass over the mapped files (the reference reads every file twice: once for
 // load_meta_data, SequenceRecordIterator.cpp:31-71, once for the records). Phase 1 (sequential, memchr) finds the lines and
-// applies the record rules; phase 2 copies the sequence bytes into one contiguous buffer (what hga_scan takes) with several
-// threads. The buffer is 2 MB aligned and advised MADV_HUGEPAGE: first-touch page faults, not memcpy, are what bounds the copy
-// (measured on 1.2 GB: 1.17 s single thread with 4 KB pages, 0.29 s with huge pages and 8 threads). Headers and qualities stay
-// views into the mappings.
+// applies the record rules; phase 2 writes the sequences into one contiguous buffer with several threads: the ASCII bytes (what
+// hga_scan and hga_count_kmers take) or, with `packed`, the 2-bit codes and exception runs of hga_scan_packed, a quarter of the
+// bytes, written straight from the mappings. The buffer is 2 MB aligned and advised MADV_HUGEPAGE: first-touch page faults, not
+// memcpy, are what bounds the copy (measured on 1.2 GB: 1.17 s single thread with 4 KB pages, 0.29 s with huge pages and 8 threads).
+// Headers, sequences and qualities stay views into the mappings.
 struct SequenceRecords {
     struct View { uint32_t file; uint32_t len; uint64_t off; };
     std::vector<std::string> paths;
     std::vector<MappedFile> files;
     std::vector<MetaData> file_meta;
     MetaData meta;
-    char *bases_data = nullptr;          // sequences back to back
+    char *bases_data = nullptr;          // ASCII mode: sequences back to back
+    uint8_t *packed_data = nullptr;      // packed mode: the same stream, 2-bit codes, (bases_size + 3) / 4 bytes
+    std::vector<uint64_t> exc_start, exc_end;   // packed mode: maximal runs of bytes other than A C G T, stream positions
     uint64_t bases_size = 0;
     std::vector<uint64_t> seq_off;       // n_reads + 1
     std::vector<View> header_v, quality_v, seq_v;
@@ -204,8 +209,8 @@ struct SequenceRecords {
     size_t n_reads() const { return header_v.size(); }
     std::string_view header(size_t i) const { return {files[header_v[i].file].data + header_v[i].off, header_v[i].len}; }
     std::string_view quality(size_t i) const { return is_fastq[i] ? std::string_view{files[quality_v[i].file].data + quality_v[i].off, quality_v[i].len} : std::string_view{}; }
-    std::string_view sequence(size_t i) const { return {bases_data + seq_off[i], (size_t) (seq_off[i + 1] - seq_off[i])}; }
-    ~SequenceRecords() { free(bases_data); }
+    std::string_view sequence(size_t i) const { return {files[seq_v[i].file].data + seq_v[i].off, seq_v[i].len}; }
+    ~SequenceRecords() { free(bases_data); free(packed_data); }
     SequenceRecords(const SequenceRecords &) = delete;
     SequenceRecords &operator=(const SequenceRecords &) = delete;
 
@@ -221,7 +226,8 @@ struct SequenceRecords {
         return o.str();
     }
 
-    explicit SequenceRecords(const std::vector<std::string> &read_paths, int threads = 0) : paths(read_paths), file_meta(read_paths.size()) {
+    // threads <= 0: automatic (one thread below 8 MB of bases)
+    explicit SequenceRecords(const std::vector<std::string> &read_paths, int threads = 0, bool packed = false) : paths(read_paths), file_meta(read_paths.size()) {
         files.reserve(paths.size());
         int cur = -1, method = 4;
         const char *p = nullptr, *end = nullptr;       // cursor in the current file
@@ -313,10 +319,12 @@ struct SequenceRecords {
         // phase 2: the sequence bytes, in parallel
         bases_size = seq_off.back();
         const size_t huge = (size_t) 1 << 21;
-        const size_t cap = ((size_t) bases_size + 64 + huge - 1) & ~(huge - 1);
-        bases_data = (char *) aligned_alloc(huge, cap);
-        if (!bases_data) throw std::bad_alloc();
-        madvise(bases_data, cap, MADV_HUGEPAGE);
+        const size_t cap = ((size_t) (packed ? (bases_size + 3) / 4 : bases_size) + 64 + huge - 1) & ~(huge - 1);
+        void *buf = aligned_alloc(huge, cap);
+        if (!buf) throw std::bad_alloc();
+        madvise(buf, cap, MADV_HUGEPAGE);
+        if (packed) { packed_data = (uint8_t *) buf; pack_from_mappings(threads); return; }
+        bases_data = (char *) buf;
         int T = threads > 0 ? threads : (int) std::min(16u, std::max(1u, std::thread::hardware_concurrency()));
         if (bases_size < ((uint64_t) 8 << 20)) T = 1;
         const size_t n = seq_v.size();
@@ -337,7 +345,37 @@ struct SequenceRecords {
             }
             for (auto &th : pool) th.join();
         }
-        std::vector<View>().swap(seq_v);
+    }
+
+private:
+    // packed mode of phase 2: thread t packs stream positions [per * t, per * (t + 1)) (per: a multiple of 4, so a thread owns whole
+    // bytes) piece by piece from the mappings; the runs of neighbouring threads are joined at the seams
+    void pack_from_mappings(int threads) {
+        const uint64_t n_bytes = (bases_size + 3) / 4;
+        int T = threads > 0 ? threads : (bases_size < ((uint64_t) 8 << 20) ? 1 : (int) std::min(16u, std::max(1u, std::thread::hardware_concurrency())));
+        T = (int) std::max<uint64_t>(1, std::min<uint64_t>((uint64_t) T, n_bytes));
+        const uint64_t per = (n_bytes + T - 1) / T * 4;
+        std::vector<hga_pack::Packer> part;
+        part.reserve(T);
+        for (int t = 0; t < T; t++) part.emplace_back(packed_data, std::min(bases_size, per * t));
+        auto work = [&](int t) {
+            const uint64_t a = std::min(bases_size, per * t), b = std::min(bases_size, per * (t + 1));
+            if (a >= b) return;
+            size_t i = (size_t) (std::upper_bound(seq_off.begin(), seq_off.end(), a) - seq_off.begin()) - 1;     // the read holding a
+            for (; i < seq_v.size() && seq_off[i] < b; i++) {
+                const uint64_t lo = std::max(a, seq_off[i]), hi = std::min(b, seq_off[i + 1]);
+                if (lo < hi) part[t].put(files[seq_v[i].file].data + seq_v[i].off + (lo - seq_off[i]), hi - lo);
+            }
+        };
+        if (T == 1) work(0);
+        else {
+            std::vector<std::thread> pool;
+            for (int t = 0; t < T; t++) pool.emplace_back(work, t);
+            for (auto &th : pool) th.join();
+        }
+        hga_pack::Runs all;
+        for (int t = 0; t < T; t++) all.append(part[t].runs);
+        exc_start.swap(all.start); exc_end.swap(all.end);
     }
 };
 

@@ -144,7 +144,7 @@ void hga_destroy(hga_handle *h) {
     cudaDeviceSynchronize();
     hga_comm_destroy(h);
     DevBuf *dev[] = {&h->d_keys, &h->d_slot_kid, &h->d_kid_slot, &h->d_filter, &h->d_bases, &h->d_read_off, &h->d_row_off, &h->d_hit_slot, &h->d_hit_pos, &h->d_pos_tmp,
-                     &h->d_tile_state, &h->d_tile_dir, &h->d_scan_scalars, &h->d_x_slot, &h->d_x_row, &h->d_g_kid, &h->d_g_row_off, &h->d_inv_off, &h->d_inv_row, &h->d_sort_a,
+                     &h->d_tile_state, &h->d_tile_dir, &h->d_scan_scalars, &h->d_exc, &h->d_exc_dir, &h->d_x_slot, &h->d_x_row, &h->d_g_kid, &h->d_g_row_off, &h->d_inv_off, &h->d_inv_row, &h->d_sort_a,
                      &h->d_index_tmp, &h->d_index_goff, &h->d_sort_b, &h->d_sort_tmp, &h->d_pair_key, &h->d_pair_score, &h->d_pair_key2, &h->d_pair_score2, &h->d_pair_scalars,
                      &h->d_heavy_list, &h->d_mid_list, &h->d_redo_list, &h->d_heavy_tab, &h->d_pivot_flag, &h->d_pivot_order, &h->d_pivot_rows, &h->d_hist, &h->d_sel_key, &h->d_sel_score, &h->d_sel_scalars, &h->d_parent,
                      &h->d_comp_size, &h->d_comp_label, &h->d_comp_scalars, &h->d_export_a, &h->d_export_b, &h->d_export_c, &h->d_enr_parent, &h->d_enr_core_of,
@@ -193,6 +193,63 @@ int hga_scan(hga_handle *h, const char *bases, const uint64_t *read_off, uint64_
     HGA_CUDA(cudaMemcpyAsync(h->d_read_off.p, read_off, (n_reads + 1) * 8, cudaMemcpyHostToDevice, h->stream));
     h->read_id_base = read_id_base;
     return hga_scan_run(h, h->d_bases.as<char>(), h->d_read_off.as<uint64_t>(), n_reads, n_bases, bases);
+}
+
+// read_off of a host entry: read_off[0] == 0, monotone, no read of 2^30 bases or more
+static int check_read_off(const char *who, const uint64_t *read_off, uint64_t n_reads) {
+    if (read_off[0] != 0) { hga_set_error("%s: read_off[0] must be 0", who); return HGA_E_ARG; }
+    for (uint64_t i = 0; i < n_reads; i++) {
+        if (read_off[i + 1] < read_off[i]) { hga_set_error("%s: read_off is not monotone at read %llu", who, (unsigned long long) i); return HGA_E_ARG; }
+        if (read_off[i + 1] - read_off[i] >= (1ull << 30)) { hga_set_error("%s: read %llu is longer than 2^30 bases", who, (unsigned long long) i); return HGA_E_ARG; }
+    }
+    return HGA_OK;
+}
+
+int hga_scan_packed(hga_handle *h, const uint8_t *packed, uint64_t first_base, const uint64_t *read_off, uint64_t n_reads, const uint64_t *exc_start,
+                    const uint64_t *exc_end, uint64_t n_exc, uint32_t read_id_base) {
+    if (!h) { hga_set_error("NULL handle"); return HGA_E_ARG; }
+    if (!read_off) { hga_set_error("hga_scan_packed: read_off is NULL"); return HGA_E_ARG; }
+    HGA_TRY(use_device(h));
+    HGA_TRY(check_read_off("hga_scan_packed", read_off, n_reads));
+    const uint64_t n_bases = read_off[n_reads];
+    if (n_bases && !packed) { hga_set_error("hga_scan_packed: packed is NULL"); return HGA_E_ARG; }
+    if (n_exc && (!exc_start || !exc_end)) { hga_set_error("hga_scan_packed: exception runs are NULL"); return HGA_E_ARG; }
+    for (uint64_t i = 0; i < n_exc; i++) {
+        if (exc_start[i] >= exc_end[i] || exc_end[i] > n_bases || (i && exc_start[i] < exc_end[i - 1])) {
+            hga_set_error("hga_scan_packed: exception run %llu [%llu, %llu) is empty, out of order, overlaps its predecessor or lies outside [0, %llu)",
+                          (unsigned long long) i, (unsigned long long) exc_start[i], (unsigned long long) exc_end[i], (unsigned long long) n_bases);
+            return HGA_E_ARG;
+        }
+    }
+    // only the bytes that hold the read set travel; on the device they start at an aligned buffer, first_base % 4 bases into its first byte
+    const uint32_t sub = (uint32_t) (first_base & 3);
+    const uint64_t n_bytes = n_bases ? (sub + n_bases + 3) / 4 : 0;
+    HGA_TRY(h->d_bases.ensure(n_bytes + 64));
+    HGA_TRY(h->d_read_off.ensure((n_reads + 1) * 8));
+    HGA_TRY(h->d_exc.ensure(n_exc * 16 + 16));
+    h->metrics.h2d_ms = 0;
+    HGA_CUDA(cudaMemcpyAsync(h->d_read_off.p, read_off, (n_reads + 1) * 8, cudaMemcpyHostToDevice, h->stream));
+    h->read_id_base = read_id_base;
+    ScanPackedInput in;
+    in.sub = sub;
+    in.d_exc_start = h->d_exc.as<uint64_t>(); in.d_exc_end = in.d_exc_start + n_exc;
+    in.h_exc_start = exc_start; in.h_exc_end = exc_end; in.n_exc = n_exc; in.check = false;
+    return hga_scan_run(h, h->d_bases.as<char>(), h->d_read_off.as<uint64_t>(), n_reads, n_bases, n_bytes ? reinterpret_cast<const char *>(packed + first_base / 4) : nullptr,
+                        &in);
+}
+
+int hga_scan_packed_device(hga_handle *h, const uint8_t *d_packed, uint64_t first_base, const uint64_t *d_read_off, uint64_t n_reads, uint64_t n_bases,
+                           const uint64_t *d_exc_start, const uint64_t *d_exc_end, uint64_t n_exc, uint32_t read_id_base) {
+    if (!h) { hga_set_error("NULL handle"); return HGA_E_ARG; }
+    if ((n_bases && !d_packed) || !d_read_off) { hga_set_error("hga_scan_packed_device: NULL buffer"); return HGA_E_ARG; }
+    if (n_exc && (!d_exc_start || !d_exc_end)) { hga_set_error("hga_scan_packed_device: exception runs are NULL"); return HGA_E_ARG; }
+    if (n_exc > n_bases) { hga_set_error("hga_scan_packed_device: %llu exception runs for %llu bases", (unsigned long long) n_exc, (unsigned long long) n_bases); return HGA_E_ARG; }
+    HGA_TRY(use_device(h));
+    h->read_id_base = read_id_base;
+    ScanPackedInput in;
+    in.sub = (uint32_t) (first_base & 3);
+    in.d_exc_start = d_exc_start; in.d_exc_end = d_exc_end; in.h_exc_start = in.h_exc_end = nullptr; in.n_exc = n_exc; in.check = true;
+    return hga_scan_run(h, reinterpret_cast<const char *>(d_packed + first_base / 4), d_read_off, n_reads, n_bases, nullptr, &in);
 }
 
 int hga_get_hits(hga_handle *h, int sorted_by_kmer_id, hga_hits *out) {

@@ -288,6 +288,7 @@ struct hga_handle {
     double scan_density = 0;              // hits per base of the previous scan on this handle (sizes the next one's hit buffers)
     bool pos_pending = false;
     DevBuf d_tile_state, d_tile_dir, d_scan_scalars;
+    DevBuf d_exc, d_exc_dir;              // packed scans: exception runs (host entry: starts then ends), first run touching each tile + check flag
     bool have_scan = false;
 
     // row space of the inverted index, pairs and components (this GPU's reads; ALL reads with a communicator)
@@ -347,8 +348,18 @@ struct hga_handle {
 
 // stage launchers (each in its own .cu)
 int hga_table_build(hga_handle *h, const uint64_t *host_kmers);
+// A packed scan (hga_scan_packed*): d_bases / h_bases point at the byte that holds the first base, `sub` bases into it (0..3).
+struct ScanPackedInput {
+    uint32_t sub;
+    const uint64_t *d_exc_start, *d_exc_end;  // device, n_exc each (the host entry's runs are copied there first: h_exc_* != nullptr)
+    const uint64_t *h_exc_start, *h_exc_end;
+    uint64_t n_exc;
+    bool check;                               // device entry: validate the runs on the GPU, fail with HGA_E_ARG
+};
 // h_bases != nullptr: the bases are still on the host; the run copies them (in chunks, overlapped with the scan when large)
-int hga_scan_run(hga_handle *h, const char *d_bases, const uint64_t *d_read_off, uint64_t n_reads, uint64_t n_bases, const char *h_bases);
+// packed == nullptr: ASCII bases, one byte each
+int hga_scan_run(hga_handle *h, const char *d_bases, const uint64_t *d_read_off, uint64_t n_reads, uint64_t n_bases, const char *h_bases,
+                 const ScanPackedInput *packed = nullptr);
 int hga_scan_finish_positions(hga_handle *h);
 int hga_index_run(hga_handle *h);
 int hga_build_lists(hga_handle *h, const uint32_t *d_keys, const uint64_t *d_row_off, uint64_t n_rows, uint64_t E, uint32_t n_keys);

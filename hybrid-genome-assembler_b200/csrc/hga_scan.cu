@@ -76,6 +76,11 @@ struct ScanParams {
     uint32_t chunk;                   // hit-buffer entries a warp reserves per atomic
     unsigned long long *warp_chunks;  // chunked launches: every warp's open chunk [pos, end) survives from one launch to the next (nullptr: one launch)
     int diag;                         // HGA_SCAN_DIAG experiment: 1 = no key probes (results are WRONG), 2 = metrics.n_candidates counts sector probes
+    // packed input (hga_scan_packed*; appended so that the parameter offsets of the ASCII kernels stay as they were). frame is then 4 B aligned
+    // and lead counts bases (0..15)
+    const uint64_t *exc_start, *exc_end;  // exception runs, half-open stream positions, sorted and disjoint
+    uint64_t n_exc;
+    const unsigned long long *exc_dir;    // per tile: the first run that touches its staged span, ~0 = none (nullptr: no runs, never read)
 };
 
 // shared memory of one warp
@@ -384,7 +389,9 @@ __device__ __forceinline__ uint32_t phase_c(const TileCtx &c, int lane, uint32_t
 // TMA (experiment, HGA_SCAN_TMA=1): the tile's 512 bytes arrive by a 1-D bulk copy (cp.async.bulk, evict-first in L2) into a per-warp double buffer and
 // complete on an mbarrier; the copy of the NEXT tile is in flight while the current one is processed, so phase A never waits for HBM.
 #define SCAN_STAGE_BYTES (2 * SCAN_SPAN + 16)    // two tile buffers + two mbarriers per warp
-template<int MINB, bool TMA>
+// PACKED: the bases arrive 2-bit packed (4 per byte, first base most significant): a lane loads one 4-byte word = its 16 bases, the
+// exception runs of the tile come from the run directory. Phases B and C, the drain and the hit staging are the same code.
+template<int MINB, bool TMA, bool PACKED = false>
 __global__ void __launch_bounds__(SCAN_THREADS, MINB) scan_probe_kernel(const __grid_constant__ ScanParams p) {
     extern __shared__ __align__(16) unsigned char s_raw[];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -475,7 +482,34 @@ __global__ void __launch_bounds__(SCAN_THREADS, MINB) scan_probe_kernel(const __
 
         // ---- phase A: 16 bases per lane, packed to one word per strand -----------------------------------------------
         uint32_t P[3], Q[3], bad = 0;
-        {
+        if (PACKED) {
+            const int64_t u = ubase + SCAN_LANE * lane;
+            uint32_t w = 0;                                                            // outside the stream: code 0 (never inside a valid window)
+            if (u >= 0 && u < u_end)
+                asm volatile("ld.global.L1::no_allocate.L2::cache_hint.u32 %0, [%1], %2;" : "=r"(w) : "l"(p.frame + u / 4), "l"(pol_stream));
+            P[2] = __byte_perm(w, 0u, 0x0123u);                                        // byte 0 holds the first 4 bases: to the top
+            uint32_t x = __brev(P[2]);                                                 // base j's pair at bits 2j, 2j + 1, its two bits swapped
+            x = ((x >> 1) & 0x55555555u) | ((x & 0x55555555u) << 1);
+            Q[2] = ~x;                                                                 // complement codes (3 - c), first base least significant
+            if (p.exc_dir != nullptr) {
+                const unsigned long long r0 = __ldg(&p.exc_dir[tile]);
+                if (r0 != ~0ull) {                                                     // rare: the runs that touch the tile, warp uniform
+                    const int64_t g0 = gbase + SCAN_LANE * lane, g_end = gbase + SCAN_SPAN;
+                    for (uint64_t r = r0; r < p.n_exc; r++) {
+                        const int64_t s = (int64_t) __ldg(&p.exc_start[r]);
+                        if (s >= g_end) break;
+                        const int64_t e = (int64_t) __ldg(&p.exc_end[r]);
+                        const int64_t lo = max(s - g0, (int64_t) 0), hi = min(e - g0, (int64_t) SCAN_LANE);
+                        if (lo < hi) bad |= (0xFFFFu >> (SCAN_LANE - (int) (hi - lo))) << (int) lo;
+                    }
+                    uint32_t m = bad;                                                  // bit j -> bits 2j, 2j + 1: clear those codes on both strands
+                    m = (m | (m << 8)) & 0x00FF00FFu; m = (m | (m << 4)) & 0x0F0F0F0Fu;
+                    m = (m | (m << 2)) & 0x33333333u; m = (m | (m << 1)) & 0x55555555u;
+                    m *= 3u;
+                    Q[2] &= ~m; P[2] &= ~__brev(m);
+                }
+            }
+        } else {
             const int64_t u = ubase + SCAN_LANE * lane;
             uint32_t v[4];
             if (u >= 0 && u < u_end) {
@@ -609,6 +643,28 @@ __global__ void scan_tile_dir_kernel(const uint64_t *__restrict__ read_off, uint
     }
 }
 
+// packed scans: per tile, the first exception run that touches the tile's staged span (stream positions [480 t - 32 - lead, + 512)), ~0
+// when none does, so that a tile without exceptions pays one directory load
+__global__ void scan_exc_dir_kernel(const uint64_t *__restrict__ exc_start, const uint64_t *__restrict__ exc_end, uint64_t n_exc, uint64_t n_tiles, uint32_t lead,
+                                    unsigned long long *dir) {
+    for (uint64_t t = blockIdx.x * (uint64_t) blockDim.x + threadIdx.x; t < n_tiles; t += (uint64_t) gridDim.x * blockDim.x) {
+        const int64_t s0 = (int64_t) (t * SCAN_TILE) - 32 - (int64_t) lead;
+        uint64_t lo = 0, hi = n_exc;          // first run ending after s0
+        while (lo < hi) { const uint64_t mid = (lo + hi) >> 1; if ((int64_t) exc_end[mid] <= s0) lo = mid + 1; else hi = mid; }
+        dir[t] = (lo < n_exc && (int64_t) exc_start[lo] < s0 + SCAN_SPAN) ? lo : ~0ull;
+    }
+}
+
+// device entry of a packed scan: read_off[0] must be 0 and the runs non-empty, sorted, disjoint and inside [0, n_bases); a violation sets *bad
+__global__ void scan_exc_check_kernel(const uint64_t *__restrict__ read_off, const uint64_t *__restrict__ exc_start, const uint64_t *__restrict__ exc_end,
+                                      uint64_t n_exc, uint64_t n_bases, unsigned long long *bad) {
+    if (blockIdx.x == 0 && threadIdx.x == 0 && read_off[0] != 0) *bad = 1;
+    for (uint64_t i = blockIdx.x * (uint64_t) blockDim.x + threadIdx.x; i < n_exc; i += (uint64_t) gridDim.x * blockDim.x) {
+        const uint64_t s = exc_start[i], e = exc_end[i];
+        if (s >= e || e > n_bases || (i + 1 < n_exc && exc_start[i + 1] < e)) *bad = 1;
+    }
+}
+
 // tile segments (completion order, with the gaps the chunked allocation leaves) -> stream order. A warp takes 32 consecutive tiles: their
 // directory entries arrive in three coalesced loads (one tile per lane) and are handed round with shuffles; the 32 destinations are
 // one contiguous range. (One warp per tile with three dependent scalar loads each: 3.1 ms at config 4, r2q.)
@@ -657,16 +713,17 @@ bool scan_tma_variant() {
 }
 
 typedef void (*scan_kernel_t)(const ScanParams);
-scan_kernel_t scan_kernel() {
+scan_kernel_t scan_kernel(bool packed) {
+    if (packed) return scan_probe_kernel<4, false, true>;          // the experiment switches apply to ASCII input only
     if (scan_tma_variant()) return scan_probe_kernel<4, true>;
     if (scan_occ_variant() == 3) return scan_probe_kernel<3, false>;
     if (scan_occ_variant() == 5) return scan_probe_kernel<5, false>;
     return scan_probe_kernel<4, false>;
 }
-size_t scan_smem_bytes() { return SCAN_WARPS * sizeof(WarpTile) + (scan_tma_variant() ? (size_t) SCAN_WARPS * SCAN_STAGE_BYTES : 0); }
+size_t scan_smem_bytes(bool packed) { return SCAN_WARPS * sizeof(WarpTile) + (!packed && scan_tma_variant() ? (size_t) SCAN_WARPS * SCAN_STAGE_BYTES : 0); }
 
-int launch_scan(hga_handle *h, const ScanParams &p, int grid) {
-    scan_kernel()<<<grid, SCAN_THREADS, scan_smem_bytes(), h->stream>>>(p);
+int launch_scan(hga_handle *h, const ScanParams &p, int grid, bool packed) {
+    scan_kernel(packed)<<<grid, SCAN_THREADS, scan_smem_bytes(packed), h->stream>>>(p);
     HGA_CUDA(cudaGetLastError());
     h->metrics.kernel_launches++;
     return HGA_OK;
@@ -674,14 +731,21 @@ int launch_scan(hga_handle *h, const ScanParams &p, int grid) {
 
 }  // namespace
 
-int hga_scan_run(hga_handle *h, const char *d_bases, const uint64_t *d_read_off, uint64_t n_reads, uint64_t n_bases, const char *h_bases) {
+int hga_scan_run(hga_handle *h, const char *d_bases, const uint64_t *d_read_off, uint64_t n_reads, uint64_t n_bases, const char *h_bases,
+                 const ScanPackedInput *packed) {
     h->have_scan = h->have_index = h->have_pairs = h->have_selection = h->have_components = h->have_enrichment = false;
     h->n_reads = n_reads; h->n_bases = n_bases; h->n_hits = 0;
     if (n_reads >= (1ull << 32) - 1) { hga_set_error("hga_scan: more than 2^32-2 reads per GPU"); return HGA_E_ARG; }
     HGA_TRY(h->d_row_off.ensure((n_reads + 1) * 8));
     HGA_TRY(h->d_scan_scalars.ensure(sizeof(ScanScalars) + (size_t) h->sm_count * 8 * SCAN_WARPS * 16));   // + the warps' open chunks (chunked launches)
     ScanScalars *d_sc = h->d_scan_scalars.as<ScanScalars>();
-    const uint32_t lead = (uint32_t) (reinterpret_cast<uintptr_t>(d_bases) & 15);   // the kernel loads aligned 16 B pieces: frame = the bases aligned down
+    // the kernel loads aligned 16 B pieces (packed: 4 B words): frame = the bases aligned down; lead = bases between frame and the first base
+    const bool pk = packed != nullptr;
+    const uint32_t frame_bytes = (uint32_t) (reinterpret_cast<uintptr_t>(d_bases) & (pk ? 3 : 15));
+    const uint32_t lead = pk ? 4 * frame_bytes + packed->sub : frame_bytes;
+    const uint64_t per_byte = pk ? 4 : 1;                                          // bases per byte
+    const uint64_t src_bytes = n_bases == 0 ? 0 : pk ? (packed->sub + n_bases + 3) / 4 : n_bases;   // bytes from d_bases / h_bases on
+    const uint64_t n_exc = pk ? packed->n_exc : 0;
     const uint64_t n_tiles = (n_reads == 0 || n_bases == 0) ? 0 : (lead + n_bases + SCAN_TILE - 1) / SCAN_TILE;
     HGA_TRY(h->d_tile_state.ensure((n_tiles + 2) * (8 + 8 + 4)));   // tile directory: tmp offset | final offset | count
     unsigned long long *tile_tmp_off = h->d_tile_state.as<unsigned long long>();
@@ -691,20 +755,30 @@ int hga_scan_run(hga_handle *h, const char *d_bases, const uint64_t *d_read_off,
 
     ScanParams p;
     memset(&p, 0, sizeof(p));
-    p.frame = d_bases - lead; p.lead = lead; p.n_bases = n_bases; p.read_off = d_read_off; p.n_reads = n_reads;
+    p.frame = d_bases - frame_bytes; p.lead = lead; p.n_bases = n_bases; p.read_off = d_read_off; p.n_reads = n_reads;
     p.t = h->table;
     p.row_off = h->d_row_off.as<uint64_t>();
     p.tile_dir = h->d_tile_dir.as<uint2>();
     p.tile_tmp_off = tile_tmp_off; p.tile_cnt = tile_cnt;
     p.scalars = d_sc;
     if (const char *e = getenv("HGA_SCAN_DIAG")) p.diag = atoi(e);
+    unsigned long long *exc_dir = nullptr;
+    const bool check = pk && packed->check;
+    if (n_exc || check) {                                                          // run directory: n_tiles entries + the check flag
+        HGA_TRY(h->d_exc_dir.ensure((n_tiles + 1) * 8));
+        exc_dir = h->d_exc_dir.as<unsigned long long>();
+    }
+    if (n_exc) {
+        p.exc_start = packed->d_exc_start; p.exc_end = packed->d_exc_end; p.n_exc = n_exc; p.exc_dir = exc_dir;
+    }
 
     int occ = 0;
-    HGA_CUDA(cudaFuncSetAttribute(scan_kernel(), cudaFuncAttributeMaxDynamicSharedMemorySize, (int) scan_smem_bytes()));
-    HGA_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, scan_kernel(), SCAN_THREADS, scan_smem_bytes()));
+    HGA_CUDA(cudaFuncSetAttribute(scan_kernel(pk), cudaFuncAttributeMaxDynamicSharedMemorySize, (int) scan_smem_bytes(pk)));
+    HGA_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, scan_kernel(pk), SCAN_THREADS, scan_smem_bytes(pk)));
     if (occ < 1) occ = 1;
     const int grid_full = (int) std::min<uint64_t>((uint64_t) h->sm_count * occ, std::max<uint64_t>((n_tiles + SCAN_WARPS - 1) / SCAN_WARPS, 1));
 
+    auto launch_scan_pk = [&](const ScanParams &lp, int grid) { return launch_scan(h, lp, grid, pk); };
     StageTimer timer(h, &h->metrics.scan_ms);
     ScanScalars sc;
     memset(&sc, 0, sizeof(sc));
@@ -726,9 +800,32 @@ int hga_scan_run(hga_handle *h, const char *d_bases, const uint64_t *d_read_off,
     if (const char *e = getenv("HGA_SCAN_CHUNK_MB")) chunk_mb = std::max(1, atoi(e));
     const uint64_t chunk_tiles = (chunk_mb << 20) / SCAN_TILE;
     const bool pipelined = h_bases != nullptr && n_tiles > 2 * chunk_tiles && h->copy_stream != nullptr;
+    // the host entry of a packed scan copies its runs with the bases (pipelined: with the first chunk)
+    auto copy_runs = [&](cudaStream_t st) -> int {
+        if (!pk || !packed->h_exc_start || !n_exc) return HGA_OK;
+        HGA_CUDA(cudaMemcpyAsync(const_cast<uint64_t *>(packed->d_exc_start), packed->h_exc_start, n_exc * 8, cudaMemcpyHostToDevice, st));
+        HGA_CUDA(cudaMemcpyAsync(const_cast<uint64_t *>(packed->d_exc_end), packed->h_exc_end, n_exc * 8, cudaMemcpyHostToDevice, st));
+        return HGA_OK;
+    };
+    auto launch_exc_dir = [&]() -> int {
+        if (check) {
+            HGA_CUDA(cudaMemsetAsync(exc_dir + n_tiles, 0, 8, h->stream));
+            scan_exc_check_kernel<<<(int) std::min<uint64_t>((n_exc + 256) / 256, (uint64_t) h->sm_count * 8), 256, 0, h->stream>>>(d_read_off, p.exc_start, p.exc_end, n_exc,
+                                                                                                                                    n_bases, exc_dir + n_tiles);
+            h->metrics.kernel_launches++;
+        }
+        if (n_exc && n_tiles > 0) {
+            scan_exc_dir_kernel<<<(int) std::min<uint64_t>((n_tiles + 255) / 256, (uint64_t) h->sm_count * 8), 256, 0, h->stream>>>(p.exc_start, p.exc_end, n_exc, n_tiles, lead,
+                                                                                                                                    exc_dir);
+            h->metrics.kernel_launches++;
+        }
+        HGA_CUDA(cudaGetLastError());
+        return HGA_OK;
+    };
     if (h_bases != nullptr && !pipelined && n_bases) {
         StageTimer t(h, &h->metrics.h2d_ms, true);
-        HGA_CUDA(cudaMemcpyAsync(const_cast<char *>(d_bases), h_bases, n_bases, cudaMemcpyHostToDevice, h->stream));
+        HGA_CUDA(cudaMemcpyAsync(const_cast<char *>(d_bases), h_bases, src_bytes, cudaMemcpyHostToDevice, h->stream));
+        HGA_TRY(copy_runs(h->stream));
         t.stop();
     }
     if (n_tiles > 0) {
@@ -737,11 +834,16 @@ int hga_scan_run(hga_handle *h, const char *d_bases, const uint64_t *d_read_off,
         h->metrics.kernel_launches++;
         HGA_CUDA(cudaGetLastError());
     }
+    if (!pipelined) HGA_TRY(launch_exc_dir());
     bool done = false;
     if (pipelined) {
         const uint64_t n_chunks = (n_tiles + chunk_tiles - 1) / chunk_tiles;
         std::vector<cudaEvent_t> landed(n_chunks, nullptr);
-        auto chunk_bytes = [&](uint64_t c, uint64_t &lo, uint64_t &hi) { lo = c * chunk_tiles * SCAN_TILE; hi = std::min<uint64_t>(n_bases, (c + 1) * chunk_tiles * SCAN_TILE); };
+        // chunk c = the bytes of tiles [c * chunk_tiles, (c + 1) * chunk_tiles): a tile reads no base past its own end (the host entries' device buffers
+        // start aligned, so frame and d_bases coincide)
+        auto chunk_bytes = [&](uint64_t c, uint64_t &lo, uint64_t &hi) {
+            lo = c * chunk_tiles * SCAN_TILE / per_byte; hi = std::min<uint64_t>(src_bytes, (c + 1) * chunk_tiles * SCAN_TILE / per_byte);
+        };
         cudaEvent_t ev_begin = nullptr, ev_end = nullptr;
         HGA_CUDA(cudaEventCreate(&ev_begin)); HGA_CUDA(cudaEventCreate(&ev_end));
         HGA_CUDA(cudaEventRecord(ev_begin, h->stream));
@@ -750,18 +852,20 @@ int hga_scan_run(hga_handle *h, const char *d_bases, const uint64_t *d_read_off,
             uint64_t lo, hi;
             chunk_bytes(c, lo, hi);
             HGA_CUDA(cudaMemcpyAsync(const_cast<char *>(d_bases) + lo, h_bases + lo, hi - lo, cudaMemcpyHostToDevice, h->copy_stream));
+            if (c == 0) HGA_TRY(copy_runs(h->copy_stream));
             HGA_CUDA(cudaEventCreateWithFlags(&landed[c], cudaEventDisableTiming));
             HGA_CUDA(cudaEventRecord(landed[c], h->copy_stream));
         }
         HGA_CUDA(cudaEventRecord(ev_end, h->copy_stream));
         // capacity from a count-only sample of the first chunk (1 tile in 16)
         HGA_CUDA(cudaStreamWaitEvent(h->stream, landed[0], 0));
+        HGA_TRY(launch_exc_dir());
         {
             const uint64_t stride = 16, n_sample = (chunk_tiles + stride - 1) / stride;
             HGA_CUDA(cudaMemsetAsync(d_sc, 0, sizeof(ScanScalars), h->stream));
             ScanParams ps = p;
             ps.tile_stride = stride; ps.n_tiles = n_sample; ps.tile_begin = 0; ps.capacity = 0;
-            HGA_TRY(launch_scan(h, ps, (int) std::min<uint64_t>((uint64_t) h->sm_count * occ, (n_sample + SCAN_WARPS - 1) / SCAN_WARPS)));
+            HGA_TRY(launch_scan_pk(ps, (int) std::min<uint64_t>((uint64_t) h->sm_count * occ, (n_sample + SCAN_WARPS - 1) / SCAN_WARPS)));
             HGA_CUDA(cudaMemcpyAsync(&sc, d_sc, sizeof(sc), cudaMemcpyDeviceToHost, h->stream));
             HGA_CUDA(cudaStreamSynchronize(h->stream));
             const double est = (double) sc.total * (double) n_tiles / (double) n_sample;
@@ -777,7 +881,7 @@ int hga_scan_run(hga_handle *h, const char *d_bases, const uint64_t *d_read_off,
             HGA_CUDA(cudaStreamWaitEvent(h->stream, landed[c], 0));
             p.tile_begin = c * chunk_tiles; p.n_tiles = std::min<uint64_t>(chunk_tiles, n_tiles - p.tile_begin);
             HGA_CUDA(cudaMemsetAsync(&d_sc->ticket, 0, 8, h->stream));
-            HGA_TRY(launch_scan(h, p, (int) std::min<uint64_t>((uint64_t) h->sm_count * occ, (p.n_tiles + SCAN_WARPS - 1) / SCAN_WARPS)));
+            HGA_TRY(launch_scan_pk(p, (int) std::min<uint64_t>((uint64_t) h->sm_count * occ, (p.n_tiles + SCAN_WARPS - 1) / SCAN_WARPS)));
         }
         HGA_CUDA(cudaMemcpyAsync(&sc, d_sc, sizeof(sc), cudaMemcpyDeviceToHost, h->stream));
         HGA_CUDA(cudaStreamSynchronize(h->stream));
@@ -807,7 +911,7 @@ int hga_scan_run(hga_handle *h, const char *d_bases, const uint64_t *d_read_off,
             ScanParams ps = p;
             ps.tile_stride = stride; ps.n_tiles = n_sample; ps.capacity = 0;
             const int grid_s = (int) std::min<uint64_t>((uint64_t) h->sm_count * occ, (n_sample + SCAN_WARPS - 1) / SCAN_WARPS);
-            HGA_TRY(launch_scan(h, ps, grid_s));
+            HGA_TRY(launch_scan_pk(ps, grid_s));
             HGA_CUDA(cudaMemcpyAsync(&sc, d_sc, sizeof(sc), cudaMemcpyDeviceToHost, h->stream));
             HGA_CUDA(cudaStreamSynchronize(h->stream));
             const double est = (double) sc.total * (double) n_tiles / (double) n_sample;
@@ -821,7 +925,7 @@ int hga_scan_run(hga_handle *h, const char *d_bases, const uint64_t *d_read_off,
         p.out_slot = h->d_sort_a.as<uint32_t>(); p.out_pos = h->d_pos_tmp.as<uint32_t>();
         p.capacity = capacity; p.n_tiles = n_tiles; p.tile_begin = 0; p.tile_stride = 0; p.chunk = SCAN_CHUNK;
         HGA_CUDA(cudaMemsetAsync(d_sc, 0, sizeof(ScanScalars), h->stream));
-        HGA_TRY(launch_scan(h, p, grid_full));
+        HGA_TRY(launch_scan_pk(p, grid_full));
         HGA_CUDA(cudaMemcpyAsync(&sc, d_sc, sizeof(sc), cudaMemcpyDeviceToHost, h->stream));
         HGA_CUDA(cudaStreamSynchronize(h->stream));
         E = sc.total;
@@ -831,6 +935,16 @@ int hga_scan_run(hga_handle *h, const char *d_bases, const uint64_t *d_read_off,
         h->metrics.scan_retries++;
     }
 
+    if (check) {                                                                   // the check ran before the scan; its flag is read now
+        unsigned long long bad = 0;
+        HGA_CUDA(cudaMemcpyAsync(&bad, exc_dir + n_tiles, 8, cudaMemcpyDeviceToHost, h->stream));
+        HGA_CUDA(cudaStreamSynchronize(h->stream));
+        if (bad) {
+            hga_set_error("hga_scan_packed_device: read_off[0] must be 0 and the exception runs non-empty, sorted, non-overlapping and inside [0, %llu)",
+                          (unsigned long long) n_bases);
+            return HGA_E_ARG;
+        }
+    }
     HGA_TRY(h->d_hit_slot.ensure((E + 1) * 4));
     if (n_tiles > 0) {
         size_t tmp_bytes = 0;

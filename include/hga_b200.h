@@ -7,6 +7,7 @@
  *   hga_create           <- load_text_file_kmers' set + KmerIndex           read_clustering.cpp:18-33,
  *                                                                           clustering/ReadClusteringEngine.cpp:237-241
  *   hga_scan[_device]    <- construct_indices, per-read half                clustering/ReadClusteringEngine.cpp:246-277
+ *   hga_scan_packed[_device]   the same from 2-bit packed bases (hga_host_pack_bases packs on the host)
  *                           (KmerIterator semantics: common/KmerIterator.cpp:23-76)
  *   hga_build_index      <- construct_indices, kmer_component_index half    clustering/ReadClusteringEngine.cpp:262-269,282-284
  *   hga_pair_count       <- get_connections / get_all_connections           clustering/ReadClusteringEngine.cpp:301-339
@@ -84,6 +85,27 @@ int hga_set_stream(hga_handle *h, void *cuda_stream);
 int hga_scan(hga_handle *h, const char *bases, const uint64_t *read_off, uint64_t n_reads, uint32_t read_id_base);
 int hga_scan_device(hga_handle *h, const char *d_bases, const uint64_t *d_read_off, uint64_t n_reads, uint64_t n_bases,
                     uint32_t read_id_base);
+
+/* Packed bases: the same scan from 2-bit codes, a quarter of the bytes on the wire and in HBM. Results (hits and every later stage) are
+ * identical to an ASCII scan of the same bytes.
+ *   codes      : A0 C1 G2 T3, four bases per byte, the first base in the most significant bits: base i of a buffer is
+ *                (packed[i >> 2] >> (6 - 2 * (i & 3))) & 3
+ *   exceptions : every byte other than uppercase A C G T (lowercase, N, '\r', ...) has code 0 on BOTH strands in the reference, which two
+ *                bits cannot express. Such bases travel as half-open runs [exc_start[j], exc_end[j]): sorted, non-overlapping,
+ *                non-empty, in the coordinates of read_off. The packer writes code 0 under a run; the scan ignores the codes there.
+ * hga_host_pack_bases: host arithmetic, no GPU. Packs n_bases ASCII bytes; packed needs (n_bases + 3) / 4 bytes. Writes the maximal
+ *   exception runs of the whole stream. If more than exc_capacity runs are needed: HGA_E_ARG and *n_exc = the number needed (retry with
+ *   that capacity). threads <= 0: automatic. */
+int hga_host_pack_bases(const char *bases, uint64_t n_bases, uint8_t *packed, uint64_t *exc_start, uint64_t *exc_end,
+                        uint64_t exc_capacity, uint64_t *n_exc, int threads);
+/* The read set = bases first_base + read_off[0 .. n_reads] of `packed` (read_off[0] == 0, the same rules as for ASCII), so a slice of
+ * a larger packed buffer is scanned in place; the exception runs are relative to first_base and lie inside [0, read_off[n_reads]).
+ * The host entry copies only the bytes that hold the read set and checks read_off and the runs (HGA_E_ARG with a message). The device
+ * entry takes device pointers (d_packed at any byte address) and checks read_off[0] and the runs on the GPU: HGA_E_ARG, no hits. */
+int hga_scan_packed(hga_handle *h, const uint8_t *packed, uint64_t first_base, const uint64_t *read_off, uint64_t n_reads,
+                    const uint64_t *exc_start, const uint64_t *exc_end, uint64_t n_exc, uint32_t read_id_base);
+int hga_scan_packed_device(hga_handle *h, const uint8_t *d_packed, uint64_t first_base, const uint64_t *d_read_off, uint64_t n_reads,
+                           uint64_t n_bases, const uint64_t *d_exc_start, const uint64_t *d_exc_end, uint64_t n_exc, uint32_t read_id_base);
 
 typedef struct {
     uint64_t n_reads;          /* rows scanned */

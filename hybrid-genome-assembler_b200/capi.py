@@ -67,8 +67,8 @@ class Metrics(C.Structure):
 
 # every symbol include/hga_b200.h declares (tests check the .so exports exactly these)
 EXPORTS = ["hga_last_error", "hga_version", "hga_device_count", "hga_init", "hga_host_alloc", "hga_host_free", "hga_create", "hga_destroy", "hga_set_stream",
-           "hga_scan", "hga_scan_device", "hga_host_pack_bases", "hga_scan_packed", "hga_scan_packed_device", "hga_get_hits", "hga_build_index", "hga_get_index", "hga_pair_count", "hga_get_pairs", "hga_select_edges",
-           "hga_get_selection", "hga_components", "hga_get_components", "hga_enrich", "hga_enrich_ex", "hga_enrich_full", "hga_get_tail_block", "hga_count_kmers", "hga_free_kmer_counts", "hga_host_sdk_merge", "hga_host_sdk_specificity", "hga_host_sdk_select", "hga_get_enrichment", "hga_get_purged_index", "hga_get_core_kmers", "hga_spectral_clustering", "hga_host_tail_connections", "hga_host_sym_eigen",
+           "hga_scan", "hga_scan_device", "hga_host_pack_bases", "hga_host_pack_bases_folded", "hga_scan_packed", "hga_scan_packed_device", "hga_get_hits", "hga_build_index", "hga_get_index", "hga_pair_count", "hga_get_pairs", "hga_select_edges",
+           "hga_get_selection", "hga_components", "hga_get_components", "hga_enrich", "hga_enrich_ex", "hga_enrich_full", "hga_get_tail_block", "hga_count_kmers", "hga_count_kmers_packed", "hga_free_kmer_counts", "hga_host_sdk_merge", "hga_host_sdk_specificity", "hga_host_sdk_select", "hga_get_enrichment", "hga_get_purged_index", "hga_get_core_kmers", "hga_spectral_clustering", "hga_host_tail_connections", "hga_host_sym_eigen",
            "hga_metrics", "hga_comm_unique_id", "hga_comm_init", "hga_comm_gather_root"]
 
 
@@ -93,6 +93,7 @@ def load_library():
         lib.hga_scan.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint32]
         lib.hga_scan_device.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint32]
         lib.hga_host_pack_bases.argtypes = [C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64), C.c_int]
+        lib.hga_host_pack_bases_folded.argtypes = lib.hga_host_pack_bases.argtypes
         lib.hga_scan_packed.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint32]
         lib.hga_scan_packed_device.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64, C.c_uint64, C.c_void_p, C.c_void_p, C.c_uint64,
                                                C.c_uint32]
@@ -143,19 +144,22 @@ def _host_bytes(bases):
     return b, C.cast(C.c_char_p(b), C.c_void_p), len(b)
 
 
-def pack_bases(bases, threads=0, capacity=64):
+def pack_bases(bases, threads=0, capacity=64, fold_case=False):
     """hga_host_pack_bases: ASCII bases -> (packed uint8[(n + 3) // 4], exc_start uint64[], exc_end uint64[]), the input of Handle.scan_packed.
     Codes A0 C1 G2 T3, four bases per byte, first base in the most significant bits; every byte other than uppercase ACGT is code 0 under
-    a maximal exception run [start, end). Starts with `capacity` runs and retries once with the exact count."""
+    a maximal exception run [start, end). Starts with `capacity` runs and retries once with the exact count.
+    fold_case=True (hga_host_pack_bases_folded): the case-folded packing count_kmers_packed takes; lowercase acgt are packed as their
+    bases and only bytes outside ACGTacgt are exceptions."""
     lib = load_library()
+    pack = lib.hga_host_pack_bases_folded if fold_case else lib.hga_host_pack_bases
     keep, ptr, n = _host_bytes(bases)
     packed = np.zeros((n + 3) // 4, dtype=np.uint8)
     n_exc = C.c_uint64()
     while True:
         cap = max(int(capacity), 1)
         st = np.zeros(cap, dtype=np.uint64); en = np.zeros(cap, dtype=np.uint64)
-        rc = lib.hga_host_pack_bases(ptr, n, packed.ctypes.data_as(C.c_void_p), st.ctypes.data_as(C.c_void_p), en.ctypes.data_as(C.c_void_p), cap,
-                                     C.byref(n_exc), int(threads))
+        rc = pack(ptr, n, packed.ctypes.data_as(C.c_void_p), st.ctypes.data_as(C.c_void_p), en.ctypes.data_as(C.c_void_p), cap, C.byref(n_exc),
+                  int(threads))
         if rc == 2 and n_exc.value > cap:
             capacity = n_exc.value
             continue
@@ -207,6 +211,28 @@ def count_kmers(bases, read_off, k, min_count=2, device=0):
     ro = np.ascontiguousarray(read_off, dtype=np.uint64)
     out = _KmerCounts()
     _check(lib.hga_count_kmers(int(device), int(k), bytes(bases), ro.ctypes.data_as(C.c_void_p), ro.shape[0] - 1, int(min_count), C.byref(out)))
+    try:
+        return _arr(out.kmer, out.n, np.uint64), _arr(out.count, out.n, np.uint32)
+    finally:
+        lib.hga_free_kmer_counts(C.byref(out))
+
+
+def count_kmers_packed(packed, read_off, exc_start, exc_end, k, min_count=2, first_base=0, device=0):
+    """hga_count_kmers_packed: count_kmers from the case-folded packing (pack_bases(..., fold_case=True)). The read set is bases
+    first_base + read_off[..] of `packed` (read_off[0] == 0); exc_start / exc_end are the exception runs relative to first_base. Returns
+    what count_kmers returns on the ASCII bytes."""
+    lib = load_library()
+    lib.hga_count_kmers_packed.argtypes = [C.c_int, C.c_int, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint32,
+                                           C.POINTER(_KmerCounts)]
+    lib.hga_free_kmer_counts.argtypes = [C.POINTER(_KmerCounts)]
+    lib.hga_free_kmer_counts.restype = None
+    keep, ptr, _ = _host_bytes(packed)
+    ro = np.ascontiguousarray(read_off, dtype=np.uint64)
+    st = np.ascontiguousarray(exc_start, dtype=np.uint64); en = np.ascontiguousarray(exc_end, dtype=np.uint64)
+    out = _KmerCounts()
+    _check(lib.hga_count_kmers_packed(int(device), int(k), ptr, int(first_base), ro.ctypes.data_as(C.c_void_p), ro.shape[0] - 1, st.ctypes.data_as(C.c_void_p),
+                                      en.ctypes.data_as(C.c_void_p), st.shape[0], int(min_count), C.byref(out)))
+    del keep
     try:
         return _arr(out.kmer, out.n, np.uint64), _arr(out.count, out.n, np.uint32)
     finally:

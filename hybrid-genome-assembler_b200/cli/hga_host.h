@@ -187,7 +187,7 @@ struct MetaData {
 // load_meta_data, SequenceRecordIterator.cpp:31-71, once for the records). Phase 1 (sequential, memchr) finds the lines and
 // applies the record rules; phase 2 writes the sequences into one contiguous buffer with several threads: the ASCII bytes (what
 // hga_scan and hga_count_kmers take) or, with `packed`, the 2-bit codes and exception runs of hga_scan_packed, a quarter of the
-// bytes, written straight from the mappings. The buffer is 2 MB aligned and advised MADV_HUGEPAGE: first-touch page faults, not
+// bytes, written straight from the mappings; `packed` with `fold_case`: the case-folded packing of hga_count_kmers_packed. The buffer is 2 MB aligned and advised MADV_HUGEPAGE: first-touch page faults, not
 // memcpy, are what bounds the copy (measured on 1.2 GB: 1.17 s single thread with 4 KB pages, 0.29 s with huge pages and 8 threads).
 // Headers, sequences and qualities stay views into the mappings.
 struct SequenceRecords {
@@ -198,7 +198,7 @@ struct SequenceRecords {
     MetaData meta;
     char *bases_data = nullptr;          // ASCII mode: sequences back to back
     uint8_t *packed_data = nullptr;      // packed mode: the same stream, 2-bit codes, (bases_size + 3) / 4 bytes
-    std::vector<uint64_t> exc_start, exc_end;   // packed mode: maximal runs of bytes other than A C G T, stream positions
+    std::vector<uint64_t> exc_start, exc_end;   // packed mode: maximal runs of bytes other than A C G T (folded: A C G T a c g t), stream positions
     uint64_t bases_size = 0;
     std::vector<uint64_t> seq_off;       // n_reads + 1
     std::vector<View> header_v, quality_v, seq_v;
@@ -227,7 +227,8 @@ struct SequenceRecords {
     }
 
     // threads <= 0: automatic (one thread below 8 MB of bases)
-    explicit SequenceRecords(const std::vector<std::string> &read_paths, int threads = 0, bool packed = false) : paths(read_paths), file_meta(read_paths.size()) {
+    explicit SequenceRecords(const std::vector<std::string> &read_paths, int threads = 0, bool packed = false, bool fold_case = false)
+        : paths(read_paths), file_meta(read_paths.size()) {
         files.reserve(paths.size());
         int cur = -1, method = 4;
         const char *p = nullptr, *end = nullptr;       // cursor in the current file
@@ -323,7 +324,7 @@ struct SequenceRecords {
         void *buf = aligned_alloc(huge, cap);
         if (!buf) throw std::bad_alloc();
         madvise(buf, cap, MADV_HUGEPAGE);
-        if (packed) { packed_data = (uint8_t *) buf; pack_from_mappings(threads); return; }
+        if (packed) { packed_data = (uint8_t *) buf; pack_from_mappings(threads, fold_case); return; }
         bases_data = (char *) buf;
         int T = threads > 0 ? threads : (int) std::min(16u, std::max(1u, std::thread::hardware_concurrency()));
         if (bases_size < ((uint64_t) 8 << 20)) T = 1;
@@ -350,14 +351,14 @@ struct SequenceRecords {
 private:
     // packed mode of phase 2: thread t packs stream positions [per * t, per * (t + 1)) (per: a multiple of 4, so a thread owns whole
     // bytes) piece by piece from the mappings; the runs of neighbouring threads are joined at the seams
-    void pack_from_mappings(int threads) {
+    void pack_from_mappings(int threads, bool fold_case) {
         const uint64_t n_bytes = (bases_size + 3) / 4;
         int T = threads > 0 ? threads : (bases_size < ((uint64_t) 8 << 20) ? 1 : (int) std::min(16u, std::max(1u, std::thread::hardware_concurrency())));
         T = (int) std::max<uint64_t>(1, std::min<uint64_t>((uint64_t) T, n_bytes));
         const uint64_t per = (n_bytes + T - 1) / T * 4;
         std::vector<hga_pack::Packer> part;
         part.reserve(T);
-        for (int t = 0; t < T; t++) part.emplace_back(packed_data, std::min(bases_size, per * t));
+        for (int t = 0; t < T; t++) part.emplace_back(packed_data, std::min(bases_size, per * t), fold_case);
         auto work = [&](int t) {
             const uint64_t a = std::min(bases_size, per * t), b = std::min(bases_size, per * (t + 1));
             if (a >= b) return;

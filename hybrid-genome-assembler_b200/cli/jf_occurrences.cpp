@@ -5,12 +5,16 @@
 //
 // Same options as jellyfish_occurrences.cpp:22-30 (read_paths, --k-size / -k, --output / -o, --help). Where the reference shells out
 // to jellyfish once per read file (occurrences/run_jellyfish.sh) this program counts the canonical k-mers of every file on the GPU
-// (hga_count_kmers: exact counts, k-mers seen at least twice); the merge of the per-file lists, the specificity table and the
+// (hga_count_kmers_packed: exact counts, k-mers seen at least twice). The reads are packed while they load, in the case-folded 2-bit
+// form (lowercase a c g t are bases, as for jellyfish; other bytes travel as exception runs), so a quarter of the bytes crosses to the
+// GPU; a file is counted in place as a slice of that stream, with its runs clipped to the slice and rebased. The counts equal
+// hga_count_kmers on the ASCII bytes, so every output is unchanged. The merge of the per-file lists, the specificity table and the
 // export of a count range are the reader's host arithmetic (hga_host_sdk_*; JellyfishOccurrenceReader.cpp:63-134). Differences,
 // on purpose: the specificity table is printed as text (the reference pipes it into a Python plot, Plotting.cpp); without -k the k
 // sweep of get_unique_k_length (occurrences/KmerAnalysis.cpp:41-56: k = 11, 13, ... until the number of distinct k-mers changes by
 // less than 10 %) uses EXACT distinct counts instead of a HyperLogLog estimate; the `percent` sampling draws from a generator
 // seeded with --seed (default 0) instead of std::random_device. No GPU, no result: there is no CPU path.
+#include <algorithm>
 #include <cmath>
 #include <cstdint>
 #include <cstdio>
@@ -64,15 +68,27 @@ int main(int argc, char **argv) {
     }
     if (read_paths.empty()) throw std::invalid_argument("You need to specify paths to read files");      // jellyfish_occurrences.cpp:38
 
-    hga_host::SequenceRecords reads(read_paths, threads);
+    hga_host::SequenceRecords reads(read_paths, threads, /*packed=*/true, /*fold_case=*/true);
     std::vector<uint64_t> file_first{0};                       // first read of every file
     for (const auto &m : reads.file_meta) file_first.push_back(file_first.back() + m.records);
+    // reads [lo, hi) counted in place: bases seq_off[lo] .. seq_off[hi] of the packed stream, their runs clipped to them and rebased
+    auto count = [&](int kk, size_t lo, size_t hi, uint32_t min_count, hga_kmer_counts_t *c) {
+        const uint64_t b0 = reads.seq_off[lo], b1 = reads.seq_off[hi];
+        std::vector<uint64_t> off(hi - lo + 1), es, ee;
+        for (size_t i = lo; i <= hi; i++) off[i - lo] = reads.seq_off[i] - b0;
+        for (size_t j = (size_t) (std::upper_bound(reads.exc_end.begin(), reads.exc_end.end(), b0) - reads.exc_end.begin());
+             j < reads.exc_start.size() && reads.exc_start[j] < b1; j++) {
+            es.push_back(std::max(reads.exc_start[j], b0) - b0);
+            ee.push_back(std::min(reads.exc_end[j], b1) - b0);
+        }
+        check(hga_count_kmers_packed(device, kk, reads.packed_data, b0, off.data(), hi - lo, es.data(), ee.data(), es.size(), min_count, c), "hga_count_kmers_packed");
+    };
 
     if (k == 0) {
         // get_unique_k_length (KmerAnalysis.cpp:41-56) with exact distinct counts
         auto distinct = [&](int kk) {
             hga_kmer_counts_t c;
-            check(hga_count_kmers(device, kk, reads.bases_data, reads.seq_off.data(), reads.n_reads(), 1, &c), "hga_count_kmers");
+            count(kk, 0, reads.n_reads(), 1, &c);
             const uint64_t n = c.n;
             hga_free_kmer_counts(&c);
             return (long long) n;
@@ -94,7 +110,7 @@ int main(int argc, char **argv) {
     std::vector<uint32_t> counts;
     for (size_t f = 0; f + 1 < file_first.size(); f++) {
         hga_kmer_counts_t c;
-        check(hga_count_kmers(device, k, reads.bases_data, reads.seq_off.data() + file_first[f], file_first[f + 1] - file_first[f], 2, &c), "hga_count_kmers");
+        count(k, file_first[f], file_first[f + 1], 2, &c);
         kmers.insert(kmers.end(), c.kmer, c.kmer + c.n);
         counts.insert(counts.end(), c.count, c.count + c.n);
         file_off.push_back(kmers.size());

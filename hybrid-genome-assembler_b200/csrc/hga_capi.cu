@@ -205,6 +205,19 @@ static int check_read_off(const char *who, const uint64_t *read_off, uint64_t n_
     return HGA_OK;
 }
 
+// exception runs of a packed host entry: sorted, non-empty, non-overlapping, inside [0, n_bases)
+static int check_exc_runs(const char *who, const uint64_t *exc_start, const uint64_t *exc_end, uint64_t n_exc, uint64_t n_bases) {
+    if (n_exc && (!exc_start || !exc_end)) { hga_set_error("%s: exception runs are NULL", who); return HGA_E_ARG; }
+    for (uint64_t i = 0; i < n_exc; i++) {
+        if (exc_start[i] >= exc_end[i] || exc_end[i] > n_bases || (i && exc_start[i] < exc_end[i - 1])) {
+            hga_set_error("%s: exception run %llu [%llu, %llu) is empty, out of order, overlaps its predecessor or lies outside [0, %llu)", who,
+                          (unsigned long long) i, (unsigned long long) exc_start[i], (unsigned long long) exc_end[i], (unsigned long long) n_bases);
+            return HGA_E_ARG;
+        }
+    }
+    return HGA_OK;
+}
+
 int hga_scan_packed(hga_handle *h, const uint8_t *packed, uint64_t first_base, const uint64_t *read_off, uint64_t n_reads, const uint64_t *exc_start,
                     const uint64_t *exc_end, uint64_t n_exc, uint32_t read_id_base) {
     if (!h) { hga_set_error("NULL handle"); return HGA_E_ARG; }
@@ -213,14 +226,7 @@ int hga_scan_packed(hga_handle *h, const uint8_t *packed, uint64_t first_base, c
     HGA_TRY(check_read_off("hga_scan_packed", read_off, n_reads));
     const uint64_t n_bases = read_off[n_reads];
     if (n_bases && !packed) { hga_set_error("hga_scan_packed: packed is NULL"); return HGA_E_ARG; }
-    if (n_exc && (!exc_start || !exc_end)) { hga_set_error("hga_scan_packed: exception runs are NULL"); return HGA_E_ARG; }
-    for (uint64_t i = 0; i < n_exc; i++) {
-        if (exc_start[i] >= exc_end[i] || exc_end[i] > n_bases || (i && exc_start[i] < exc_end[i - 1])) {
-            hga_set_error("hga_scan_packed: exception run %llu [%llu, %llu) is empty, out of order, overlaps its predecessor or lies outside [0, %llu)",
-                          (unsigned long long) i, (unsigned long long) exc_start[i], (unsigned long long) exc_end[i], (unsigned long long) n_bases);
-            return HGA_E_ARG;
-        }
-    }
+    HGA_TRY(check_exc_runs("hga_scan_packed", exc_start, exc_end, n_exc, n_bases));
     // only the bytes that hold the read set travel; on the device they start at an aligned buffer, first_base % 4 bases into its first byte
     const uint32_t sub = (uint32_t) (first_base & 3);
     const uint64_t n_bytes = n_bases ? (sub + n_bases + 3) / 4 : 0;
@@ -236,6 +242,19 @@ int hga_scan_packed(hga_handle *h, const uint8_t *packed, uint64_t first_base, c
     in.h_exc_start = exc_start; in.h_exc_end = exc_end; in.n_exc = n_exc; in.check = false;
     return hga_scan_run(h, h->d_bases.as<char>(), h->d_read_off.as<uint64_t>(), n_reads, n_bases, n_bytes ? reinterpret_cast<const char *>(packed + first_base / 4) : nullptr,
                         &in);
+}
+
+int hga_count_kmers_packed(int device, int k, const uint8_t *packed, uint64_t first_base, const uint64_t *read_off, uint64_t n_reads, const uint64_t *exc_start,
+                           const uint64_t *exc_end, uint64_t n_exc, uint32_t min_count, hga_kmer_counts_t *out) {
+    if (!out) { hga_set_error("hga_count_kmers_packed: NULL argument"); return HGA_E_ARG; }
+    out->n = 0; out->kmer = nullptr; out->count = nullptr;
+    if (!read_off) { hga_set_error("hga_count_kmers_packed: read_off is NULL"); return HGA_E_ARG; }
+    if (k < 1 || k > 32) { hga_set_error("Kmer size is too big or too small (k = %d)", k); return HGA_E_ARG; }
+    HGA_TRY(check_read_off("hga_count_kmers_packed", read_off, n_reads));
+    const uint64_t n_bases = read_off[n_reads];
+    if (n_bases && !packed) { hga_set_error("hga_count_kmers_packed: packed is NULL"); return HGA_E_ARG; }
+    HGA_TRY(check_exc_runs("hga_count_kmers_packed", exc_start, exc_end, n_exc, n_bases));
+    return hga_count_run("hga_count_kmers_packed", device, k, nullptr, packed, first_base, read_off, n_reads, exc_start, exc_end, n_exc, min_count, out);
 }
 
 int hga_scan_packed_device(hga_handle *h, const uint8_t *d_packed, uint64_t first_base, const uint64_t *d_read_off, uint64_t n_reads, uint64_t n_bases,

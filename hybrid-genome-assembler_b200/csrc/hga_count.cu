@@ -17,9 +17,15 @@
 // runs to the host result; ranges ascend, so the result is sorted without a merge and every k-mer is counted in exactly one pass. A
 // range that overflows the budget is split at its midpoint and redone. HBM-bound by the sort passes of the emitted keys plus one read
 // of the bases per pass.
+// Packed input (hga_count_kmers_packed: the case-folded 2-bit codes, exception runs for the bytes outside ACGTacgt): the same two modes
+// with count_emit_packed_kernel in place of the two emit kernels. A thread owns a span of consecutive window starts; it searches once for
+// its read and once for the first exception run that can touch the span, then rolls the forward and reverse-complement values over the
+// span plus k - 1 bases, reading one 32-bit word per 16 bases and stepping over read ends and runs. Every later step (sort, run-length
+// encode, filter, quantiles, range splitting) is shared with the ASCII input, so the results are the same values in the same order.
 #include "hga_internal.cuh"
 
 #include <algorithm>
+#include <cstdio>
 #include <cstdlib>
 
 #include <cub/device/device_radix_sort.cuh>
@@ -102,38 +108,153 @@ __global__ void count_emit_range_kernel(const char *__restrict__ bases, const ui
     }
 }
 
+// ---- packed input ----------------------------------------------------------------------------------------------------------------
+// Base i of a slice sits at position g = sub + i of the device buffer (which starts at the byte holding the slice's first base): bits
+// 30 - 2 * (g & 15) of 32-bit word g >> 4 once its bytes are swapped (the first base of a byte is in its most significant bits).
+#define COUNT_PACKED_SPAN 32            // window starts per thread where every window is emitted (one pass, key-range passes)
+__device__ __forceinline__ uint32_t count_packed_word(const uint32_t *__restrict__ words, uint64_t w) {
+#ifdef __CUDA_ARCH__
+    return __byte_perm(__ldg(words + w), 0, 0x0123);
+#else
+    return __builtin_bswap32(words[w]);
+#endif
+}
+
+// The rolling state of one thread: push() takes base q and says whether the k bases ending at q form a window to count (all in one
+// read, none under an exception run). rend = the end of read r (the read holding q); [xs, xe) = run x, the first run that ends after q.
+struct CountRoll {
+    const uint32_t *words;
+    const uint64_t *read_off, *exc_start, *exc_end;
+    uint64_t n_exc, q, g, r, rend, x, xs, xe;
+    unsigned long long fwd, rc, mask;
+    uint32_t word;
+    int k, vlen;
+
+    __device__ __forceinline__ void start(const uint32_t *w, uint32_t sub, const uint64_t *ro, uint64_t n_reads, const uint64_t *es, const uint64_t *ee, uint64_t ne, int kk,
+                                          uint64_t p0) {
+        words = w; read_off = ro; exc_start = es; exc_end = ee; n_exc = ne; k = kk; vlen = 0; fwd = rc = 0;
+        mask = k < 32 ? (1ull << (2 * k)) - 1 : ~0ull;
+        uint64_t lo = 0, hi = n_reads;                      // the read that holds p0: the last r with read_off[r] <= p0
+        while (lo < hi) { const uint64_t mid = (lo + hi + 1) >> 1; if (read_off[mid] <= p0) lo = mid; else hi = mid - 1; }
+        r = lo; rend = read_off[r + 1];
+        lo = 0; hi = n_exc;                                 // the first run that ends after p0 (the ends ascend)
+        while (lo < hi) { const uint64_t mid = (lo + hi) >> 1; if (exc_end[mid] <= p0) lo = mid + 1; else hi = mid; }
+        x = lo;
+        xs = x < n_exc ? exc_start[x] : ~0ull; xe = x < n_exc ? exc_end[x] : ~0ull;
+        q = p0; g = sub + p0;
+        word = count_packed_word(words, g >> 4);
+    }
+    // q < read_off[n_reads]
+    __device__ __forceinline__ bool push() {
+        if ((g & 15) == 0) word = count_packed_word(words, g >> 4);
+        const uint32_t c = (word >> (30 - 2 * (uint32_t) (g & 15))) & 3u;
+        if (q == rend) { do rend = read_off[++r + 1]; while (rend == q); vlen = 0; }       // a new read (empty ones skipped)
+        if (q == xe) { x++; xs = x < n_exc ? exc_start[x] : ~0ull; xe = x < n_exc ? exc_end[x] : ~0ull; }   // the next run starts at xe or later
+        fwd = ((fwd << 2) | c) & mask;
+        rc = (rc >> 2) | ((unsigned long long) (3u - c) << (2 * (k - 1)));
+        vlen = q >= xs ? 0 : vlen + 1;
+        q++; g++;
+        return vlen >= k;
+    }
+};
+
+// Window starts [p0, p0 + span) of every span_stride-th span (span: a multiple of COUNT_SPAN), in chunks of COUNT_SPAN windows.
+// RANGE == false (one pass; span_stride 1): out[p] = the key of window p or COUNT_SENTINEL, the layout of count_emit_kernel.
+// RANGE == true: the keys in [key_lo, key_hi), compacted into out as count_emit_range_kernel does (span COUNT_SPAN: the same sample).
+template<bool RANGE>
+__global__ void count_emit_packed_kernel(const uint32_t *__restrict__ words, uint32_t sub, const uint64_t *__restrict__ read_off, uint64_t n_reads,
+                                         const uint64_t *__restrict__ exc_start, const uint64_t *__restrict__ exc_end, uint64_t n_exc, int k, uint64_t n_bases,
+                                         uint32_t span, uint64_t span_stride, unsigned long long key_lo, unsigned long long key_hi,
+                                         unsigned long long *__restrict__ out, uint64_t capacity, unsigned long long *cursor) {
+    const uint64_t n_units = (n_bases + span - 1) / span, n_sel = (n_units + span_stride - 1) / span_stride;
+    const uint64_t threads = (uint64_t) gridDim.x * blockDim.x, rounds = (n_sel + threads - 1) / threads;
+    for (uint64_t round = 0; round < rounds; round++) {                      // the same trip counts for every thread: the warp stays together
+        const uint64_t t = round * threads + blockIdx.x * (uint64_t) blockDim.x + threadIdx.x;
+        const bool live = t < n_sel;
+        const uint64_t p0 = t * span_stride * span;
+        CountRoll roll;
+        if (live) {
+            roll.start(words, sub, read_off, n_reads, exc_start, exc_end, n_exc, k, p0);
+            for (int j = 0; j < k - 1 && roll.q < n_bases; j++) roll.push();      // the first k - 1 bases end no window of the span
+        }
+        for (uint32_t c0 = 0; c0 < span; c0 += COUNT_SPAN) {
+            unsigned long long keys[COUNT_SPAN];
+            #pragma unroll
+            for (int j = 0; j < COUNT_SPAN; j++) {                             // window p0 + c0 + j ends at base roll.q
+                keys[j] = COUNT_SENTINEL;
+                if (live && roll.q < n_bases && roll.push()) keys[j] = roll.fwd < roll.rc ? roll.fwd : roll.rc;
+            }
+            if (!RANGE) {
+                if (live) {
+                    #pragma unroll
+                    for (int j = 0; j < COUNT_SPAN; j++) if (p0 + c0 + j < n_bases) out[p0 + c0 + j] = keys[j];
+                }
+                continue;
+            }
+            uint32_t m = 0;
+            #pragma unroll
+            for (int j = 0; j < COUNT_SPAN; j++) if (keys[j] != COUNT_SENTINEL && keys[j] >= key_lo && keys[j] < key_hi) m |= 1u << j;
+            unsigned long long at;
+#ifdef __CUDA_ARCH__
+            const uint32_t cnt = (uint32_t) __popc(m);
+            const int lane = threadIdx.x & 31;
+            uint32_t incl = cnt;
+            #pragma unroll
+            for (int d = 1; d < 32; d <<= 1) { const uint32_t v = __shfl_up_sync(0xFFFFFFFFu, incl, d); if (lane >= d) incl += v; }
+            unsigned long long base = 0;
+            if (lane == 31 && incl) base = atomicAdd(cursor, (unsigned long long) incl);
+            base = __shfl_sync(0xFFFFFFFFu, base, 31);
+            at = base + incl - cnt;
+#else
+            at = atomicAdd(cursor, (unsigned long long) __builtin_popcount(m));
+#endif
+            #pragma unroll
+            for (int j = 0; j < COUNT_SPAN; j++) if ((m >> j) & 1u) { if (at < capacity) out[at] = keys[j]; at++; }
+        }
+    }
+}
+
 __global__ void count_flag_kernel(const unsigned long long *__restrict__ keys, const uint32_t *__restrict__ cnt, uint64_t n, uint32_t min_count, uint8_t *__restrict__ flag) {
     for (uint64_t i = blockIdx.x * (uint64_t) blockDim.x + threadIdx.x; i < n; i += (uint64_t) gridDim.x * blockDim.x)
         flag[i] = keys[i] != COUNT_SENTINEL && cnt[i] >= min_count;
 }
 
 struct Bufs {
-    DevBuf bases, off, keys, sorted, run_key, run_len, acc_key2, acc_cnt2, tmp, scalars, flag;
-    ~Bufs() { for (DevBuf *b : {&bases, &off, &keys, &sorted, &run_key, &run_len, &acc_key2, &acc_cnt2, &tmp, &scalars, &flag}) b->release(); }
+    DevBuf bases, off, exc, keys, sorted, run_key, run_len, acc_key2, acc_cnt2, tmp, scalars, flag;
+    ~Bufs() { for (DevBuf *b : {&bases, &off, &exc, &keys, &sorted, &run_key, &run_len, &acc_key2, &acc_cnt2, &tmp, &scalars, &flag}) b->release(); }
 };
 
 }  // namespace
 
-extern "C" int hga_count_kmers(int device, int k, const char *bases, const uint64_t *read_off, uint64_t n_reads, uint32_t min_count, hga_kmer_counts_t *out) {
-    if (!out) { hga_set_error("hga_count_kmers: NULL argument"); return HGA_E_ARG; }
-    out->n = 0; out->kmer = nullptr; out->count = nullptr;
-    if (k < 1 || k > 32) { hga_set_error("Kmer size is too big or too small (k = %d)", k); return HGA_E_ARG; }
-    if (n_reads && (!bases || !read_off)) { hga_set_error("hga_count_kmers: NULL argument"); return HGA_E_ARG; }
+int hga_count_run(const char *who, int device, int k, const char *bases, const uint8_t *packed, uint64_t first_base, const uint64_t *read_off,
+                  uint64_t n_reads, const uint64_t *exc_start, const uint64_t *exc_end, uint64_t n_exc, uint32_t min_count, hga_kmer_counts_t *out) {
     int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) { cudaGetLastError(); hga_set_error("hga_count_kmers: no usable CUDA device (this library has no CPU path)"); return HGA_E_CUDA; }
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) { cudaGetLastError(); hga_set_error("%s: no usable CUDA device (this library has no CPU path)", who); return HGA_E_CUDA; }
     HGA_CUDA(cudaSetDevice(device));
     if (n_reads == 0) return HGA_OK;
     const uint64_t base0 = read_off[0], n_bases = read_off[n_reads] - base0;
     if (n_bases == 0) return HGA_OK;
     cudaStream_t st = nullptr;      // legacy default stream: every call below is ordered on it
     Bufs b;
-    HGA_TRY(b.bases.ensure(n_bases + 64));
+    // only the bytes that hold the read set travel; packed, they start at an aligned buffer, first_base % 4 bases into its first byte
+    const uint32_t sub = (uint32_t) (first_base & 3);
+    const uint64_t in_bytes = packed ? (sub + n_bases + 3) / 4 : n_bases;
+    HGA_TRY(b.bases.ensure(in_bytes + 64));
     HGA_TRY(b.off.ensure((n_reads + 1) * 8));
     HGA_TRY(b.scalars.ensure(64));
     std::vector<uint64_t> off(n_reads + 1);
     for (uint64_t i = 0; i <= n_reads; i++) off[i] = read_off[i] - base0;
-    HGA_CUDA(cudaMemcpyAsync(b.bases.p, bases + base0, n_bases, cudaMemcpyHostToDevice, st));
+    HGA_CUDA(cudaMemcpyAsync(b.bases.p, packed ? (const void *) (packed + first_base / 4) : (const void *) (bases + base0), in_bytes, cudaMemcpyHostToDevice, st));
     HGA_CUDA(cudaMemcpyAsync(b.off.p, off.data(), (n_reads + 1) * 8, cudaMemcpyHostToDevice, st));
+    if (packed) {
+        HGA_TRY(b.exc.ensure(n_exc * 16 + 16));
+        if (n_exc) {
+            HGA_CUDA(cudaMemcpyAsync(b.exc.p, exc_start, n_exc * 8, cudaMemcpyHostToDevice, st));
+            HGA_CUDA(cudaMemcpyAsync(b.exc.as<uint64_t>() + n_exc, exc_end, n_exc * 8, cudaMemcpyHostToDevice, st));
+        }
+    }
+    const uint32_t *d_words = b.bases.as<uint32_t>();
+    const uint64_t *d_off = b.off.as<uint64_t>(), *d_xs = b.exc.as<uint64_t>(), *d_xe = d_xs + n_exc;
     unsigned long long *d_scal = b.scalars.as<unsigned long long>();
     // keys per pass (the scratch is ~6 arrays of this many entries); HGA_COUNT_CHUNK overrides it (tests force the multi-pass path on small inputs with it)
     const char *ch_env = getenv("HGA_COUNT_CHUNK");
@@ -189,7 +310,12 @@ extern "C" int hga_count_kmers(int device, int k, const char *bases, const uint6
     if (n_bases <= B) {
         // one pass: a key (or the sentinel) per window start
         HGA_TRY(b.keys.ensure(n_bases * 8));
-        count_emit_kernel<<<grid(n_bases), 256, 0, st>>>(b.bases.as<char>(), b.off.as<uint64_t>(), n_reads, k, 0, n_bases, b.keys.as<unsigned long long>());
+        if (packed)
+            count_emit_packed_kernel<false><<<grid((n_bases + COUNT_PACKED_SPAN - 1) / COUNT_PACKED_SPAN), 256, 0, st>>>(d_words, sub, d_off, n_reads, d_xs, d_xe, n_exc, k, n_bases,
+                                                                                                                    COUNT_PACKED_SPAN, 1, 0ull, COUNT_SENTINEL, b.keys.as<unsigned long long>(),
+                                                                                                                    n_bases, nullptr);
+        else
+            count_emit_kernel<<<grid(n_bases), 256, 0, st>>>(b.bases.as<char>(), b.off.as<uint64_t>(), n_reads, k, 0, n_bases, b.keys.as<unsigned long long>());
         HGA_TRY(finish_pass(n_bases));
     } else {
         // key-range passes. Quantiles of the key distribution from a strided sample of the windows (about 2^24 of them, all of them when the input is small)
@@ -198,8 +324,13 @@ extern "C" int hga_count_kmers(int device, int k, const char *bases, const uint6
         const uint64_t sample_stride = std::max<uint64_t>(1, n_bases / std::min<uint64_t>(B, 1ull << 24));
         const uint64_t sample_cap = std::min<uint64_t>(B, (n_spans + sample_stride - 1) / sample_stride * COUNT_SPAN);
         HGA_CUDA(cudaMemsetAsync(d_scal + 1, 0, 8, st));
-        count_emit_range_kernel<<<grid((n_spans + sample_stride - 1) / sample_stride), 256, 0, st>>>(b.bases.as<char>(), b.off.as<uint64_t>(), n_reads, k, n_bases, 0ull, COUNT_SENTINEL,
-                                                                                                    sample_stride, b.keys.as<unsigned long long>(), sample_cap, d_scal + 1);
+        if (packed)
+            count_emit_packed_kernel<true><<<grid((n_spans + sample_stride - 1) / sample_stride), 256, 0, st>>>(d_words, sub, d_off, n_reads, d_xs, d_xe, n_exc, k, n_bases, COUNT_SPAN,
+                                                                                                           sample_stride, 0ull, COUNT_SENTINEL, b.keys.as<unsigned long long>(),
+                                                                                                           sample_cap, d_scal + 1);
+        else
+            count_emit_range_kernel<<<grid((n_spans + sample_stride - 1) / sample_stride), 256, 0, st>>>(b.bases.as<char>(), b.off.as<uint64_t>(), n_reads, k, n_bases, 0ull, COUNT_SENTINEL,
+                                                                                                        sample_stride, b.keys.as<unsigned long long>(), sample_cap, d_scal + 1);
         unsigned long long n_sample = 0;
         HGA_CUDA(cudaMemcpyAsync(&n_sample, d_scal + 1, 8, cudaMemcpyDeviceToHost, st));
         HGA_CUDA(cudaStreamSynchronize(st));
@@ -220,12 +351,19 @@ extern "C" int hga_count_kmers(int device, int k, const char *bases, const uint6
         }
         // the ranges, ascending; one that overflows the budget is split at its midpoint and redone (a single value that overflows IS its own count)
         std::vector<std::pair<unsigned long long, unsigned long long>> todo;
+        uint64_t passes = 0, splits = 0;
         for (uint64_t r = n_ranges; r-- > 0;) if (cut[r] < cut[r + 1]) todo.push_back({cut[r], cut[r + 1]});
         while (!todo.empty()) {
             const unsigned long long lo = todo.back().first, hi = todo.back().second;
             todo.pop_back();
+            passes++;
             HGA_CUDA(cudaMemsetAsync(d_scal + 1, 0, 8, st));
-            count_emit_range_kernel<<<grid(n_spans), 256, 0, st>>>(b.bases.as<char>(), b.off.as<uint64_t>(), n_reads, k, n_bases, lo, hi, 1, b.keys.as<unsigned long long>(), B, d_scal + 1);
+            if (packed)
+                count_emit_packed_kernel<true><<<grid((n_bases + COUNT_PACKED_SPAN - 1) / COUNT_PACKED_SPAN), 256, 0, st>>>(d_words, sub, d_off, n_reads, d_xs, d_xe, n_exc, k, n_bases,
+                                                                                                                       COUNT_PACKED_SPAN, 1, lo, hi, b.keys.as<unsigned long long>(), B,
+                                                                                                                       d_scal + 1);
+            else
+                count_emit_range_kernel<<<grid(n_spans), 256, 0, st>>>(b.bases.as<char>(), b.off.as<uint64_t>(), n_reads, k, n_bases, lo, hi, 1, b.keys.as<unsigned long long>(), B, d_scal + 1);
             HGA_CUDA(cudaGetLastError());
             unsigned long long m = 0;
             HGA_CUDA(cudaMemcpyAsync(&m, d_scal + 1, 8, cudaMemcpyDeviceToHost, st));
@@ -235,6 +373,7 @@ extern "C" int hga_count_kmers(int device, int k, const char *bases, const uint6
                     if (m >= min_count) { res_k.push_back(lo); res_c.push_back((uint32_t) std::min<unsigned long long>(m, 0xFFFFFFFFull)); }
                     continue;
                 }
+                splits++;
                 const unsigned long long mid = lo + (hi - lo) / 2;
                 todo.push_back({mid, hi});
                 todo.push_back({lo, mid});
@@ -242,14 +381,24 @@ extern "C" int hga_count_kmers(int device, int k, const char *bases, const uint6
             }
             HGA_TRY(finish_pass(m));
         }
+        // HGA_COUNT_STATS=1: how the key range was cut (a split range counts its pass and the passes of its halves)
+        if (getenv("HGA_COUNT_STATS")) fprintf(stderr, "%s: %llu key-range passes (%llu ranges split)\n", who, (unsigned long long) passes, (unsigned long long) splits);
     }
     const uint64_t n_out = res_k.size();
     uint64_t *hk = (uint64_t *) std::malloc((n_out + 1) * 8);
     uint32_t *hc = (uint32_t *) std::malloc((n_out + 1) * 4);
-    if (!hk || !hc) { std::free(hk); std::free(hc); hga_set_error("hga_count_kmers: out of host memory"); return HGA_E_NOMEM; }
+    if (!hk || !hc) { std::free(hk); std::free(hc); hga_set_error("%s: out of host memory", who); return HGA_E_NOMEM; }
     if (n_out) { std::memcpy(hk, res_k.data(), n_out * 8); std::memcpy(hc, res_c.data(), n_out * 4); }
     out->n = n_out; out->kmer = hk; out->count = hc;
     return HGA_OK;
+}
+
+extern "C" int hga_count_kmers(int device, int k, const char *bases, const uint64_t *read_off, uint64_t n_reads, uint32_t min_count, hga_kmer_counts_t *out) {
+    if (!out) { hga_set_error("hga_count_kmers: NULL argument"); return HGA_E_ARG; }
+    out->n = 0; out->kmer = nullptr; out->count = nullptr;
+    if (k < 1 || k > 32) { hga_set_error("Kmer size is too big or too small (k = %d)", k); return HGA_E_ARG; }
+    if (n_reads && (!bases || !read_off)) { hga_set_error("hga_count_kmers: NULL argument"); return HGA_E_ARG; }
+    return hga_count_run("hga_count_kmers", device, k, bases, nullptr, 0, read_off, n_reads, nullptr, nullptr, 0, min_count, out);
 }
 
 extern "C" void hga_free_kmer_counts(hga_kmer_counts_t *c) {

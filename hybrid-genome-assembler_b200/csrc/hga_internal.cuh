@@ -361,6 +361,11 @@ struct ScanPackedInput {
 int hga_scan_run(hga_handle *h, const char *d_bases, const uint64_t *d_read_off, uint64_t n_reads, uint64_t n_bases, const char *h_bases,
                  const ScanPackedInput *packed = nullptr);
 int hga_scan_finish_positions(hga_handle *h);
+// the k-mer count behind hga_count_kmers and hga_count_kmers_packed (csrc/hga_count.cu), arguments already checked.
+// packed == nullptr: ASCII `bases`, read set bases[read_off[0] .. read_off[n_reads]). Otherwise the case-folded packing, bases
+// first_base + read_off[0 .. n_reads] (read_off[0] == 0) and the exception runs relative to first_base.
+int hga_count_run(const char *who, int device, int k, const char *bases, const uint8_t *packed, uint64_t first_base, const uint64_t *read_off,
+                  uint64_t n_reads, const uint64_t *exc_start, const uint64_t *exc_end, uint64_t n_exc, uint32_t min_count, hga_kmer_counts_t *out);
 int hga_index_run(hga_handle *h);
 int hga_build_lists(hga_handle *h, const uint32_t *d_keys, const uint64_t *d_row_off, uint64_t n_rows, uint64_t E, uint32_t n_keys);
 int hga_pairs_run(hga_handle *h, uint32_t min_score, const uint32_t *pivots, uint64_t n_pivots);

@@ -18,6 +18,7 @@
  *   hga_enrich           <- merge_components(scaffolds), get_connections(cores, min), union_find(conns, cores, 2, -1),
  *                           merge_components, get_component_ids             clustering/ReadClusteringEngine.cpp:349-422, :764, :785-794
  *   hga_count_kmers / hga_host_sdk_* <- jellyfish + JellyfishOccurrenceReader (the --kmers file)          occurrences/ (all files), jellyfish_occurrences.cpp
+ *   hga_count_kmers_packed     the same count from case-folded 2-bit packed bases (hga_host_pack_bases_folded packs on the host)
  *   hga_enrich_full      <- the same plus the tail / spectral block in between (second merge_components)     :764-794
  *
  * Conventions
@@ -98,6 +99,10 @@ int hga_scan_device(hga_handle *h, const char *d_bases, const uint64_t *d_read_o
  *   that capacity). threads <= 0: automatic. */
 int hga_host_pack_bases(const char *bases, uint64_t n_bases, uint8_t *packed, uint64_t *exc_start, uint64_t *exc_end,
                         uint64_t exc_capacity, uint64_t *n_exc, int threads);
+/* hga_host_pack_bases_folded: the same with the case-folded packing that hga_count_kmers_packed takes (jellyfish's rule): lowercase
+ *   a c g t are packed as their bases, and only bytes outside A C G T a c g t are covered by exception runs. */
+int hga_host_pack_bases_folded(const char *bases, uint64_t n_bases, uint8_t *packed, uint64_t *exc_start, uint64_t *exc_end,
+                               uint64_t exc_capacity, uint64_t *n_exc, int threads);
 /* The read set = bases first_base + read_off[0 .. n_reads] of `packed` (read_off[0] == 0, the same rules as for ASCII), so a slice of
  * a larger packed buffer is scanned in place; the exception runs are relative to first_base and lie inside [0, read_off[n_reads]).
  * The host entry copies only the bytes that hold the read set and checks read_off and the runs (HGA_E_ARG with a message). The device
@@ -270,6 +275,12 @@ typedef struct {
     const uint32_t *count;
 } hga_kmer_counts_t;
 int hga_count_kmers(int device, int k, const char *bases, const uint64_t *read_off, uint64_t n_reads, uint32_t min_count, hga_kmer_counts_t *out);
+/* hga_count_kmers_packed: the same counts from the case-folded packing of hga_host_pack_bases_folded, identical to hga_count_kmers on
+ *   the ASCII bytes (same k-mers, counts and order). The read set and the runs follow hga_scan_packed's rules: bases first_base +
+ *   read_off[0 .. n_reads] of `packed` with read_off[0] == 0, runs relative to first_base, sorted, non-empty, non-overlapping, inside
+ *   [0, read_off[n_reads]). Only the bytes that hold the read set are copied. Bad input: HGA_E_ARG with a message. */
+int hga_count_kmers_packed(int device, int k, const uint8_t *packed, uint64_t first_base, const uint64_t *read_off, uint64_t n_reads,
+                           const uint64_t *exc_start, const uint64_t *exc_end, uint64_t n_exc, uint32_t min_count, hga_kmer_counts_t *out);
 void hga_free_kmer_counts(hga_kmer_counts_t *c);
 int hga_host_sdk_merge(int n_files, const uint64_t *file_off, const uint64_t *kmer, const uint32_t *count, uint64_t *out_kmer, uint32_t *out_total,
                        uint32_t *out_max, uint32_t *out_files, uint64_t *out_n);

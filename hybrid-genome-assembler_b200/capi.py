@@ -68,7 +68,7 @@ class Metrics(C.Structure):
 # every symbol include/hga_b200.h declares (tests check the .so exports exactly these)
 EXPORTS = ["hga_last_error", "hga_version", "hga_device_count", "hga_init", "hga_host_alloc", "hga_host_free", "hga_create", "hga_destroy", "hga_set_stream",
            "hga_scan", "hga_scan_device", "hga_host_pack_bases", "hga_host_pack_bases_folded", "hga_scan_packed", "hga_scan_packed_device", "hga_get_hits", "hga_build_index", "hga_get_index", "hga_pair_count", "hga_get_pairs", "hga_select_edges",
-           "hga_get_selection", "hga_components", "hga_get_components", "hga_enrich", "hga_enrich_ex", "hga_enrich_full", "hga_get_tail_block", "hga_count_kmers", "hga_count_kmers_packed", "hga_free_kmer_counts", "hga_host_sdk_merge", "hga_host_sdk_specificity", "hga_host_sdk_select", "hga_get_enrichment", "hga_get_purged_index", "hga_get_core_kmers", "hga_spectral_clustering", "hga_host_tail_connections", "hga_host_sym_eigen",
+           "hga_get_selection", "hga_components", "hga_get_components", "hga_enrich", "hga_enrich_ex", "hga_enrich_full", "hga_get_tail_block", "hga_count_kmers", "hga_count_kmers_packed", "hga_count_spectrum", "hga_count_spectrum_packed", "hga_free_kmer_counts", "hga_host_sdk_merge", "hga_host_sdk_specificity", "hga_host_sdk_select", "hga_get_enrichment", "hga_get_purged_index", "hga_get_core_kmers", "hga_spectral_clustering", "hga_host_tail_connections", "hga_host_sym_eigen",
            "hga_metrics", "hga_comm_unique_id", "hga_comm_init", "hga_comm_gather_root"]
 
 
@@ -237,6 +237,39 @@ def count_kmers_packed(packed, read_off, exc_start, exc_end, k, min_count=2, fir
         return _arr(out.kmer, out.n, np.uint64), _arr(out.count, out.n, np.uint32)
     finally:
         lib.hga_free_kmer_counts(C.byref(out))
+
+
+class _KmerSpectrum(C.Structure):
+    _fields_ = [("n_windows", C.c_uint64), ("n_distinct", C.c_uint64), ("max_count", C.c_uint64)]
+
+
+def count_spectrum(bases, read_off, k, n_bins=0, device=0):
+    """hga_count_spectrum: the k-mer spectrum of count_kmers(.., min_count=1) without materialising the k-mers. Returns (hist, n_windows,
+    n_distinct, max_count): hist[c - 1] = distinct k-mers seen exactly c times, the last of the n_bins entries those seen n_bins times or more."""
+    lib = load_library()
+    lib.hga_count_spectrum.argtypes = [C.c_int, C.c_int, C.c_char_p, C.c_void_p, C.c_uint64, C.c_uint32, C.c_void_p, C.POINTER(_KmerSpectrum)]
+    ro = np.ascontiguousarray(read_off, dtype=np.uint64)
+    hist = np.zeros(int(n_bins), dtype=np.uint64)
+    out = _KmerSpectrum()
+    _check(lib.hga_count_spectrum(int(device), int(k), bytes(bases), ro.ctypes.data_as(C.c_void_p), ro.shape[0] - 1, int(n_bins), hist.ctypes.data_as(C.c_void_p),
+                                  C.byref(out)))
+    return hist, out.n_windows, out.n_distinct, out.max_count
+
+
+def count_spectrum_packed(packed, read_off, exc_start, exc_end, k, n_bins=0, first_base=0, device=0):
+    """hga_count_spectrum_packed: count_spectrum from the case-folded packing, with the read set and runs of count_kmers_packed"""
+    lib = load_library()
+    lib.hga_count_spectrum_packed.argtypes = [C.c_int, C.c_int, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint32,
+                                              C.c_void_p, C.POINTER(_KmerSpectrum)]
+    keep, ptr, _ = _host_bytes(packed)
+    ro = np.ascontiguousarray(read_off, dtype=np.uint64)
+    st = np.ascontiguousarray(exc_start, dtype=np.uint64); en = np.ascontiguousarray(exc_end, dtype=np.uint64)
+    hist = np.zeros(int(n_bins), dtype=np.uint64)
+    out = _KmerSpectrum()
+    _check(lib.hga_count_spectrum_packed(int(device), int(k), ptr, int(first_base), ro.ctypes.data_as(C.c_void_p), ro.shape[0] - 1, st.ctypes.data_as(C.c_void_p),
+                                         en.ctypes.data_as(C.c_void_p), st.shape[0], int(n_bins), hist.ctypes.data_as(C.c_void_p), C.byref(out)))
+    del keep
+    return hist, out.n_windows, out.n_distinct, out.max_count
 
 
 def sdk_merge(per_file):

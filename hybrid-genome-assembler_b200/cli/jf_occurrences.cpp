@@ -12,7 +12,8 @@
 // export of a count range are the reader's host arithmetic (hga_host_sdk_*; JellyfishOccurrenceReader.cpp:63-134). Differences,
 // on purpose: the specificity table is printed as text (the reference pipes it into a Python plot, Plotting.cpp); without -k the k
 // sweep of get_unique_k_length (occurrences/KmerAnalysis.cpp:41-56: k = 11, 13, ... until the number of distinct k-mers changes by
-// less than 10 %) uses EXACT distinct counts instead of a HyperLogLog estimate; the `percent` sampling draws from a generator
+// less than 10 %) uses EXACT distinct counts instead of a HyperLogLog estimate (hga_count_spectrum_packed: the distinct count of every
+// k of the sweep is computed on the GPU, so host memory does not grow with the number of distinct k-mers); the `percent` sampling draws from a generator
 // seeded with --seed (default 0) instead of std::random_device. No GPU, no result: there is no CPU path.
 #include <algorithm>
 #include <cmath>
@@ -71,27 +72,35 @@ int main(int argc, char **argv) {
     hga_host::SequenceRecords reads(read_paths, threads, /*packed=*/true, /*fold_case=*/true);
     std::vector<uint64_t> file_first{0};                       // first read of every file
     for (const auto &m : reads.file_meta) file_first.push_back(file_first.back() + m.records);
-    // reads [lo, hi) counted in place: bases seq_off[lo] .. seq_off[hi] of the packed stream, their runs clipped to them and rebased
-    auto count = [&](int kk, size_t lo, size_t hi, uint32_t min_count, hga_kmer_counts_t *c) {
-        const uint64_t b0 = reads.seq_off[lo], b1 = reads.seq_off[hi];
-        std::vector<uint64_t> off(hi - lo + 1), es, ee;
-        for (size_t i = lo; i <= hi; i++) off[i - lo] = reads.seq_off[i] - b0;
-        for (size_t j = (size_t) (std::upper_bound(reads.exc_end.begin(), reads.exc_end.end(), b0) - reads.exc_end.begin());
+    // reads [lo, hi) in place: bases seq_off[lo] .. seq_off[hi] of the packed stream, their runs clipped to them and rebased
+    struct Slice { uint64_t b0; std::vector<uint64_t> off, es, ee; };
+    auto slice = [&](size_t lo, size_t hi) {
+        Slice s;
+        s.b0 = reads.seq_off[lo];
+        const uint64_t b1 = reads.seq_off[hi];
+        for (size_t i = lo; i <= hi; i++) s.off.push_back(reads.seq_off[i] - s.b0);
+        for (size_t j = (size_t) (std::upper_bound(reads.exc_end.begin(), reads.exc_end.end(), s.b0) - reads.exc_end.begin());
              j < reads.exc_start.size() && reads.exc_start[j] < b1; j++) {
-            es.push_back(std::max(reads.exc_start[j], b0) - b0);
-            ee.push_back(std::min(reads.exc_end[j], b1) - b0);
+            s.es.push_back(std::max(reads.exc_start[j], s.b0) - s.b0);
+            s.ee.push_back(std::min(reads.exc_end[j], b1) - s.b0);
         }
-        check(hga_count_kmers_packed(device, kk, reads.packed_data, b0, off.data(), hi - lo, es.data(), ee.data(), es.size(), min_count, c), "hga_count_kmers_packed");
+        return s;
+    };
+    auto count = [&](int kk, size_t lo, size_t hi, uint32_t min_count, hga_kmer_counts_t *c) {
+        const Slice s = slice(lo, hi);
+        check(hga_count_kmers_packed(device, kk, reads.packed_data, s.b0, s.off.data(), hi - lo, s.es.data(), s.ee.data(), s.es.size(), min_count, c),
+              "hga_count_kmers_packed");
     };
 
     if (k == 0) {
-        // get_unique_k_length (KmerAnalysis.cpp:41-56) with exact distinct counts
+        // get_unique_k_length (KmerAnalysis.cpp:41-56) with exact distinct counts: the spectrum's totals, no k-mer leaves the GPU
+        const Slice all = slice(0, reads.n_reads());
         auto distinct = [&](int kk) {
-            hga_kmer_counts_t c;
-            count(kk, 0, reads.n_reads(), 1, &c);
-            const uint64_t n = c.n;
-            hga_free_kmer_counts(&c);
-            return (long long) n;
+            hga_kmer_spectrum_t sp;
+            check(hga_count_spectrum_packed(device, kk, reads.packed_data, all.b0, all.off.data(), reads.n_reads(), all.es.data(), all.ee.data(), all.es.size(), 0,
+                                            nullptr, &sp),
+                  "hga_count_spectrum_packed");
+            return (long long) sp.n_distinct;
         };
         k = 11;
         long long previous = distinct(k);

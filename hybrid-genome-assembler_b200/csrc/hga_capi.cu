@@ -254,7 +254,21 @@ int hga_count_kmers_packed(int device, int k, const uint8_t *packed, uint64_t fi
     const uint64_t n_bases = read_off[n_reads];
     if (n_bases && !packed) { hga_set_error("hga_count_kmers_packed: packed is NULL"); return HGA_E_ARG; }
     HGA_TRY(check_exc_runs("hga_count_kmers_packed", exc_start, exc_end, n_exc, n_bases));
-    return hga_count_run("hga_count_kmers_packed", device, k, nullptr, packed, first_base, read_off, n_reads, exc_start, exc_end, n_exc, min_count, out);
+    return hga_count_run("hga_count_kmers_packed", device, k, nullptr, packed, first_base, read_off, n_reads, exc_start, exc_end, n_exc, min_count, out, nullptr, 0, nullptr);
+}
+
+int hga_count_spectrum_packed(int device, int k, const uint8_t *packed, uint64_t first_base, const uint64_t *read_off, uint64_t n_reads, const uint64_t *exc_start,
+                              const uint64_t *exc_end, uint64_t n_exc, uint32_t n_bins, uint64_t *hist, hga_kmer_spectrum_t *out) {
+    if (out) std::memset(out, 0, sizeof *out);
+    if (hist && n_bins) std::memset(hist, 0, (size_t) n_bins * 8);
+    if (!out || (n_bins && !hist)) { hga_set_error("hga_count_spectrum_packed: NULL argument"); return HGA_E_ARG; }
+    if (!read_off) { hga_set_error("hga_count_spectrum_packed: read_off is NULL"); return HGA_E_ARG; }
+    if (k < 1 || k > 32) { hga_set_error("Kmer size is too big or too small (k = %d)", k); return HGA_E_ARG; }
+    HGA_TRY(check_read_off("hga_count_spectrum_packed", read_off, n_reads));
+    const uint64_t n_bases = read_off[n_reads];
+    if (n_bases && !packed) { hga_set_error("hga_count_spectrum_packed: packed is NULL"); return HGA_E_ARG; }
+    HGA_TRY(check_exc_runs("hga_count_spectrum_packed", exc_start, exc_end, n_exc, n_bases));
+    return hga_count_run("hga_count_spectrum_packed", device, k, nullptr, packed, first_base, read_off, n_reads, exc_start, exc_end, n_exc, 0, nullptr, out, n_bins, hist);
 }
 
 int hga_scan_packed_device(hga_handle *h, const uint8_t *d_packed, uint64_t first_base, const uint64_t *d_read_off, uint64_t n_reads, uint64_t n_bases,

@@ -22,6 +22,8 @@
 // its read and once for the first exception run that can touch the span, then rolls the forward and reverse-complement values over the
 // span plus k - 1 bases, reading one 32-bit word per 16 bases and stepping over read ends and runs. Every later step (sort, run-length
 // encode, filter, quantiles, range splitting) is shared with the ASCII input, so the results are the same values in the same order.
+// Spectrum mode (hga_count_spectrum[_packed]): the same emits, passes and sorts; count_spectrum_kernel then adds each pass's runs to a
+// device histogram and totals in place of the run-length encode, filter and D2H, so no k-mer leaves the device.
 #include "hga_internal.cuh"
 
 #include <algorithm>
@@ -219,15 +221,98 @@ __global__ void count_flag_kernel(const unsigned long long *__restrict__ keys, c
         flag[i] = keys[i] != COUNT_SENTINEL && cnt[i] >= min_count;
 }
 
+// ---- spectrum ----------------------------------------------------------------------------------------------------------------------
+#define COUNT_SPECTRUM_CHUNK 16          // sorted positions a thread owns per round
+#define COUNT_SPECTRUM_REG_BINS 4        // bins counted in registers (runs of 1..4 for error-rich reads) and reduced per warp
+#define COUNT_SPECTRUM_SHARED_BINS 4096  // bins privatised per CTA as u32 in shared memory (16 KB: 8 CTAs of 256 threads per SM)
+
+// the first index >= j whose key is not `key`, given s[j - 1] == key: doubling steps, then bisection (O(log(run length)) loads)
+__device__ __forceinline__ uint64_t count_run_end(const unsigned long long *__restrict__ s, uint64_t m, uint64_t j, unsigned long long key) {
+    uint64_t lo = j - 1, hi, step = 1;                                       // s[lo] == key
+    for (;; step <<= 1) { hi = lo + step; if (hi >= m) { hi = m; break; } if (s[hi] != key) break; lo = hi; }
+    while (hi - lo > 1) { const uint64_t mid = lo + (hi - lo) / 2; if (s[mid] == key) lo = mid; else hi = mid; }
+    return hi;
+}
+
+// The runs of s[0 .. m) (one pass's keys, ascending; the sentinels of one-pass mode sort last and are skipped) added to acc:
+// acc[0] distinct keys, acc[1] windows (the sum of the run lengths), acc[2] the longest run, acc[3 + b] for b < n_bins the runs of
+// length b + 1 (the last bin: n_bins or more). A thread owns chunks of COUNT_SPECTRUM_CHUNK positions and counts the runs that start in
+// them; a run that reaches the end of its chunk finds its end with count_run_end. The counters a thread or a CTA keeps privately stay
+// below 2^32: a pass holds at most the keys of one device allocation, far fewer than 2^32 per CTA of the persistent grid.
+__global__ void count_spectrum_kernel(const unsigned long long *__restrict__ s, uint64_t m, uint32_t n_bins, unsigned long long *__restrict__ acc) {
+    unsigned long long *bins = acc + 3;
+    unsigned long long windows = 0, longest = 0;
+    uint32_t distinct = 0, reg[COUNT_SPECTRUM_REG_BINS] = {};
+#ifdef __CUDA_ARCH__
+    __shared__ uint32_t sh[COUNT_SPECTRUM_SHARED_BINS];
+    const uint32_t n_sh = n_bins < COUNT_SPECTRUM_SHARED_BINS ? n_bins : COUNT_SPECTRUM_SHARED_BINS;
+    for (uint32_t b = threadIdx.x; b < n_sh; b += blockDim.x) sh[b] = 0;
+    __syncthreads();
+#endif
+    auto add = [&](unsigned long long c) {
+        distinct++; windows += c; longest = c > longest ? c : longest;
+        if (n_bins == 0) return;
+        const uint32_t bin = (uint32_t) ((c < n_bins ? c : n_bins) - 1);
+        if (bin < COUNT_SPECTRUM_REG_BINS) {
+            #pragma unroll
+            for (uint32_t r = 0; r < COUNT_SPECTRUM_REG_BINS; r++) reg[r] += bin == r;
+        } else {
+#ifdef __CUDA_ARCH__
+            if (bin < COUNT_SPECTRUM_SHARED_BINS) atomicAdd(&sh[bin], 1u);
+            else atomicAdd(&bins[bin], 1ull);
+#else
+            bins[bin]++;
+#endif
+        }
+    };
+    const uint64_t n_chunks = (m + COUNT_SPECTRUM_CHUNK - 1) / COUNT_SPECTRUM_CHUNK;
+    for (uint64_t t = blockIdx.x * (uint64_t) blockDim.x + threadIdx.x; t < n_chunks; t += (uint64_t) gridDim.x * blockDim.x) {
+        const uint64_t a = t * COUNT_SPECTRUM_CHUNK, e = a + COUNT_SPECTRUM_CHUNK < m ? a + COUNT_SPECTRUM_CHUNK : m;
+        uint64_t i = a;
+        if (a) { const unsigned long long before = s[a - 1]; while (i < e && s[i] == before) i++; }     // the run of the previous chunk
+        while (i < e) {
+            const unsigned long long key = s[i];
+            if (key == COUNT_SENTINEL) break;
+            uint64_t j = i + 1;
+            while (j < e && s[j] == key) j++;
+            if (j == e) j = count_run_end(s, m, j, key);
+            add(j - i);
+            i = j;
+        }
+    }
+#ifdef __CUDA_ARCH__
+    distinct = __reduce_add_sync(0xFFFFFFFFu, distinct);
+    #pragma unroll
+    for (int r = 0; r < COUNT_SPECTRUM_REG_BINS; r++) reg[r] = __reduce_add_sync(0xFFFFFFFFu, reg[r]);
+    #pragma unroll
+    for (int d = 16; d; d >>= 1) {
+        windows += __shfl_xor_sync(0xFFFFFFFFu, windows, d);
+        const unsigned long long o = __shfl_xor_sync(0xFFFFFFFFu, longest, d);
+        longest = o > longest ? o : longest;
+    }
+    if ((threadIdx.x & 31) == 0 && distinct) {
+        atomicAdd(&acc[0], (unsigned long long) distinct); atomicAdd(&acc[1], windows); atomicMax(&acc[2], longest);
+        #pragma unroll
+        for (uint32_t r = 0; r < COUNT_SPECTRUM_REG_BINS; r++) if (reg[r]) atomicAdd(&sh[r], reg[r]);       // reg[r] != 0: r < n_bins
+    }
+    __syncthreads();
+    for (uint32_t b = threadIdx.x; b < n_sh; b += blockDim.x) if (sh[b]) atomicAdd(&bins[b], (unsigned long long) sh[b]);
+#else
+    acc[0] += distinct; acc[1] += windows; acc[2] = longest > acc[2] ? longest : acc[2];
+    for (uint32_t r = 0; r < COUNT_SPECTRUM_REG_BINS; r++) if (reg[r]) bins[r] += reg[r];
+#endif
+}
+
 struct Bufs {
-    DevBuf bases, off, exc, keys, sorted, run_key, run_len, acc_key2, acc_cnt2, tmp, scalars, flag;
-    ~Bufs() { for (DevBuf *b : {&bases, &off, &exc, &keys, &sorted, &run_key, &run_len, &acc_key2, &acc_cnt2, &tmp, &scalars, &flag}) b->release(); }
+    DevBuf bases, off, exc, keys, sorted, run_key, run_len, acc_key2, acc_cnt2, tmp, scalars, flag, spectrum;
+    ~Bufs() { for (DevBuf *b : {&bases, &off, &exc, &keys, &sorted, &run_key, &run_len, &acc_key2, &acc_cnt2, &tmp, &scalars, &flag, &spectrum}) b->release(); }
 };
 
 }  // namespace
 
 int hga_count_run(const char *who, int device, int k, const char *bases, const uint8_t *packed, uint64_t first_base, const uint64_t *read_off,
-                  uint64_t n_reads, const uint64_t *exc_start, const uint64_t *exc_end, uint64_t n_exc, uint32_t min_count, hga_kmer_counts_t *out) {
+                  uint64_t n_reads, const uint64_t *exc_start, const uint64_t *exc_end, uint64_t n_exc, uint32_t min_count, hga_kmer_counts_t *out,
+                  hga_kmer_spectrum_t *spec, uint32_t n_bins, uint64_t *hist) {
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) { cudaGetLastError(); hga_set_error("%s: no usable CUDA device (this library has no CPU path)", who); return HGA_E_CUDA; }
     HGA_CUDA(cudaSetDevice(device));
@@ -267,10 +352,29 @@ int hga_count_run(const char *who, int device, int k, const char *bases, const u
     auto grid = [&](uint64_t n) { return (int) std::max<uint64_t>(1, std::min<uint64_t>((n + 255) / 256, (uint64_t) sm * 16)); };
     std::vector<uint64_t> res_k;
     std::vector<uint32_t> res_c;
+    // spectrum mode: device accumulators of count_spectrum_kernel across the passes. No count exceeds n_bases, so bins past it stay
+    // empty and the device keeps min(n_bins, n_bases) of them
+    const uint32_t spec_bins = (uint32_t) std::min<uint64_t>(n_bins, n_bases);
+    if (spec) {
+        HGA_TRY(b.spectrum.ensure((spec_bins + 3ull) * 8));
+        HGA_CUDA(cudaMemsetAsync(b.spectrum.p, 0, (spec_bins + 3ull) * 8, st));
+    }
 
-    // m unsorted keys in b.keys -> sorted runs -> (k-mer, count >= min_count, sentinel dropped) appended to the host result
+    // m unsorted keys in b.keys -> sorted runs -> (k-mer, count >= min_count, sentinel dropped) appended to the host result, or in
+    // spectrum mode the runs added to the device spectrum
     auto finish_pass = [&](uint64_t m) -> int {
         if (m == 0) return HGA_OK;
+        if (spec) {
+            HGA_TRY(b.sorted.ensure(m * 8));
+            unsigned long long *d_keys = b.keys.as<unsigned long long>(), *d_sorted = b.sorted.as<unsigned long long>();
+            size_t t1 = 0;
+            HGA_CUDA(cub::DeviceRadixSort::SortKeys(nullptr, t1, d_keys, d_sorted, m, 0, end_bit, st));
+            HGA_TRY(b.tmp.ensure(t1 + 16));
+            HGA_CUDA(cub::DeviceRadixSort::SortKeys(b.tmp.p, t1, d_keys, d_sorted, m, 0, end_bit, st));
+            count_spectrum_kernel<<<grid((m + COUNT_SPECTRUM_CHUNK - 1) / COUNT_SPECTRUM_CHUNK), 256, 0, st>>>(d_sorted, m, spec_bins, b.spectrum.as<unsigned long long>());
+            HGA_CUDA(cudaGetLastError());
+            return HGA_OK;
+        }
         HGA_TRY(b.sorted.ensure(m * 8)); HGA_TRY(b.run_key.ensure(m * 8)); HGA_TRY(b.run_len.ensure(m * 4));
         unsigned long long *d_keys = b.keys.as<unsigned long long>(), *d_sorted = b.sorted.as<unsigned long long>(), *d_rk = b.run_key.as<unsigned long long>();
         uint32_t *d_rl = b.run_len.as<uint32_t>();
@@ -370,6 +474,11 @@ int hga_count_run(const char *who, int device, int k, const char *bases, const u
             HGA_CUDA(cudaStreamSynchronize(st));
             if (m > B) {
                 if (hi - lo == 1) {                                          // one k-mer, seen m times
+                    if (spec) {
+                        spec->n_distinct++; spec->n_windows += m; spec->max_count = std::max<uint64_t>(spec->max_count, m);
+                        if (n_bins) hist[std::min<uint64_t>(m, n_bins) - 1]++;
+                        continue;
+                    }
                     if (m >= min_count) { res_k.push_back(lo); res_c.push_back((uint32_t) std::min<unsigned long long>(m, 0xFFFFFFFFull)); }
                     continue;
                 }
@@ -383,6 +492,13 @@ int hga_count_run(const char *who, int device, int k, const char *bases, const u
         }
         // HGA_COUNT_STATS=1: how the key range was cut (a split range counts its pass and the passes of its halves)
         if (getenv("HGA_COUNT_STATS")) fprintf(stderr, "%s: %llu key-range passes (%llu ranges split)\n", who, (unsigned long long) passes, (unsigned long long) splits);
+    }
+    if (spec) {
+        std::vector<unsigned long long> h(spec_bins + 3ull);
+        HGA_CUDA(cudaMemcpy(h.data(), b.spectrum.p, h.size() * 8, cudaMemcpyDeviceToHost));
+        spec->n_distinct += h[0]; spec->n_windows += h[1]; spec->max_count = std::max<uint64_t>(spec->max_count, h[2]);
+        for (uint32_t i = 0; i < spec_bins; i++) hist[i] += h[3 + i];
+        return HGA_OK;
     }
     const uint64_t n_out = res_k.size();
     uint64_t *hk = (uint64_t *) std::malloc((n_out + 1) * 8);
@@ -398,7 +514,17 @@ extern "C" int hga_count_kmers(int device, int k, const char *bases, const uint6
     out->n = 0; out->kmer = nullptr; out->count = nullptr;
     if (k < 1 || k > 32) { hga_set_error("Kmer size is too big or too small (k = %d)", k); return HGA_E_ARG; }
     if (n_reads && (!bases || !read_off)) { hga_set_error("hga_count_kmers: NULL argument"); return HGA_E_ARG; }
-    return hga_count_run("hga_count_kmers", device, k, bases, nullptr, 0, read_off, n_reads, nullptr, nullptr, 0, min_count, out);
+    return hga_count_run("hga_count_kmers", device, k, bases, nullptr, 0, read_off, n_reads, nullptr, nullptr, 0, min_count, out, nullptr, 0, nullptr);
+}
+
+extern "C" int hga_count_spectrum(int device, int k, const char *bases, const uint64_t *read_off, uint64_t n_reads, uint32_t n_bins, uint64_t *hist,
+                                  hga_kmer_spectrum_t *out) {
+    if (out) std::memset(out, 0, sizeof *out);
+    if (hist && n_bins) std::memset(hist, 0, (size_t) n_bins * 8);
+    if (!out || (n_bins && !hist)) { hga_set_error("hga_count_spectrum: NULL argument"); return HGA_E_ARG; }
+    if (k < 1 || k > 32) { hga_set_error("Kmer size is too big or too small (k = %d)", k); return HGA_E_ARG; }
+    if (n_reads && (!bases || !read_off)) { hga_set_error("hga_count_spectrum: NULL argument"); return HGA_E_ARG; }
+    return hga_count_run("hga_count_spectrum", device, k, bases, nullptr, 0, read_off, n_reads, nullptr, nullptr, 0, 0, nullptr, out, n_bins, hist);
 }
 
 extern "C" void hga_free_kmer_counts(hga_kmer_counts_t *c) {

@@ -361,11 +361,13 @@ struct ScanPackedInput {
 int hga_scan_run(hga_handle *h, const char *d_bases, const uint64_t *d_read_off, uint64_t n_reads, uint64_t n_bases, const char *h_bases,
                  const ScanPackedInput *packed = nullptr);
 int hga_scan_finish_positions(hga_handle *h);
-// the k-mer count behind hga_count_kmers and hga_count_kmers_packed (csrc/hga_count.cu), arguments already checked.
+// the k-mer count behind hga_count_kmers[_packed] and hga_count_spectrum[_packed] (csrc/hga_count.cu), arguments already checked.
 // packed == nullptr: ASCII `bases`, read set bases[read_off[0] .. read_off[n_reads]). Otherwise the case-folded packing, bases
 // first_base + read_off[0 .. n_reads] (read_off[0] == 0) and the exception runs relative to first_base.
+// spec == nullptr: the counts >= min_count into *out. Otherwise the spectrum is ADDED to *spec and hist[0 .. n_bins) (zeroed by the caller).
 int hga_count_run(const char *who, int device, int k, const char *bases, const uint8_t *packed, uint64_t first_base, const uint64_t *read_off,
-                  uint64_t n_reads, const uint64_t *exc_start, const uint64_t *exc_end, uint64_t n_exc, uint32_t min_count, hga_kmer_counts_t *out);
+                  uint64_t n_reads, const uint64_t *exc_start, const uint64_t *exc_end, uint64_t n_exc, uint32_t min_count, hga_kmer_counts_t *out,
+                  hga_kmer_spectrum_t *spec, uint32_t n_bins, uint64_t *hist);
 int hga_index_run(hga_handle *h);
 int hga_build_lists(hga_handle *h, const uint32_t *d_keys, const uint64_t *d_row_off, uint64_t n_rows, uint64_t E, uint32_t n_keys);
 int hga_pairs_run(hga_handle *h, uint32_t min_score, const uint32_t *pivots, uint64_t n_pivots);

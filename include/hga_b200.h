@@ -19,6 +19,7 @@
  *                           merge_components, get_component_ids             clustering/ReadClusteringEngine.cpp:349-422, :764, :785-794
  *   hga_count_kmers / hga_host_sdk_* <- jellyfish + JellyfishOccurrenceReader (the --kmers file)          occurrences/ (all files), jellyfish_occurrences.cpp
  *   hga_count_kmers_packed     the same count from case-folded 2-bit packed bases (hga_host_pack_bases_folded packs on the host)
+ *   hga_count_spectrum[_packed]  the k-mer spectrum of that count (distinct k-mers per count) without materialising the k-mers
  *   hga_enrich_full      <- the same plus the tail / spectral block in between (second merge_components)     :764-794
  *
  * Conventions
@@ -282,6 +283,21 @@ int hga_count_kmers(int device, int k, const char *bases, const uint64_t *read_o
 int hga_count_kmers_packed(int device, int k, const uint8_t *packed, uint64_t first_base, const uint64_t *read_off, uint64_t n_reads,
                            const uint64_t *exc_start, const uint64_t *exc_end, uint64_t n_exc, uint32_t min_count, hga_kmer_counts_t *out);
 void hga_free_kmer_counts(hga_kmer_counts_t *c);
+/* hga_count_spectrum[_packed]: the k-mer spectrum of the same count, computed on the GPU without materialising the k-mers (what
+ *   `jellyfish histo` / `stats` print; the k sweep of jf_occurrences reads n_distinct). Host memory is O(n_bins) whatever the input. */
+typedef struct {
+    uint64_t n_windows;    /* windows counted (k bases inside one read, all A C G T a c g t) = the sum of all counts */
+    uint64_t n_distinct;   /* distinct canonical k-mers = hga_count_kmers(.., min_count = 1, ..).n */
+    uint64_t max_count;    /* largest count of any k-mer, exact (not clipped at 2^32 - 1); 0 when there is no window */
+} hga_kmer_spectrum_t;
+/* hist: caller-owned, n_bins entries (NULL allowed when n_bins == 0). hist[c - 1] = distinct k-mers seen exactly c times for
+ * 1 <= c < n_bins; hist[n_bins - 1] = those seen n_bins times or more. Same k-mer rule, read-set rules and checks as hga_count_kmers /
+ * hga_count_kmers_packed; nothing is allocated for the caller. */
+int hga_count_spectrum(int device, int k, const char *bases, const uint64_t *read_off, uint64_t n_reads,
+                       uint32_t n_bins, uint64_t *hist, hga_kmer_spectrum_t *out);
+int hga_count_spectrum_packed(int device, int k, const uint8_t *packed, uint64_t first_base, const uint64_t *read_off, uint64_t n_reads,
+                              const uint64_t *exc_start, const uint64_t *exc_end, uint64_t n_exc,
+                              uint32_t n_bins, uint64_t *hist, hga_kmer_spectrum_t *out);
 int hga_host_sdk_merge(int n_files, const uint64_t *file_off, const uint64_t *kmer, const uint32_t *count, uint64_t *out_kmer, uint32_t *out_total,
                        uint32_t *out_max, uint32_t *out_files, uint64_t *out_n);
 int hga_host_sdk_specificity(uint64_t n, const uint32_t *total, const uint32_t *max, const double *thresholds, int n_thresholds, double *out_threshold,

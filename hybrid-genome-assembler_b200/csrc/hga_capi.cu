@@ -173,7 +173,7 @@ int hga_scan_device(hga_handle *h, const char *d_bases, const uint64_t *d_read_o
     if ((n_bases && !d_bases) || !d_read_off) { hga_set_error("hga_scan_device: NULL buffer"); return HGA_E_ARG; }
     HGA_TRY(use_device(h));
     h->read_id_base = read_id_base;
-    return hga_scan_run(h, d_bases, d_read_off, n_reads, n_bases, nullptr);
+    return hga_scan_run(h, d_bases, d_read_off, n_reads, n_bases, nullptr, nullptr, "hga_scan_device");
 }
 
 int hga_scan(hga_handle *h, const char *bases, const uint64_t *read_off, uint64_t n_reads, uint32_t read_id_base) {
@@ -185,7 +185,7 @@ int hga_scan(hga_handle *h, const char *bases, const uint64_t *read_off, uint64_
     if (n_bases && !bases) { hga_set_error("hga_scan: bases is NULL"); return HGA_E_ARG; }
     for (uint64_t i = 0; i < n_reads; i++) {
         if (read_off[i + 1] < read_off[i]) { hga_set_error("hga_scan: read_off is not monotone at read %llu", (unsigned long long) i); return HGA_E_ARG; }
-        if (read_off[i + 1] - read_off[i] >= (1ull << 30)) { hga_set_error("hga_scan: read %llu is longer than 2^30 bases", (unsigned long long) i); return HGA_E_ARG; }
+        if (read_off[i + 1] - read_off[i] >= (1ull << 30)) { hga_set_error("hga_scan: read %llu has 2^30 bases or more (reads must be shorter than 2^30 bases)", (unsigned long long) i); return HGA_E_ARG; }
     }
     HGA_TRY(h->d_bases.ensure(n_bases + 64));
     HGA_TRY(h->d_read_off.ensure((n_reads + 1) * 8));
@@ -200,7 +200,7 @@ static int check_read_off(const char *who, const uint64_t *read_off, uint64_t n_
     if (read_off[0] != 0) { hga_set_error("%s: read_off[0] must be 0", who); return HGA_E_ARG; }
     for (uint64_t i = 0; i < n_reads; i++) {
         if (read_off[i + 1] < read_off[i]) { hga_set_error("%s: read_off is not monotone at read %llu", who, (unsigned long long) i); return HGA_E_ARG; }
-        if (read_off[i + 1] - read_off[i] >= (1ull << 30)) { hga_set_error("%s: read %llu is longer than 2^30 bases", who, (unsigned long long) i); return HGA_E_ARG; }
+        if (read_off[i + 1] - read_off[i] >= (1ull << 30)) { hga_set_error("%s: read %llu has 2^30 bases or more (reads must be shorter than 2^30 bases)", who, (unsigned long long) i); return HGA_E_ARG; }
     }
     return HGA_OK;
 }
@@ -239,7 +239,7 @@ int hga_scan_packed(hga_handle *h, const uint8_t *packed, uint64_t first_base, c
     ScanPackedInput in;
     in.sub = sub;
     in.d_exc_start = h->d_exc.as<uint64_t>(); in.d_exc_end = in.d_exc_start + n_exc;
-    in.h_exc_start = exc_start; in.h_exc_end = exc_end; in.n_exc = n_exc; in.check = false;
+    in.h_exc_start = exc_start; in.h_exc_end = exc_end; in.n_exc = n_exc;
     return hga_scan_run(h, h->d_bases.as<char>(), h->d_read_off.as<uint64_t>(), n_reads, n_bases, n_bytes ? reinterpret_cast<const char *>(packed + first_base / 4) : nullptr,
                         &in);
 }
@@ -281,8 +281,8 @@ int hga_scan_packed_device(hga_handle *h, const uint8_t *d_packed, uint64_t firs
     h->read_id_base = read_id_base;
     ScanPackedInput in;
     in.sub = (uint32_t) (first_base & 3);
-    in.d_exc_start = d_exc_start; in.d_exc_end = d_exc_end; in.h_exc_start = in.h_exc_end = nullptr; in.n_exc = n_exc; in.check = true;
-    return hga_scan_run(h, reinterpret_cast<const char *>(d_packed + first_base / 4), d_read_off, n_reads, n_bases, nullptr, &in);
+    in.d_exc_start = d_exc_start; in.d_exc_end = d_exc_end; in.h_exc_start = in.h_exc_end = nullptr; in.n_exc = n_exc;
+    return hga_scan_run(h, reinterpret_cast<const char *>(d_packed + first_base / 4), d_read_off, n_reads, n_bases, nullptr, &in, "hga_scan_packed_device");
 }
 
 int hga_get_hits(hga_handle *h, int sorted_by_kmer_id, hga_hits *out) {

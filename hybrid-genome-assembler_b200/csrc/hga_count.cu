@@ -479,7 +479,15 @@ int hga_count_run(const char *who, int device, int k, const char *bases, const u
                         if (n_bins) hist[std::min<uint64_t>(m, n_bins) - 1]++;
                         continue;
                     }
-                    if (m >= min_count) { res_k.push_back(lo); res_c.push_back((uint32_t) std::min<unsigned long long>(m, 0xFFFFFFFFull)); }
+                    if (m > 0xFFFFFFFFull) {                                 // the counts are 32-bit: refuse rather than clip
+                        char s[33];
+                        for (int i = 0; i < k; i++) s[i] = "ACGT"[(lo >> (2 * (k - 1 - i))) & 3];
+                        s[k] = '\0';
+                        hga_set_error("%s: k-mer %s occurs %llu times, more than a 32-bit count holds (2^32 - 1); hga_count_spectrum gives its exact count",
+                                      who, s, m);
+                        return HGA_E_OVERFLOW;
+                    }
+                    if (m >= min_count) { res_k.push_back(lo); res_c.push_back((uint32_t) m); }
                     continue;
                 }
                 splits++;

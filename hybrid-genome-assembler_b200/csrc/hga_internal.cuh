@@ -288,7 +288,7 @@ struct hga_handle {
     double scan_density = 0;              // hits per base of the previous scan on this handle (sizes the next one's hit buffers)
     bool pos_pending = false;
     DevBuf d_tile_state, d_tile_dir, d_scan_scalars;
-    DevBuf d_exc, d_exc_dir;              // packed scans: exception runs (host entry: starts then ends), first run touching each tile + check flag
+    DevBuf d_exc, d_exc_dir;              // packed scans: exception runs (host entry: starts then ends), first run touching each tile
     bool have_scan = false;
 
     // row space of the inverted index, pairs and components (this GPU's reads; ALL reads with a communicator)
@@ -354,12 +354,13 @@ struct ScanPackedInput {
     const uint64_t *d_exc_start, *d_exc_end;  // device, n_exc each (the host entry's runs are copied there first: h_exc_* != nullptr)
     const uint64_t *h_exc_start, *h_exc_end;
     uint64_t n_exc;
-    bool check;                               // device entry: validate the runs on the GPU, fail with HGA_E_ARG
 };
 // h_bases != nullptr: the bases are still on the host; the run copies them (in chunks, overlapped with the scan when large)
 // packed == nullptr: ASCII bases, one byte each
+// check != nullptr: a device entry of that name; its read lengths (and, packed, read_off[0] and the runs) are checked on the GPU and a violation
+// fails with HGA_E_ARG (the host entries check their input before they call this)
 int hga_scan_run(hga_handle *h, const char *d_bases, const uint64_t *d_read_off, uint64_t n_reads, uint64_t n_bases, const char *h_bases,
-                 const ScanPackedInput *packed = nullptr);
+                 const ScanPackedInput *packed = nullptr, const char *check = nullptr);
 int hga_scan_finish_positions(hga_handle *h);
 // the k-mer count behind hga_count_kmers[_packed] and hga_count_spectrum[_packed] (csrc/hga_count.cu), arguments already checked.
 // packed == nullptr: ASCII `bases`, read set bases[read_off[0] .. read_off[n_reads]). Otherwise the case-folded packing, bases

@@ -655,13 +655,21 @@ __global__ void scan_exc_dir_kernel(const uint64_t *__restrict__ exc_start, cons
     }
 }
 
-// device entry of a packed scan: read_off[0] must be 0 and the runs non-empty, sorted, disjoint and inside [0, n_bases); a violation sets *bad
-__global__ void scan_exc_check_kernel(const uint64_t *__restrict__ read_off, const uint64_t *__restrict__ exc_start, const uint64_t *__restrict__ exc_end,
-                                      uint64_t n_exc, uint64_t n_bases, unsigned long long *bad) {
-    if (blockIdx.x == 0 && threadIdx.x == 0 && read_off[0] != 0) *bad = 1;
-    for (uint64_t i = blockIdx.x * (uint64_t) blockDim.x + threadIdx.x; i < n_exc; i += (uint64_t) gridDim.x * blockDim.x) {
-        const uint64_t s = exc_start[i], e = exc_end[i];
-        if (s >= e || e > n_bases || (i + 1 < n_exc && exc_start[i + 1] < e)) *bad = 1;
+// input of a device entry. Every read is shorter than 2^30 bases (a tile sees its reads' starts through clamp_local, 31 bits): flag[0] = the
+// first read that is not (flag[0] starts at ~0). Packed input: read_off[0] must be 0 and the runs non-empty, sorted, disjoint and inside
+// [0, n_bases); a violation sets flag[1]. The last read ends at n_bases.
+__global__ void scan_input_check_kernel(const uint64_t *__restrict__ read_off, uint64_t n_reads, const uint64_t *__restrict__ exc_start,
+                                        const uint64_t *__restrict__ exc_end, uint64_t n_exc, uint64_t n_bases, bool packed, unsigned long long *flag) {
+    if (blockIdx.x == 0 && threadIdx.x == 0 && packed && read_off[0] != 0) flag[1] = 1;
+    for (uint64_t i = blockIdx.x * (uint64_t) blockDim.x + threadIdx.x; i < n_reads || i < n_exc; i += (uint64_t) gridDim.x * blockDim.x) {
+        if (i < n_reads) {
+            const uint64_t a = read_off[i], b = i + 1 < n_reads ? read_off[i + 1] : n_bases;
+            if (b > a && b - a >= (1ull << 30)) atomicMin(&flag[0], (unsigned long long) i);
+        }
+        if (i < n_exc) {
+            const uint64_t s = exc_start[i], e = exc_end[i];
+            if (s >= e || e > n_bases || (i + 1 < n_exc && exc_start[i + 1] < e)) flag[1] = 1;
+        }
     }
 }
 
@@ -712,6 +720,13 @@ bool scan_tma_variant() {
     return v != 0;
 }
 
+// what a scan reads back at its synchronisation: the scalars and, for a device entry, the flags of scan_input_check_kernel
+struct ScanReadback {
+    ScanScalars sc;
+    unsigned long long bad_read;     // first read of 2^30 bases or more, ~0 = none
+    unsigned long long bad_runs;     // packed: read_off[0] != 0 or a bad exception run
+};
+
 typedef void (*scan_kernel_t)(const ScanParams);
 scan_kernel_t scan_kernel(bool packed) {
     if (packed) return scan_probe_kernel<4, false, true>;          // the experiment switches apply to ASCII input only
@@ -732,13 +747,16 @@ int launch_scan(hga_handle *h, const ScanParams &p, int grid, bool packed) {
 }  // namespace
 
 int hga_scan_run(hga_handle *h, const char *d_bases, const uint64_t *d_read_off, uint64_t n_reads, uint64_t n_bases, const char *h_bases,
-                 const ScanPackedInput *packed) {
+                 const ScanPackedInput *packed, const char *check) {
     h->have_scan = h->have_index = h->have_pairs = h->have_selection = h->have_components = h->have_enrichment = false;
     h->n_reads = n_reads; h->n_bases = n_bases; h->n_hits = 0;
     if (n_reads >= (1ull << 32) - 1) { hga_set_error("hga_scan: more than 2^32-2 reads per GPU"); return HGA_E_ARG; }
     HGA_TRY(h->d_row_off.ensure((n_reads + 1) * 8));
-    HGA_TRY(h->d_scan_scalars.ensure(sizeof(ScanScalars) + (size_t) h->sm_count * 8 * SCAN_WARPS * 16));   // + the warps' open chunks (chunked launches)
+    // the scalars, then the two words of the input check (read back with them), then the warps' open chunks (chunked launches)
+    HGA_TRY(h->d_scan_scalars.ensure(sizeof(ScanReadback) + (size_t) h->sm_count * 8 * SCAN_WARPS * 16));
     ScanScalars *d_sc = h->d_scan_scalars.as<ScanScalars>();
+    unsigned long long *d_check = reinterpret_cast<unsigned long long *>(h->d_scan_scalars.as<char>() + offsetof(ScanReadback, bad_read));
+    unsigned long long *d_warp_chunks = reinterpret_cast<unsigned long long *>(h->d_scan_scalars.as<char>() + sizeof(ScanReadback));
     // the kernel loads aligned 16 B pieces (packed: 4 B words): frame = the bases aligned down; lead = bases between frame and the first base
     const bool pk = packed != nullptr;
     const uint32_t frame_bytes = (uint32_t) (reinterpret_cast<uintptr_t>(d_bases) & (pk ? 3 : 15));
@@ -763,12 +781,9 @@ int hga_scan_run(hga_handle *h, const char *d_bases, const uint64_t *d_read_off,
     p.scalars = d_sc;
     if (const char *e = getenv("HGA_SCAN_DIAG")) p.diag = atoi(e);
     unsigned long long *exc_dir = nullptr;
-    const bool check = pk && packed->check;
-    if (n_exc || check) {                                                          // run directory: n_tiles entries + the check flag
+    if (n_exc) {                                                                   // run directory: n_tiles entries
         HGA_TRY(h->d_exc_dir.ensure((n_tiles + 1) * 8));
         exc_dir = h->d_exc_dir.as<unsigned long long>();
-    }
-    if (n_exc) {
         p.exc_start = packed->d_exc_start; p.exc_end = packed->d_exc_end; p.n_exc = n_exc; p.exc_dir = exc_dir;
     }
 
@@ -780,8 +795,9 @@ int hga_scan_run(hga_handle *h, const char *d_bases, const uint64_t *d_read_off,
 
     auto launch_scan_pk = [&](const ScanParams &lp, int grid) { return launch_scan(h, lp, grid, pk); };
     StageTimer timer(h, &h->metrics.scan_ms);
-    ScanScalars sc;
-    memset(&sc, 0, sizeof(sc));
+    ScanReadback rb;
+    memset(&rb, 0, sizeof(rb));
+    ScanScalars &sc = rb.sc;
     uint64_t capacity = 0, E = 0;
     h->metrics.scan_retries = 0;
     // Hit-buffer sizes. Warps reserve chunks, so the buffer holds gaps: what is left of a chunk when the next tile does not fit (less
@@ -808,10 +824,11 @@ int hga_scan_run(hga_handle *h, const char *d_bases, const uint64_t *d_read_off,
         return HGA_OK;
     };
     auto launch_exc_dir = [&]() -> int {
-        if (check) {
-            HGA_CUDA(cudaMemsetAsync(exc_dir + n_tiles, 0, 8, h->stream));
-            scan_exc_check_kernel<<<(int) std::min<uint64_t>((n_exc + 256) / 256, (uint64_t) h->sm_count * 8), 256, 0, h->stream>>>(d_read_off, p.exc_start, p.exc_end, n_exc,
-                                                                                                                                    n_bases, exc_dir + n_tiles);
+        if (check) {                                                               // device entry: its flags come back with the scalars of the scan
+            HGA_CUDA(cudaMemsetAsync(d_check, 0xFF, 8, h->stream));
+            HGA_CUDA(cudaMemsetAsync(d_check + 1, 0, 8, h->stream));
+            scan_input_check_kernel<<<(int) std::min<uint64_t>((std::max(n_reads, n_exc) + 256) / 256, (uint64_t) h->sm_count * 8), 256, 0, h->stream>>>(
+                d_read_off, n_reads, p.exc_start, p.exc_end, n_exc, n_bases, pk, d_check);
             h->metrics.kernel_launches++;
         }
         if (n_exc && n_tiles > 0) {
@@ -875,8 +892,9 @@ int hga_scan_run(hga_handle *h, const char *d_bases, const uint64_t *d_read_off,
         HGA_TRY(h->d_pos_tmp.ensure((capacity + 1) * 4));
         p.out_slot = h->d_sort_a.as<uint32_t>(); p.out_pos = h->d_pos_tmp.as<uint32_t>();
         p.capacity = capacity; p.tile_stride = 0; p.chunk = SCAN_CHUNK;
-        p.warp_chunks = reinterpret_cast<unsigned long long *>(d_sc + 1);
-        HGA_CUDA(cudaMemsetAsync(d_sc, 0, sizeof(ScanScalars) + warps_full * 16, h->stream));
+        p.warp_chunks = d_warp_chunks;
+        HGA_CUDA(cudaMemsetAsync(d_sc, 0, sizeof(ScanScalars), h->stream));
+        HGA_CUDA(cudaMemsetAsync(d_warp_chunks, 0, warps_full * 16, h->stream));
         for (uint64_t c = 0; c < n_chunks; c++) {
             HGA_CUDA(cudaStreamWaitEvent(h->stream, landed[c], 0));
             p.tile_begin = c * chunk_tiles; p.n_tiles = std::min<uint64_t>(chunk_tiles, n_tiles - p.tile_begin);
@@ -926,7 +944,7 @@ int hga_scan_run(hga_handle *h, const char *d_bases, const uint64_t *d_read_off,
         p.capacity = capacity; p.n_tiles = n_tiles; p.tile_begin = 0; p.tile_stride = 0; p.chunk = SCAN_CHUNK;
         HGA_CUDA(cudaMemsetAsync(d_sc, 0, sizeof(ScanScalars), h->stream));
         HGA_TRY(launch_scan_pk(p, grid_full));
-        HGA_CUDA(cudaMemcpyAsync(&sc, d_sc, sizeof(sc), cudaMemcpyDeviceToHost, h->stream));
+        HGA_CUDA(cudaMemcpyAsync(&rb, d_sc, check ? sizeof(rb) : sizeof(sc), cudaMemcpyDeviceToHost, h->stream));   // with the check's flags
         HGA_CUDA(cudaStreamSynchronize(h->stream));
         E = sc.total;
         if (!sc.overflow) break;
@@ -935,13 +953,18 @@ int hga_scan_run(hga_handle *h, const char *d_bases, const uint64_t *d_read_off,
         h->metrics.scan_retries++;
     }
 
-    if (check) {                                                                   // the check ran before the scan; its flag is read now
-        unsigned long long bad = 0;
-        HGA_CUDA(cudaMemcpyAsync(&bad, exc_dir + n_tiles, 8, cudaMemcpyDeviceToHost, h->stream));
-        HGA_CUDA(cudaStreamSynchronize(h->stream));
-        if (bad) {
-            hga_set_error("hga_scan_packed_device: read_off[0] must be 0 and the exception runs non-empty, sorted, non-overlapping and inside [0, %llu)",
+    if (check) {                                                                   // the check ran before the scan; its flags came back with the scalars
+        if (n_tiles == 0) {                                                        // no scan ran: read them on their own
+            HGA_CUDA(cudaMemcpyAsync(&rb, d_sc, sizeof(rb), cudaMemcpyDeviceToHost, h->stream));
+            HGA_CUDA(cudaStreamSynchronize(h->stream));
+        }
+        if (rb.bad_runs) {
+            hga_set_error("%s: read_off[0] must be 0 and the exception runs non-empty, sorted, non-overlapping and inside [0, %llu)", check,
                           (unsigned long long) n_bases);
+            return HGA_E_ARG;
+        }
+        if (rb.bad_read != ~0ull) {
+            hga_set_error("%s: read %llu has 2^30 bases or more (reads must be shorter than 2^30 bases)", check, rb.bad_read);
             return HGA_E_ARG;
         }
     }

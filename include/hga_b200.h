@@ -53,7 +53,7 @@ typedef struct hga_handle hga_handle;
 #define HGA_E_ARG 2         /* bad argument (k > 32 mirrors KmerIterator.cpp:24-26) */
 #define HGA_E_STATE 3       /* stage called out of order */
 #define HGA_E_NOMEM 4
-#define HGA_E_OVERFLOW 5    /* a 32-bit pair score or entry count overflowed */
+#define HGA_E_OVERFLOW 5    /* a 32-bit pair score, entry count or k-mer count overflowed */
 #define HGA_E_NCCL 6
 #define HGA_E_DUPLICATE 7   /* duplicate k-mer handed to hga_create */
 
@@ -83,7 +83,10 @@ int hga_set_stream(hga_handle *h, void *cuda_stream);
  * read_off[n_reads+1] : byte offset of every read in `bases`
  * Any byte other than 'A','C','G','T' follows the reference rule (code 0 on BOTH strands).
  * hga_scan copies the host buffers to the GPU inside the call; hga_scan_device takes device pointers. d_bases may have any
- * alignment (a read set can start anywhere inside a larger buffer): the scan loads the aligned 16-byte blocks that hold the bases. */
+ * alignment (a read set can start anywhere inside a larger buffer): the scan loads the aligned 16-byte blocks that hold the bases.
+ * Every read must be shorter than 2^30 bases, on every scan entry (hga_scan, hga_scan_device, hga_scan_packed, hga_scan_packed_device):
+ * a longer read fails with HGA_E_ARG and a message, and leaves no scan result. The host entries check read_off before they copy; the
+ * device entries check it on the GPU (the last read ends at n_bases). The stream itself may be longer than 2^32 bases. */
 int hga_scan(hga_handle *h, const char *bases, const uint64_t *read_off, uint64_t n_reads, uint32_t read_id_base);
 int hga_scan_device(hga_handle *h, const char *d_bases, const uint64_t *d_read_off, uint64_t n_reads, uint64_t n_bases,
                     uint32_t read_id_base);
@@ -107,7 +110,8 @@ int hga_host_pack_bases_folded(const char *bases, uint64_t n_bases, uint8_t *pac
 /* The read set = bases first_base + read_off[0 .. n_reads] of `packed` (read_off[0] == 0, the same rules as for ASCII), so a slice of
  * a larger packed buffer is scanned in place; the exception runs are relative to first_base and lie inside [0, read_off[n_reads]).
  * The host entry copies only the bytes that hold the read set and checks read_off and the runs (HGA_E_ARG with a message). The device
- * entry takes device pointers (d_packed at any byte address) and checks read_off[0] and the runs on the GPU: HGA_E_ARG, no hits. */
+ * entry takes device pointers (d_packed at any byte address) and checks read_off[0], the read lengths and the runs on the GPU: HGA_E_ARG,
+ * no hits. */
 int hga_scan_packed(hga_handle *h, const uint8_t *packed, uint64_t first_base, const uint64_t *read_off, uint64_t n_reads,
                     const uint64_t *exc_start, const uint64_t *exc_end, uint64_t n_exc, uint32_t read_id_base);
 int hga_scan_packed_device(hga_handle *h, const uint8_t *d_packed, uint64_t first_base, const uint64_t *d_read_off, uint64_t n_reads,
@@ -264,7 +268,9 @@ int hga_host_tail_connections(uint64_t n_reads, const uint64_t *row_off, const u
  * count lies in a range (:63-134).
  *   hga_count_kmers  : the counting on the GPU, no handle needed: the canonical k-mers of `bases` (windows with a byte other than
  *                      A C G T a c g t skipped, as jellyfish does) that occur at least min_count times (2 = the two-pass
- *                      Bloom-counter filter of run_jellyfish.sh without its false positives), ascending, with exact counts.
+ *                      Bloom-counter filter of run_jellyfish.sh without its false positives), ascending, with exact 32-bit
+ *                      counts: a k-mer seen more than 2^32 - 1 times fails the call with HGA_E_OVERFLOW and a message that
+ *                      names it and its count (hga_count_spectrum reports such a count exactly).
  *                      The arrays are malloc'ed by the library: release them with hga_free_kmer_counts.
  *   hga_host_sdk_*   : the reader's host arithmetic on those lists (files back to back: file f = [file_off[f], file_off[f + 1])).
  *                      merge: out arrays need room for file_off[n_files] entries. specificity: rows (threshold, total count,
@@ -278,8 +284,9 @@ typedef struct {
 int hga_count_kmers(int device, int k, const char *bases, const uint64_t *read_off, uint64_t n_reads, uint32_t min_count, hga_kmer_counts_t *out);
 /* hga_count_kmers_packed: the same counts from the case-folded packing of hga_host_pack_bases_folded, identical to hga_count_kmers on
  *   the ASCII bytes (same k-mers, counts and order). The read set and the runs follow hga_scan_packed's rules: bases first_base +
- *   read_off[0 .. n_reads] of `packed` with read_off[0] == 0, runs relative to first_base, sorted, non-empty, non-overlapping, inside
- *   [0, read_off[n_reads]). Only the bytes that hold the read set are copied. Bad input: HGA_E_ARG with a message. */
+ *   read_off[0 .. n_reads] of `packed` with read_off[0] == 0, every read shorter than 2^30 bases, runs relative to first_base, sorted,
+ *   non-empty, non-overlapping, inside [0, read_off[n_reads]). Only the bytes that hold the read set are copied. Bad input: HGA_E_ARG
+ *   with a message. */
 int hga_count_kmers_packed(int device, int k, const uint8_t *packed, uint64_t first_base, const uint64_t *read_off, uint64_t n_reads,
                            const uint64_t *exc_start, const uint64_t *exc_end, uint64_t n_exc, uint32_t min_count, hga_kmer_counts_t *out);
 void hga_free_kmer_counts(hga_kmer_counts_t *c);
@@ -292,7 +299,8 @@ typedef struct {
 } hga_kmer_spectrum_t;
 /* hist: caller-owned, n_bins entries (NULL allowed when n_bins == 0). hist[c - 1] = distinct k-mers seen exactly c times for
  * 1 <= c < n_bins; hist[n_bins - 1] = those seen n_bins times or more. Same k-mer rule, read-set rules and checks as hga_count_kmers /
- * hga_count_kmers_packed; nothing is allocated for the caller. */
+ * hga_count_kmers_packed (the packed spectrum too takes reads shorter than 2^30 bases only); nothing is allocated for the caller.
+ * No count is clipped: a k-mer seen more than 2^32 - 1 times is counted exactly. */
 int hga_count_spectrum(int device, int k, const char *bases, const uint64_t *read_off, uint64_t n_reads,
                        uint32_t n_bins, uint64_t *hist, hga_kmer_spectrum_t *out);
 int hga_count_spectrum_packed(int device, int k, const uint8_t *packed, uint64_t first_base, const uint64_t *read_off, uint64_t n_reads,

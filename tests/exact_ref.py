@@ -3,8 +3,14 @@
 It shares no code with the C oracle (oracle/hga_oracle.c) or the kernels, and unlike the oracle (O(sum of list^2) in Python-visible
 loops) it scales to tens of Mbases, so it can judge the GPU in the regimes only large inputs reach. Read ids are 1-based.
 
-  scan        uppercase ACGT input only (the rule for other bytes stays with the oracle tests): canonical k-mers of every window that
-              lies inside one read, membership and id by bisection in the sorted set, hit position = window end (seq[pos - k:pos])
+  scan        canonical k-mers of every window that lies inside one read, membership and id by bisection in the sorted set, hit
+              position = window end (seq[pos - k:pos]). A byte other than uppercase ACGT has code 0 on both strands (KmerIterator.cpp:56,62)
+  count       the k-mer count's rule instead (jellyfish): ACGT and acgt are bases, a window holding any other byte is skipped
+
+Inputs of many Gbases are built from a small library of distinct reads: a stream is a list of library indices, and since no window
+crosses a read, hits and counts of the stream follow from those of the library (library_hits, stream_hits, library_counts,
+stream_counts, spectrum). A library read may be periodic: tile(block)[:head] + tail, so that a read of 2^30 bases costs the
+reference one period and its tail.
   index       stable argsort of the hit ids: reads ascending inside every list, one entry per occurrence
   pairs       A = reads x k-mers matrix of multiplicities (duplicate hits summed), S = A A^T, pairs x < y with score >= min_score;
               with pivots, the pairs with at least one pivot
@@ -36,18 +42,43 @@ import numpy as np
 import scipy.sparse as sp
 from scipy.sparse import csgraph
 
-import datagen
-
-_CODE = np.full(256, 255, dtype=np.uint8)
+_FWD = np.zeros(256, dtype=np.uint64)          # scan rule: forward code, 0 for a byte other than ACGT
+_REV = np.zeros(256, dtype=np.uint64)          # complement code, 0 for a byte other than ACGT too
+_FOLD = np.full(256, 255, dtype=np.uint8)      # count rule: ACGT and acgt, 255 = not a base
 for _i, _c in enumerate(b"ACGT"):
-    _CODE[_c] = _i
+    _FWD[_c] = _i; _REV[_c] = 3 - _i
+    _FOLD[_c] = _FOLD[_c + 32] = _i
+
+
+def window_values(raw, k, rule="scan"):
+    """canonical value of the window starting at every position of the bytes raw (uint8 array) -> (uint64[n - k + 1], valid bool[..]).
+    rule "scan": every window is valid, a byte other than ACGT has code 0 on both strands; rule "count": ACGT and acgt are bases and a
+    window holding any other byte is not valid"""
+    raw = np.asarray(raw, dtype=np.uint8)
+    n = raw.shape[0] - k + 1
+    if n <= 0:
+        return np.zeros(0, dtype=np.uint64), np.zeros(0, dtype=bool)
+    if rule == "scan":
+        f, r = _FWD[raw], _REV[raw]
+        valid = np.ones(n, dtype=bool)
+    else:
+        c = _FOLD[raw]
+        bad = c == 255
+        f = np.where(bad, 0, c).astype(np.uint64)
+        r = np.uint64(3) - f
+        nb = np.concatenate([[0], np.cumsum(bad, dtype=np.int64)])
+        valid = nb[k:] == nb[:n]
+    fwd = np.zeros(n, dtype=np.uint64)
+    rev = np.zeros(n, dtype=np.uint64)
+    for j in range(k):
+        fwd |= f[j:j + n] << np.uint64(2 * (k - 1 - j))
+        rev |= r[j:j + n] << np.uint64(2 * j)
+    return np.minimum(fwd, rev), valid
 
 
 def scan(bases, read_off, k, kmers_sorted, chunk_bases=1 << 22):
     """-> (row_off uint64[n_reads + 1], kmer id uint32[E], window end uint32[E]) in (read, position) order"""
-    codes = _CODE[np.frombuffer(bytes(bases), dtype=np.uint8)]
-    if codes.shape[0] and codes.max() > 3:
-        raise ValueError("exact_ref.scan takes uppercase ACGT input only")
+    codes = np.frombuffer(bases, dtype=np.uint8) if isinstance(bases, (bytes, bytearray)) else np.asarray(bases, dtype=np.uint8)
     kmers_sorted = np.asarray(kmers_sorted, dtype=np.uint64)
     off = np.asarray(read_off, dtype=np.int64)
     n_reads = off.shape[0] - 1
@@ -59,7 +90,7 @@ def scan(bases, read_off, k, kmers_sorted, chunk_bases=1 << 22):
         r1 = max(r0 + 1, int(np.searchsorted(off, off[r0] + chunk_bases, side="right")) - 1)
         r1 = min(r1, n_reads)
         seg = codes[off[r0]:off[r1]]
-        km = datagen.canonical_kmers(seg, k)               # window starting at every position of the segment
+        km, _ = window_values(seg, k)                      # window starting at every position of the segment
         if km.shape[0]:
             start = np.arange(km.shape[0], dtype=np.int64)
             rel = off[r0:r1 + 1] - off[r0]
@@ -395,3 +426,115 @@ def enrich(row_off, kid, n_kmers, ex, ey, min_size, enrich_min, max_size=-1, clu
     return dict(core_id=cores, core_kmers=core_kmers, core_reads=core_reads, purged_off=purged_off, purged_read=purged_read,
                 econn=(cx, cy, cs), final_id=final, final_reads=final_reads, assignment=assignment,
                 scaffold=scaffold, trees=trees, first_merge=first)
+
+
+# ---- streams built from a library of reads -----------------------------------------------------------------------------------
+
+class LibRead:
+    """a library read: tile(block)[:head] + tail (block None, head 0: the tail alone). bytes() materialises it."""
+
+    def __init__(self, tail, block=None, head=0):
+        self.tail = np.asarray(tail, dtype=np.uint8)
+        self.block = None if block is None else np.asarray(block, dtype=np.uint8)
+        self.head = int(head)
+
+    def __len__(self):
+        return self.head + self.tail.shape[0]
+
+    def bytes(self):
+        if not self.head:
+            return self.tail
+        reps = -(-self.head // self.block.shape[0])
+        return np.concatenate([np.tile(self.block, reps)[:self.head], self.tail])
+
+    def cyclic(self, k):
+        """the bytes of every window of the periodic part (one period and k - 1 more)"""
+        return np.concatenate([self.block, np.tile(self.block, -(-(k - 1) // self.block.shape[0]))[:k - 1]])
+
+    def end_part(self, k):
+        """(bytes of the windows that end in the tail, their first base in the read): k - 1 bases of context and the tail"""
+        if not self.head:
+            return self.tail, 0
+        L = self.block.shape[0]
+        c0 = max(self.head - (k - 1), 0)
+        ctx = np.array([self.block[i % L] for i in range(c0, self.head)], dtype=np.uint8)
+        return np.concatenate([ctx, self.tail]), c0
+
+    def head_windows(self, k):
+        """windows that lie inside the periodic part"""
+        return max(self.head - k + 1, 0)
+
+
+def library_hits(lib, k, kmers_sorted):
+    """scan of every library read on its own -> list of (kmer id uint32[], window end uint32[]). The windows of a periodic read's
+    head must hold no k-mer of the set (checked)."""
+    out = []
+    for r in lib:
+        if r.head:
+            v, _ = window_values(r.cyclic(k), k)
+            at = np.searchsorted(kmers_sorted, v)
+            assert not np.any(kmers_sorted[np.minimum(at, kmers_sorted.shape[0] - 1)] == v), "the periodic part of a read holds a k-mer of the set"
+        part, p0 = r.end_part(k)
+        _, kid, pos = scan(part, np.array([0, part.shape[0]], dtype=np.uint64), k, kmers_sorted)
+        out.append((kid, (pos.astype(np.int64) + p0).astype(np.uint32)))
+    return out
+
+
+def stream_hits(lib_hits, order):
+    """the scan of the stream whose reads are lib[order[0]], lib[order[1]], ... -> (row_off, kmer id, window end)"""
+    order = np.asarray(order, dtype=np.int64)
+    n = np.array([h[0].shape[0] for h in lib_hits], dtype=np.int64)
+    row_off = np.zeros(order.shape[0] + 1, dtype=np.uint64)
+    np.cumsum(n[order], out=row_off[1:])
+    used = [i for i in order.tolist() if n[i]]
+    cat = lambda j, dt: np.concatenate([lib_hits[i][j] for i in used]) if used else np.zeros(0, dtype=dt)
+    return row_off, cat(0, np.uint32), cat(1, np.uint32)
+
+
+def library_counts(lib, k):
+    """canonical k-mer counts of every library read on its own (count rule) -> list of (k-mers ascending uint64, counts int64)"""
+    out = []
+    for r in lib:
+        part, _ = r.end_part(k)
+        v, ok = window_values(part, k, "count")
+        vals, wts = [v[ok]], [np.ones(int(ok.sum()), dtype=np.int64)]
+        if r.head:
+            cv, cok = window_values(r.cyclic(k), k, "count")
+            N, L = r.head_windows(k), r.block.shape[0]
+            per = np.full(L, N // L, dtype=np.int64) + (np.arange(L) < N % L)      # windows of the head at cyclic position i
+            vals.append(cv[cok]); wts.append(per[cok])
+        out.append(_sum_by_value(np.concatenate(vals), np.concatenate(wts)))
+    return out
+
+
+def _sum_by_value(v, w):
+    """(distinct values ascending, summed weights > 0)"""
+    o = np.argsort(v, kind="stable")
+    v, w = v[o], np.asarray(w, dtype=np.int64)[o]
+    if v.shape[0] == 0:
+        return v, w
+    start = np.concatenate([[0], np.flatnonzero(v[1:] != v[:-1]) + 1])
+    u, c = v[start], np.add.reduceat(w, start)
+    keep = c > 0
+    return u[keep], c[keep]
+
+
+def stream_counts(lib_counts, order, min_count=1):
+    """the counts of the stream lib[order[0]], lib[order[1]], ...: every library read's counts times its multiplicity, summed. ->
+    (k-mers ascending uint64, counts int64 >= min_count)"""
+    mult = np.bincount(np.asarray(order, dtype=np.int64), minlength=len(lib_counts))
+    used = [i for i in range(len(lib_counts)) if mult[i] and lib_counts[i][0].shape[0]]
+    if not used:
+        return np.zeros(0, dtype=np.uint64), np.zeros(0, dtype=np.int64)
+    u, c = _sum_by_value(np.concatenate([lib_counts[i][0] for i in used]), np.concatenate([lib_counts[i][1] * mult[i] for i in used]))
+    keep = c >= max(int(min_count), 1)
+    return u[keep], c[keep]
+
+
+def spectrum(counts, n_bins):
+    """-> (hist uint64[n_bins], n_windows, n_distinct, max_count) of exact counts, as hga_count_spectrum returns them"""
+    c = np.asarray(counts, dtype=np.int64)
+    hist = np.zeros(int(n_bins), dtype=np.uint64)
+    if n_bins and c.shape[0]:
+        hist[:] = np.bincount(np.minimum(c, n_bins) - 1, minlength=int(n_bins))
+    return hist, int(c.sum()), int(c.shape[0]), int(c.max(initial=0))

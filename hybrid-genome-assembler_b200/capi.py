@@ -68,7 +68,7 @@ class Metrics(C.Structure):
 # every symbol include/hga_b200.h declares (tests check the .so exports exactly these)
 EXPORTS = ["hga_last_error", "hga_version", "hga_device_count", "hga_init", "hga_host_alloc", "hga_host_free", "hga_create", "hga_destroy", "hga_set_stream",
            "hga_scan", "hga_scan_device", "hga_host_pack_bases", "hga_host_pack_bases_folded", "hga_scan_packed", "hga_scan_packed_device", "hga_get_hits", "hga_build_index", "hga_get_index", "hga_pair_count", "hga_get_pairs", "hga_select_edges",
-           "hga_get_selection", "hga_components", "hga_get_components", "hga_enrich", "hga_enrich_ex", "hga_enrich_full", "hga_get_tail_block", "hga_count_kmers", "hga_count_kmers_packed", "hga_count_spectrum", "hga_count_spectrum_packed", "hga_free_kmer_counts", "hga_host_sdk_merge", "hga_host_sdk_specificity", "hga_host_sdk_select", "hga_get_enrichment", "hga_get_purged_index", "hga_get_core_kmers", "hga_spectral_clustering", "hga_host_tail_connections", "hga_host_sym_eigen",
+           "hga_get_selection", "hga_components", "hga_get_components", "hga_enrich", "hga_enrich_ex", "hga_enrich_full", "hga_get_tail_block", "hga_count_kmers", "hga_count_kmers_packed", "hga_count_spectrum", "hga_count_spectrum_packed", "hga_free_kmer_counts", "hga_host_sdk_merge", "hga_host_sdk_specificity", "hga_host_sdk_select", "hga_sdk_count_packed", "hga_sdk_size", "hga_sdk_specificity", "hga_sdk_range", "hga_free_sdk_range", "hga_sdk_free", "hga_get_enrichment", "hga_get_purged_index", "hga_get_core_kmers", "hga_spectral_clustering", "hga_host_tail_connections", "hga_host_sym_eigen",
            "hga_metrics", "hga_comm_unique_id", "hga_comm_init", "hga_comm_gather_root"]
 
 
@@ -320,6 +320,89 @@ def sdk_select(total, files, lower, upper, percent=1.0, seed=0):
     _check(lib.hga_host_sdk_select(t.shape[0], t.ctypes.data_as(P), f.ctypes.data_as(P), int(lower), int(upper), float(percent), int(seed), sel.ctypes.data_as(P),
                                    C.byref(ns), C.byref(nd)))
     return sel[:t.shape[0]].astype(bool), int(ns.value), int(nd.value)
+
+
+class _SdkRange(C.Structure):
+    _fields_ = [("n", C.c_uint64), ("kmer", u64p), ("total", u32p), ("max", u32p), ("files", u32p)]
+
+
+def _sdk_lib():
+    lib = load_library()
+    P = C.c_void_p
+    lib.hga_sdk_count_packed.argtypes = [C.c_int, C.c_int, P, C.c_uint64, P, C.c_uint64, P, P, C.c_uint64, C.c_int, P, C.c_uint32, C.POINTER(C.c_void_p)]
+    lib.hga_sdk_size.argtypes = [P, C.POINTER(C.c_uint64)]
+    lib.hga_sdk_specificity.argtypes = [P, P, C.c_int, P, P, P, C.c_uint64, C.POINTER(C.c_uint64)]
+    lib.hga_sdk_range.argtypes = [P, C.c_uint32, C.c_uint32, C.POINTER(_SdkRange)]
+    lib.hga_free_sdk_range.argtypes = [C.POINTER(_SdkRange)]
+    lib.hga_free_sdk_range.restype = None
+    lib.hga_sdk_free.argtypes = [P]
+    lib.hga_sdk_free.restype = None
+    return lib
+
+
+class SdkTable:
+    """The merged k-mer table of sdk_count_packed, held in device memory until close() (or the end of a `with` block)."""
+
+    def __init__(self, ptr):
+        self._p = ptr
+        n = C.c_uint64()
+        _check(_sdk_lib().hga_sdk_size(self._p, C.byref(n)))
+        self.n = int(n.value)
+
+    def specificity(self, thresholds=SDK_THRESHOLDS):
+        """hga_sdk_specificity: the rows of sdk_specificity on the merged table (upper specificity, total count, number of k-mers)"""
+        lib = _sdk_lib()
+        P = C.c_void_p
+        thr = np.ascontiguousarray(thresholds, dtype=np.float64)
+        n = C.c_uint64()
+        _check(lib.hga_sdk_specificity(self._p, thr.ctypes.data_as(P), thr.shape[0], None, None, None, 0, C.byref(n)))
+        cap = max(n.value, 1)
+        ot = np.zeros(cap, dtype=np.float64); oo = np.zeros(cap, dtype=np.uint32); ou = np.zeros(cap, dtype=np.uint64)
+        _check(lib.hga_sdk_specificity(self._p, thr.ctypes.data_as(P), thr.shape[0], ot.ctypes.data_as(P), oo.ctypes.data_as(P), ou.ctypes.data_as(P), cap,
+                                       C.byref(n)))
+        return ot[:n.value], oo[:n.value], ou[:n.value]
+
+    def range(self, lower=0, upper=0xFFFFFFFF):
+        """hga_sdk_range: (k-mers ascending, total, largest per-file count, files) of the entries with lower <= total <= upper"""
+        lib = _sdk_lib()
+        out = _SdkRange()
+        _check(lib.hga_sdk_range(self._p, int(lower), int(upper), C.byref(out)))
+        try:
+            return (_arr(out.kmer, out.n, np.uint64), _arr(out.total, out.n, np.uint32), _arr(out.max, out.n, np.uint32),
+                    _arr(out.files, out.n, np.uint32))
+        finally:
+            lib.hga_free_sdk_range(C.byref(out))
+
+    def close(self):
+        if self._p:
+            _sdk_lib().hga_sdk_free(self._p)
+            self._p = None
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    def __del__(self):
+        self.close()
+
+
+def sdk_count_packed(packed, read_off, exc_start, exc_end, k, file_first_read, min_count=2, first_base=0, device=0):
+    """hga_sdk_count_packed: the read set of count_kmers_packed cut into files (file f = reads file_first_read[f] ..
+    file_first_read[f + 1]), every file counted with min_count and the files merged on the GPU. Returns an SdkTable holding what
+    sdk_merge returns on the per-file count_kmers_packed lists."""
+    lib = _sdk_lib()
+    P = C.c_void_p
+    keep, ptr, _ = _host_bytes(packed)
+    ro = np.ascontiguousarray(read_off, dtype=np.uint64)
+    st = np.ascontiguousarray(exc_start, dtype=np.uint64); en = np.ascontiguousarray(exc_end, dtype=np.uint64)
+    ff = np.ascontiguousarray(file_first_read, dtype=np.uint64)
+    out = C.c_void_p()
+    _check(lib.hga_sdk_count_packed(int(device), int(k), ptr, int(first_base), ro.ctypes.data_as(P), ro.shape[0] - 1, st.ctypes.data_as(P), en.ctypes.data_as(P),
+                                    st.shape[0], ff.shape[0] - 1, ff.ctypes.data_as(P), int(min_count), C.byref(out)))
+    del keep
+    return SdkTable(out.value)
 
 
 def host_tail_connections(row_off, kmer_id, pos, read_len, avg_read_length, comp_off, comp_member, tree_off, tree_x, tree_y, purged_off, purged_read,

@@ -5,11 +5,12 @@
 //
 // Same options as jellyfish_occurrences.cpp:22-30 (read_paths, --k-size / -k, --output / -o, --help). Where the reference shells out
 // to jellyfish once per read file (occurrences/run_jellyfish.sh) this program counts the canonical k-mers of every file on the GPU
-// (hga_count_kmers_packed: exact counts, k-mers seen at least twice). The reads are packed while they load, in the case-folded 2-bit
-// form (lowercase a c g t are bases, as for jellyfish; other bytes travel as exception runs), so a quarter of the bytes crosses to the
-// GPU; a file is counted in place as a slice of that stream, with its runs clipped to the slice and rebased. The counts equal
-// hga_count_kmers on the ASCII bytes, so every output is unchanged. The merge of the per-file lists, the specificity table and the
-// export of a count range are the reader's host arithmetic (hga_host_sdk_*; JellyfishOccurrenceReader.cpp:63-134). Differences,
+// (exact counts, k-mers seen at least twice in the file). The reads are packed while they load, in the case-folded 2-bit form
+// (lowercase a c g t are bases, as for jellyfish; other bytes travel as exception runs), so a quarter of the bytes crosses to the GPU.
+// One call (hga_sdk_count_packed) counts every file and merges the files' counts on the GPU; the merged table stays there, the
+// specificity table is computed there (hga_sdk_specificity) and only the k-mers of the chosen count range come back (hga_sdk_range).
+// The results are those of the reader's host arithmetic on the per-file hga_count_kmers_packed lists (hga_host_sdk_merge /
+// _specificity; JellyfishOccurrenceReader.cpp:63-134), and the sampling stays on the host (hga_host_sdk_select on the range). Differences,
 // on purpose: the specificity table is printed as text (the reference pipes it into a Python plot, Plotting.cpp); without -k the k
 // sweep of get_unique_k_length (occurrences/KmerAnalysis.cpp:41-56: k = 11, 13, ... until the number of distinct k-mers changes by
 // less than 10 %) uses EXACT distinct counts instead of a HyperLogLog estimate (hga_count_spectrum_packed: the distinct count of every
@@ -86,11 +87,6 @@ int main(int argc, char **argv) {
         }
         return s;
     };
-    auto count = [&](int kk, size_t lo, size_t hi, uint32_t min_count, hga_kmer_counts_t *c) {
-        const Slice s = slice(lo, hi);
-        check(hga_count_kmers_packed(device, kk, reads.packed_data, s.b0, s.off.data(), hi - lo, s.es.data(), s.ee.data(), s.es.size(), min_count, c),
-              "hga_count_kmers_packed");
-    };
 
     if (k == 0) {
         // get_unique_k_length (KmerAnalysis.cpp:41-56) with exact distinct counts: the spectrum's totals, no k-mer leaves the GPU
@@ -114,31 +110,23 @@ int main(int argc, char **argv) {
         }
     }
 
-    // per file: exact canonical counts, k-mers seen at least twice (run_jellyfish.sh: bc + count --bc + dump + sort)
-    std::vector<uint64_t> file_off{0}, kmers;
-    std::vector<uint32_t> counts;
-    for (size_t f = 0; f + 1 < file_first.size(); f++) {
-        hga_kmer_counts_t c;
-        count(k, file_first[f], file_first[f + 1], 2, &c);
-        kmers.insert(kmers.end(), c.kmer, c.kmer + c.n);
-        counts.insert(counts.end(), c.count, c.count + c.n);
-        file_off.push_back(kmers.size());
-        hga_free_kmer_counts(&c);
+    // per file: exact canonical counts, k-mers seen at least twice (run_jellyfish.sh: bc + count --bc + dump + sort), merged over
+    // the files; the merged table stays on the GPU
+    hga_sdk *sdk = nullptr;
+    {
+        const Slice all = slice(0, reads.n_reads());
+        check(hga_sdk_count_packed(device, k, reads.packed_data, all.b0, all.off.data(), reads.n_reads(), all.es.data(), all.ee.data(), all.es.size(),
+                                   (int) (file_first.size() - 1), file_first.data(), 2, &sdk),
+              "hga_sdk_count_packed");
     }
-    const uint64_t cap = kmers.size() + 1;
-    std::vector<uint64_t> m_kmer(cap);
-    std::vector<uint32_t> m_total(cap), m_max(cap), m_files(cap);
-    uint64_t n = 0;
-    check(hga_host_sdk_merge((int) (file_off.size() - 1), file_off.data(), kmers.data(), counts.data(), m_kmer.data(), m_total.data(), m_max.data(), m_files.data(), &n),
-          "hga_host_sdk_merge");
 
     const double thresholds[] = {70, 85, 90, 95, 99, 100, 100.01};      // jellyfish_occurrences.cpp:47
     uint64_t rows = 0;
-    check(hga_host_sdk_specificity(n, m_total.data(), m_max.data(), thresholds, 7, nullptr, nullptr, nullptr, 0, &rows), "hga_host_sdk_specificity");
+    check(hga_sdk_specificity(sdk, thresholds, 7, nullptr, nullptr, nullptr, 0, &rows), "hga_sdk_specificity");
     std::vector<double> s_thr(rows + 1);
     std::vector<uint32_t> s_occ(rows + 1);
     std::vector<uint64_t> s_cnt(rows + 1);
-    check(hga_host_sdk_specificity(n, m_total.data(), m_max.data(), thresholds, 7, s_thr.data(), s_occ.data(), s_cnt.data(), rows, &rows), "hga_host_sdk_specificity");
+    check(hga_sdk_specificity(sdk, thresholds, 7, s_thr.data(), s_occ.data(), s_cnt.data(), rows, &rows), "hga_sdk_specificity");
     std::cout << "# k = " << k << ": upper specificity, occurrences, unique k-mers\n";
     for (uint64_t i = 0; i < rows; i++) std::printf("%.2f %u %llu\n", s_thr[i], s_occ[i], (unsigned long long) s_cnt[i]);
     std::fflush(stdout);
@@ -152,13 +140,19 @@ int main(int argc, char **argv) {
         std::snprintf(buf, sizeof buf, "%d-mers_%d_%d_%g%%.txt", k, lower, upper, percent * 100);      // :57
         output_path = buf;
     }
-    std::vector<uint8_t> sel(n + 1);
+    // only the k-mers of the count range come back; the sampler draws for in-range k-mers only, in ascending order, so it keeps the
+    // same ones as on the whole merged table
+    const uint32_t lo = (uint32_t) std::max(lower, 0), hi = (uint32_t) std::max(upper, 0);
+    hga_sdk_range_t r;
+    check(hga_sdk_range(sdk, lo, hi, &r), "hga_sdk_range");
+    hga_sdk_free(sdk);
+    std::vector<uint8_t> sel(r.n + 1);
     uint64_t n_sel = 0, n_disc = 0;
-    check(hga_host_sdk_select(n, m_total.data(), m_files.data(), (uint32_t) std::max(lower, 0), (uint32_t) std::max(upper, 0), percent, seed, sel.data(), &n_sel, &n_disc),
-          "hga_host_sdk_select");
+    check(hga_host_sdk_select(r.n, r.total, r.files, lo, hi, percent, seed, sel.data(), &n_sel, &n_disc), "hga_host_sdk_select");
     std::ofstream out(output_path);
-    for (uint64_t i = 0; i < n; i++) if (sel[i]) out << number_to_sequence(m_kmer[i], k) << "\n";
+    for (uint64_t i = 0; i < r.n; i++) if (sel[i]) out << number_to_sequence(r.kmer[i], k) << "\n";
     out.close();
+    hga_free_sdk_range(&r);
     std::cout << n_disc << " out of " << n_sel << " exported kmers are discriminative\n";      // :132
     return 0;
 }

@@ -257,6 +257,26 @@ int hga_count_kmers_packed(int device, int k, const uint8_t *packed, uint64_t fi
     return hga_count_run("hga_count_kmers_packed", device, k, nullptr, packed, first_base, read_off, n_reads, exc_start, exc_end, n_exc, min_count, out, nullptr, 0, nullptr);
 }
 
+int hga_sdk_count_packed(int device, int k, const uint8_t *packed, uint64_t first_base, const uint64_t *read_off, uint64_t n_reads, const uint64_t *exc_start,
+                         const uint64_t *exc_end, uint64_t n_exc, int n_files, const uint64_t *file_first_read, uint32_t min_count, hga_sdk **out) {
+    if (!out) { hga_set_error("hga_sdk_count_packed: NULL argument"); return HGA_E_ARG; }
+    *out = nullptr;
+    if (!read_off) { hga_set_error("hga_sdk_count_packed: read_off is NULL"); return HGA_E_ARG; }
+    if (k < 1 || k > 32) { hga_set_error("Kmer size is too big or too small (k = %d)", k); return HGA_E_ARG; }
+    HGA_TRY(check_read_off("hga_sdk_count_packed", read_off, n_reads));
+    const uint64_t n_bases = read_off[n_reads];
+    if (n_bases && !packed) { hga_set_error("hga_sdk_count_packed: packed is NULL"); return HGA_E_ARG; }
+    HGA_TRY(check_exc_runs("hga_sdk_count_packed", exc_start, exc_end, n_exc, n_bases));
+    if (n_files < 1 || !file_first_read) { hga_set_error("hga_sdk_count_packed: %s", n_files < 1 ? "n_files must be at least 1" : "file_first_read is NULL"); return HGA_E_ARG; }
+    if (file_first_read[0] != 0 || file_first_read[n_files] != n_reads) {
+        hga_set_error("hga_sdk_count_packed: file_first_read must start at 0 and end at n_reads (%llu)", (unsigned long long) n_reads);
+        return HGA_E_ARG;
+    }
+    for (int f = 0; f < n_files; f++)
+        if (file_first_read[f + 1] < file_first_read[f]) { hga_set_error("hga_sdk_count_packed: file_first_read decreases at file %d", f); return HGA_E_ARG; }
+    return hga_sdk_run("hga_sdk_count_packed", device, k, packed, first_base, read_off, n_reads, exc_start, exc_end, n_exc, n_files, file_first_read, min_count, out);
+}
+
 int hga_count_spectrum_packed(int device, int k, const uint8_t *packed, uint64_t first_base, const uint64_t *read_off, uint64_t n_reads, const uint64_t *exc_start,
                               const uint64_t *exc_end, uint64_t n_exc, uint32_t n_bins, uint64_t *hist, hga_kmer_spectrum_t *out) {
     if (out) std::memset(out, 0, sizeof *out);

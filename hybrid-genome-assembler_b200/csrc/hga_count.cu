@@ -24,6 +24,14 @@
 // encode, filter, quantiles, range splitting) is shared with the ASCII input, so the results are the same values in the same order.
 // Spectrum mode (hga_count_spectrum[_packed]): the same emits, passes and sorts; count_spectrum_kernel then adds each pass's runs to a
 // device histogram and totals in place of the run-length encode, filter and D2H, so no k-mer leaves the device.
+// SDK mode (hga_sdk_count_packed: the read set cut into files): the same sample, key ranges, passes and splits over the whole stream.
+// A pass emits file by file, so file f's keys fill one contiguous segment (one pass: the segment of its bases; key-range passes: one
+// emit launch per file on its own rebased read_off and runs, the shared cursor snapshotted after each launch). Each segment is sorted,
+// run-length encoded and filtered (count >= min_count) on its own; the survivors, tagged (count, file), are sorted by k-mer together
+// and sdk_merge_kernel writes one (k-mer, total, max, files) entry per distinct k-mer into a device chunk of exactly that many entries.
+// A range split down to one k-mer gets its entry from the per-file cursor snapshots. hga_sdk_specificity (sdk_spec_kernel: dense
+// [threshold][total] bins for small totals, a sorted (threshold, total) list for the rest) and hga_sdk_range (count, then an exactly
+// sized select) run over the chunks; only the rows and the range come back to the host.
 #include "hga_internal.cuh"
 
 #include <algorithm>
@@ -33,6 +41,7 @@
 #include <cub/device/device_radix_sort.cuh>
 #include <cub/device/device_reduce.cuh>
 #include <cub/device/device_run_length_encode.cuh>
+#include <cub/device/device_scan.cuh>
 #include <cub/device/device_select.cuh>
 
 namespace {
@@ -303,16 +312,146 @@ __global__ void count_spectrum_kernel(const unsigned long long *__restrict__ s, 
 #endif
 }
 
+// ---- SDK selection (hga_sdk_*) ---------------------------------------------------------------------------------------------------
+// One file's runs of a pass (k-mer, count), n of them: flag[i] = the run is a k-mer (not the sentinel) seen at least min_count times,
+// tag[i] = its count in the high 32 bits and the file in the low 32 bits (what the merge needs once the files' runs are mixed).
+__global__ void sdk_tag_kernel(const unsigned long long *__restrict__ keys, const uint32_t *__restrict__ cnt, uint64_t n, uint32_t min_count, uint32_t file,
+                               uint8_t *__restrict__ flag, unsigned long long *__restrict__ tag) {
+    for (uint64_t i = blockIdx.x * (uint64_t) blockDim.x + threadIdx.x; i < n; i += (uint64_t) gridDim.x * blockDim.x) {
+        flag[i] = keys[i] != COUNT_SENTINEL && cnt[i] >= min_count;
+        tag[i] = ((unsigned long long) cnt[i] << 32) | file;
+    }
+}
+
+// The merge of one pass: distinct k-mer j = ukey[j] holds the tags [start[j], start[j] + len[j]) of the pass's tags sorted by k-mer, one
+// per file that keeps it, so at most n_files of them. Writes (k-mer, total, largest count, files) to entry j (j < capacity) and sets
+// *overflow when a total does not fit 32 bits.
+__global__ void sdk_merge_kernel(const unsigned long long *__restrict__ ukey, const uint32_t *__restrict__ len, const unsigned long long *__restrict__ start,
+                                 const unsigned long long *__restrict__ tag, uint64_t n_uniq, uint64_t n_tag, uint32_t n_files, unsigned long long *__restrict__ out_kmer,
+                                 uint32_t *__restrict__ out_total, uint32_t *__restrict__ out_max, uint32_t *__restrict__ out_files, uint64_t capacity,
+                                 unsigned long long *__restrict__ overflow) {
+    const uint64_t n = n_uniq < capacity ? n_uniq : capacity;
+    for (uint64_t j = blockIdx.x * (uint64_t) blockDim.x + threadIdx.x; j < n; j += (uint64_t) gridDim.x * blockDim.x) {
+        const uint64_t s = start[j], l = len[j] < n_files ? len[j] : n_files, e = s + l < n_tag ? s + l : n_tag;
+        unsigned long long total = 0;
+        uint32_t mx = 0, files = 0;
+        for (uint64_t i = s; i < e; i++) {
+            const uint32_t c = (uint32_t) (tag[i] >> 32);
+            total += c; mx = c > mx ? c : mx; files += c > 0;
+        }
+        if (total > 0xFFFFFFFFull) *overflow = 1;
+        out_kmer[j] = ukey[j]; out_total[j] = (uint32_t) total; out_max[j] = mx; out_files[j] = files;
+    }
+}
+
+// Specificity of n merged k-mers (entries base .. base + n of the table): bin = the first of the n_thr ascending thresholds strictly
+// greater than ((double) max / (double) total) * 100. COUNT pass: totals below dense_lim are added to dense[bin * dense_lim + total],
+// the others are counted in *cursor, and the smallest entry without a bin goes to *bad. FILL pass: the others are written as
+// bin << 32 | total to tail (below capacity).
+template<bool FILL>
+__global__ void sdk_spec_kernel(const uint32_t *__restrict__ total, const uint32_t *__restrict__ max, uint64_t n, const double *__restrict__ thr, uint32_t n_thr,
+                                uint32_t dense_lim, unsigned long long *__restrict__ dense, unsigned long long *__restrict__ tail, uint64_t capacity,
+                                unsigned long long *cursor, unsigned long long *bad, uint64_t base) {
+    for (uint64_t i = blockIdx.x * (uint64_t) blockDim.x + threadIdx.x; i < n; i += (uint64_t) gridDim.x * blockDim.x) {
+        const double v = ((double) max[i] / (double) total[i]) * 100;
+        uint32_t lo = 0, hi = n_thr;
+        while (lo < hi) { const uint32_t mid = (lo + hi) >> 1; if (thr[mid] > v) hi = mid; else lo = mid + 1; }
+        if (lo == n_thr) {
+            if (!FILL) {
+#ifdef __CUDA_ARCH__
+                atomicMin(bad, (unsigned long long) (base + i));
+#else
+                if (base + i < *bad) *bad = base + i;
+#endif
+            }
+            continue;
+        }
+        if (total[i] < dense_lim) {
+            if (!FILL) atomicAdd(&dense[(uint64_t) lo * dense_lim + total[i]], 1ull);
+            continue;
+        }
+        const unsigned long long at = atomicAdd(cursor, 1ull);
+        if (FILL && at < capacity) tail[at] = ((unsigned long long) lo << 32) | total[i];
+    }
+}
+
+// lower <= total[i] <= upper: flag[i] (when flag is not NULL), and the number of such entries added to *count
+__global__ void sdk_range_kernel(const uint32_t *__restrict__ total, uint64_t n, uint32_t lower, uint32_t upper, uint8_t *__restrict__ flag, unsigned long long *count) {
+    unsigned long long c = 0;
+    for (uint64_t i = blockIdx.x * (uint64_t) blockDim.x + threadIdx.x; i < n; i += (uint64_t) gridDim.x * blockDim.x) {
+        const bool in = lower <= total[i] && total[i] <= upper;
+        if (flag) flag[i] = in;
+        c += in;
+    }
+    if (c) atomicAdd(count, c);
+}
+
 struct Bufs {
-    DevBuf bases, off, exc, keys, sorted, run_key, run_len, acc_key2, acc_cnt2, tmp, scalars, flag, spectrum;
-    ~Bufs() { for (DevBuf *b : {&bases, &off, &exc, &keys, &sorted, &run_key, &run_len, &acc_key2, &acc_cnt2, &tmp, &scalars, &flag, &spectrum}) b->release(); }
+    DevBuf bases, off, exc, keys, sorted, run_key, run_len, acc_key2, acc_cnt2, tmp, scalars, flag, spectrum, f_off, f_exc, f_cnt, tag, sel_tag, m_key, m_tag, m_start;
+    ~Bufs() {
+        for (DevBuf *b : {&bases, &off, &exc, &keys, &sorted, &run_key, &run_len, &acc_key2, &acc_cnt2, &tmp, &scalars, &flag, &spectrum, &f_off, &f_exc, &f_cnt, &tag,
+                          &sel_tag, &m_key, &m_tag, &m_start})
+            b->release();
+    }
 };
 
+// the message of a k-mer whose count does not fit the 32-bit counts
+void count_too_many(const char *who, int k, unsigned long long kmer, unsigned long long m) {
+    char s[33];
+    for (int i = 0; i < k; i++) s[i] = "ACGT"[(kmer >> (2 * (k - 1 - i))) & 3];
+    s[k] = '\0';
+    hga_set_error("%s: k-mer %s occurs %llu times, more than a 32-bit count holds (2^32 - 1); hga_count_spectrum gives its exact count", who, s, m);
+}
+
 }  // namespace
+
+// The merged table of hga_sdk_count_packed: chunks in ascending k-mer order, each one device block of exactly its entries (one chunk
+// per key-range pass, plus one per range split down to a single k-mer). A chunk is never grown or copied once written.
+struct hga_sdk {
+    struct Chunk {
+        void *p;
+        uint64_t n;
+        unsigned long long *kmer() const { return (unsigned long long *) p; }
+        uint32_t *total() const { return (uint32_t *) (kmer() + n); }
+        uint32_t *max() const { return total() + n; }
+        uint32_t *files() const { return max() + n; }
+    };
+    int device = 0;
+    uint64_t n = 0;
+    std::vector<Chunk> chunks;
+    int add(uint64_t n_entries, Chunk *c) {            // a new chunk of n_entries entries, owned by the handle from here on
+        void *p = nullptr;
+        const cudaError_t e = cudaMalloc(&p, n_entries * 20);
+        if (e != cudaSuccess) { hga_set_error("cudaMalloc(%llu) failed: %s", (unsigned long long) n_entries * 20, cudaGetErrorString(e)); cudaGetLastError(); return HGA_E_NOMEM; }
+        chunks.push_back({p, n_entries});
+        n += n_entries;
+        *c = chunks.back();
+        return HGA_OK;
+    }
+};
+
+// the files of hga_sdk_count_packed: file f = reads [first[f], first[f + 1])
+struct SdkFiles {
+    int n;
+    const uint64_t *first;
+};
+
+static int count_run(const char *who, int device, int k, const char *bases, const uint8_t *packed, uint64_t first_base, const uint64_t *read_off,
+                     uint64_t n_reads, const uint64_t *exc_start, const uint64_t *exc_end, uint64_t n_exc, uint32_t min_count, hga_kmer_counts_t *out,
+                     hga_kmer_spectrum_t *spec, uint32_t n_bins, uint64_t *hist, const SdkFiles *files, hga_sdk *sdk);
 
 int hga_count_run(const char *who, int device, int k, const char *bases, const uint8_t *packed, uint64_t first_base, const uint64_t *read_off,
                   uint64_t n_reads, const uint64_t *exc_start, const uint64_t *exc_end, uint64_t n_exc, uint32_t min_count, hga_kmer_counts_t *out,
                   hga_kmer_spectrum_t *spec, uint32_t n_bins, uint64_t *hist) {
+    return count_run(who, device, k, bases, packed, first_base, read_off, n_reads, exc_start, exc_end, n_exc, min_count, out, spec, n_bins, hist, nullptr, nullptr);
+}
+
+// SDK mode (files != NULL, packed input): every pass's keys are emitted file by file into one contiguous segment per file, each
+// segment is counted on its own (sort, run-length encode, count >= min_count), and the files' runs are merged by k-mer on the device
+// into a new chunk of sdk; nothing per k-mer comes back to the host.
+static int count_run(const char *who, int device, int k, const char *bases, const uint8_t *packed, uint64_t first_base, const uint64_t *read_off,
+                     uint64_t n_reads, const uint64_t *exc_start, const uint64_t *exc_end, uint64_t n_exc, uint32_t min_count, hga_kmer_counts_t *out,
+                     hga_kmer_spectrum_t *spec, uint32_t n_bins, uint64_t *hist, const SdkFiles *files, hga_sdk *sdk) {
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) { cudaGetLastError(); hga_set_error("%s: no usable CUDA device (this library has no CPU path)", who); return HGA_E_CUDA; }
     HGA_CUDA(cudaSetDevice(device));
@@ -359,6 +498,89 @@ int hga_count_run(const char *who, int device, int k, const char *bases, const u
         HGA_TRY(b.spectrum.ensure((spec_bins + 3ull) * 8));
         HGA_CUDA(cudaMemsetAsync(b.spectrum.p, 0, (spec_bins + 3ull) * 8, st));
     }
+    // SDK mode: fb[f] = the first base of file f (relative to the read set); its keys of a one-pass run are keys[fb[f] .. fb[f + 1])
+    const uint32_t n_files = files ? (uint32_t) files->n : 0;
+    std::vector<uint64_t> fb(n_files + 1);
+    if (files) {
+        for (uint32_t f = 0; f <= n_files; f++) fb[f] = off[files->first[f]];
+        HGA_TRY(b.f_cnt.ensure(n_files * 8ull + 8));
+    }
+
+    // SDK mode: the keys of one pass, file f's in keys[seg[f] .. seg[f + 1]) -> the merged entries of the pass as a new chunk of sdk
+    auto merge_pass = [&](const std::vector<uint64_t> &seg) -> int {
+        const uint64_t m = seg[n_files];
+        if (m == 0) return HGA_OK;
+        HGA_TRY(b.sorted.ensure(m * 8)); HGA_TRY(b.run_key.ensure(m * 8)); HGA_TRY(b.run_len.ensure(m * 4));
+        HGA_TRY(b.flag.ensure(m + 16)); HGA_TRY(b.tag.ensure(m * 8));
+        unsigned long long *d_keys = b.keys.as<unsigned long long>(), *d_sorted = b.sorted.as<unsigned long long>(), *d_rk = b.run_key.as<unsigned long long>();
+        unsigned long long *d_fcnt = b.f_cnt.as<unsigned long long>(), *d_tag = b.tag.as<unsigned long long>();
+        uint32_t *d_rl = b.run_len.as<uint32_t>();
+        uint8_t *d_flag = b.flag.as<uint8_t>();
+        // each file on its own: its segment sorted and run-length encoded into the same positions of the run arrays (a segment of n keys
+        // has at most n runs), the number of runs to d_fcnt[f]
+        HGA_CUDA(cudaMemsetAsync(d_fcnt, 0, n_files * 8ull, st));
+        for (uint32_t f = 0; f < n_files; f++) {
+            const uint64_t s0 = seg[f], n = seg[f + 1] - seg[f];
+            if (n == 0) continue;
+            size_t t1 = 0, t2 = 0;
+            HGA_CUDA(cub::DeviceRadixSort::SortKeys(nullptr, t1, d_keys + s0, d_sorted + s0, n, 0, end_bit, st));
+            HGA_CUDA(cub::DeviceRunLengthEncode::Encode(nullptr, t2, d_sorted + s0, d_rk + s0, d_rl + s0, d_fcnt + f, n, st));
+            HGA_TRY(b.tmp.ensure(std::max(t1, t2) + 16));
+            HGA_CUDA(cub::DeviceRadixSort::SortKeys(b.tmp.p, t1, d_keys + s0, d_sorted + s0, n, 0, end_bit, st));
+            HGA_CUDA(cub::DeviceRunLengthEncode::Encode(b.tmp.p, t2, d_sorted + s0, d_rk + s0, d_rl + s0, d_fcnt + f, n, st));
+        }
+        HGA_CUDA(cudaGetLastError());
+        std::vector<unsigned long long> runs(n_files);
+        HGA_CUDA(cudaMemcpyAsync(runs.data(), d_fcnt, n_files * 8ull, cudaMemcpyDeviceToHost, st));
+        HGA_CUDA(cudaStreamSynchronize(st));
+        // the runs that reach min_count, tagged with count and file; the positions past a file's runs stay unflagged
+        HGA_CUDA(cudaMemsetAsync(d_flag, 0, m, st));
+        for (uint32_t f = 0; f < n_files; f++) {
+            const uint64_t r = std::min<uint64_t>(runs[f], seg[f + 1] - seg[f]);
+            if (r) sdk_tag_kernel<<<grid(r), 256, 0, st>>>(d_rk + seg[f], d_rl + seg[f], r, min_count, f, d_flag + seg[f], d_tag + seg[f]);
+        }
+        HGA_CUDA(cudaGetLastError());
+        HGA_TRY(b.acc_key2.ensure(m * 8)); HGA_TRY(b.sel_tag.ensure(m * 8));
+        unsigned long long *d_sk = b.acc_key2.as<unsigned long long>(), *d_st = b.sel_tag.as<unsigned long long>();
+        size_t t1 = 0, t2 = 0;
+        HGA_CUDA(cub::DeviceSelect::Flagged(nullptr, t1, d_rk, d_flag, d_sk, d_scal, m, st));
+        HGA_CUDA(cub::DeviceSelect::Flagged(nullptr, t2, d_tag, d_flag, d_st, d_scal + 3, m, st));
+        HGA_TRY(b.tmp.ensure(std::max(t1, t2) + 16));
+        HGA_CUDA(cub::DeviceSelect::Flagged(b.tmp.p, t1, d_rk, d_flag, d_sk, d_scal, m, st));
+        HGA_CUDA(cub::DeviceSelect::Flagged(b.tmp.p, t2, d_tag, d_flag, d_st, d_scal + 3, m, st));
+        HGA_CUDA(cudaGetLastError());
+        unsigned long long ns = 0;
+        HGA_CUDA(cudaMemcpyAsync(&ns, d_scal, 8, cudaMemcpyDeviceToHost, st));
+        HGA_CUDA(cudaStreamSynchronize(st));
+        if (ns == 0) return HGA_OK;
+        // the files' runs mixed and sorted by k-mer (a k-mer has one run per file that keeps it), then one entry per distinct k-mer
+        HGA_TRY(b.m_key.ensure(ns * 8)); HGA_TRY(b.m_tag.ensure(ns * 8));
+        unsigned long long *d_mk = b.m_key.as<unsigned long long>(), *d_mt = b.m_tag.as<unsigned long long>();
+        HGA_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, t1, d_sk, d_mk, d_st, d_mt, ns, 0, end_bit, st));
+        HGA_CUDA(cub::DeviceRunLengthEncode::Encode(nullptr, t2, d_mk, d_rk, d_rl, d_scal, ns, st));
+        HGA_TRY(b.tmp.ensure(std::max(t1, t2) + 16));
+        HGA_CUDA(cub::DeviceRadixSort::SortPairs(b.tmp.p, t1, d_sk, d_mk, d_st, d_mt, ns, 0, end_bit, st));
+        HGA_CUDA(cub::DeviceRunLengthEncode::Encode(b.tmp.p, t2, d_mk, d_rk, d_rl, d_scal, ns, st));
+        HGA_CUDA(cudaGetLastError());
+        unsigned long long nu = 0;
+        HGA_CUDA(cudaMemcpyAsync(&nu, d_scal, 8, cudaMemcpyDeviceToHost, st));
+        HGA_CUDA(cudaStreamSynchronize(st));
+        HGA_TRY(b.m_start.ensure(nu * 8));
+        unsigned long long *d_ms = b.m_start.as<unsigned long long>();
+        HGA_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, t1, d_rl, d_ms, nu, st));
+        HGA_TRY(b.tmp.ensure(t1 + 16));
+        HGA_CUDA(cub::DeviceScan::ExclusiveSum(b.tmp.p, t1, d_rl, d_ms, nu, st));
+        hga_sdk::Chunk c;
+        HGA_TRY(sdk->add(nu, &c));
+        HGA_CUDA(cudaMemsetAsync(d_scal + 2, 0, 8, st));
+        sdk_merge_kernel<<<grid(nu), 256, 0, st>>>(d_rk, d_rl, d_ms, d_mt, nu, ns, n_files, c.kmer(), c.total(), c.max(), c.files(), c.n, d_scal + 2);
+        HGA_CUDA(cudaGetLastError());
+        unsigned long long overflow = 0;
+        HGA_CUDA(cudaMemcpyAsync(&overflow, d_scal + 2, 8, cudaMemcpyDeviceToHost, st));
+        HGA_CUDA(cudaStreamSynchronize(st));
+        if (overflow) { hga_set_error("%s: total count overflows 32 bits", who); return HGA_E_OVERFLOW; }
+        return HGA_OK;
+    };
 
     // m unsorted keys in b.keys -> sorted runs -> (k-mer, count >= min_count, sentinel dropped) appended to the host result, or in
     // spectrum mode the runs added to the device spectrum
@@ -420,7 +642,8 @@ int hga_count_run(const char *who, int device, int k, const char *bases, const u
                                                                                                                     n_bases, nullptr);
         else
             count_emit_kernel<<<grid(n_bases), 256, 0, st>>>(b.bases.as<char>(), b.off.as<uint64_t>(), n_reads, k, 0, n_bases, b.keys.as<unsigned long long>());
-        HGA_TRY(finish_pass(n_bases));
+        if (files) HGA_TRY(merge_pass(fb));       // the reads of a file are contiguous, so are the keys (and sentinels) of its windows
+        else HGA_TRY(finish_pass(n_bases));
     } else {
         // key-range passes. Quantiles of the key distribution from a strided sample of the windows (about 2^24 of them, all of them when the input is small)
         HGA_TRY(b.keys.ensure(B * 8));
@@ -457,11 +680,81 @@ int hga_count_run(const char *who, int device, int k, const char *bases, const u
         std::vector<std::pair<unsigned long long, unsigned long long>> todo;
         uint64_t passes = 0, splits = 0;
         for (uint64_t r = n_ranges; r-- > 0;) if (cut[r] < cut[r + 1]) todo.push_back({cut[r], cut[r + 1]});
+        // SDK mode: every file as a read set of its own (read_off rebased to its first base, its runs clipped to it and rebased),
+        // uploaded once; after file f's emit the cursor is copied to d_snap[f], so file f's keys of a pass are keys[snap[f - 1] .. snap[f])
+        std::vector<uint64_t> f_off_at(n_files + 1, 0), f_exc_at(n_files + 1, 0), snap(n_files + 1, 0);
+        unsigned long long *d_snap = b.f_cnt.as<unsigned long long>();
+        const uint64_t *d_foff = nullptr, *d_fxs = nullptr, *d_fxe = nullptr;
+        if (files) {
+            std::vector<uint64_t> f_off, f_es, f_ee;
+            f_off.reserve(n_reads + n_files);
+            for (uint32_t f = 0; f < n_files; f++) {
+                f_off_at[f] = f_off.size();
+                for (uint64_t i = files->first[f]; i <= files->first[f + 1]; i++) f_off.push_back(off[i] - fb[f]);
+                f_exc_at[f] = f_es.size();
+                for (uint64_t j = (uint64_t) (std::upper_bound(exc_end, exc_end + n_exc, fb[f]) - exc_end); j < n_exc && exc_start[j] < fb[f + 1]; j++) {
+                    f_es.push_back(std::max(exc_start[j], fb[f]) - fb[f]);
+                    f_ee.push_back(std::min(exc_end[j], fb[f + 1]) - fb[f]);
+                }
+            }
+            f_off_at[n_files] = f_off.size(); f_exc_at[n_files] = f_es.size();
+            HGA_TRY(b.f_off.ensure(f_off.size() * 8 + 8)); HGA_TRY(b.f_exc.ensure(f_es.size() * 16 + 16));
+            HGA_CUDA(cudaMemcpy(b.f_off.p, f_off.data(), f_off.size() * 8, cudaMemcpyHostToDevice));
+            if (!f_es.empty()) {
+                HGA_CUDA(cudaMemcpy(b.f_exc.p, f_es.data(), f_es.size() * 8, cudaMemcpyHostToDevice));
+                HGA_CUDA(cudaMemcpy(b.f_exc.as<uint64_t>() + f_es.size(), f_ee.data(), f_ee.size() * 8, cudaMemcpyHostToDevice));
+            }
+            d_foff = b.f_off.as<uint64_t>(); d_fxs = b.f_exc.as<uint64_t>(); d_fxe = d_fxs + f_es.size();
+        }
         while (!todo.empty()) {
             const unsigned long long lo = todo.back().first, hi = todo.back().second;
             todo.pop_back();
             passes++;
             HGA_CUDA(cudaMemsetAsync(d_scal + 1, 0, 8, st));
+            if (files) {
+                for (uint32_t f = 0; f < n_files; f++) {
+                    const uint64_t nb = fb[f + 1] - fb[f], g0 = sub + fb[f];
+                    if (nb)
+                        count_emit_packed_kernel<true><<<grid((nb + COUNT_PACKED_SPAN - 1) / COUNT_PACKED_SPAN), 256, 0, st>>>(d_words + (g0 >> 4), (uint32_t) (g0 & 15), d_foff + f_off_at[f],
+                                                                                                                        files->first[f + 1] - files->first[f], d_fxs + f_exc_at[f],
+                                                                                                                        d_fxe + f_exc_at[f], f_exc_at[f + 1] - f_exc_at[f], k, nb,
+                                                                                                                        COUNT_PACKED_SPAN, 1, lo, hi, b.keys.as<unsigned long long>(), B,
+                                                                                                                        d_scal + 1);
+                    HGA_CUDA(cudaMemcpyAsync(d_snap + f, d_scal + 1, 8, cudaMemcpyDeviceToDevice, st));
+                }
+                HGA_CUDA(cudaGetLastError());
+                HGA_CUDA(cudaMemcpyAsync(snap.data() + 1, d_snap, n_files * 8ull, cudaMemcpyDeviceToHost, st));
+                HGA_CUDA(cudaStreamSynchronize(st));
+                const unsigned long long m = snap[n_files];
+                if (m <= B) { HGA_TRY(merge_pass(snap)); continue; }
+                if (hi - lo > 1) {
+                    splits++;
+                    const unsigned long long mid = lo + (hi - lo) / 2;
+                    todo.push_back({mid, hi});
+                    todo.push_back({lo, mid});
+                    continue;
+                }
+                // one k-mer, seen snap[f + 1] - snap[f] times in file f: its merged entry is built here, a chunk of its own
+                unsigned long long total = 0;
+                uint32_t mx = 0, nf = 0;
+                for (uint32_t f = 0; f < n_files; f++) {
+                    const unsigned long long c = snap[f + 1] - snap[f];
+                    if (c > 0xFFFFFFFFull) { count_too_many(who, k, lo, c); return HGA_E_OVERFLOW; }
+                    if (c == 0 || c < min_count) continue;
+                    total += c; mx = std::max<uint32_t>(mx, (uint32_t) c); nf++;
+                }
+                if (nf == 0) continue;
+                if (total > 0xFFFFFFFFull) { hga_set_error("%s: total count overflows 32 bits", who); return HGA_E_OVERFLOW; }
+                hga_sdk::Chunk c;
+                HGA_TRY(sdk->add(1, &c));
+                const unsigned long long key = lo;
+                const uint32_t tot = (uint32_t) total;
+                HGA_CUDA(cudaMemcpy(c.kmer(), &key, 8, cudaMemcpyHostToDevice));
+                HGA_CUDA(cudaMemcpy(c.total(), &tot, 4, cudaMemcpyHostToDevice));
+                HGA_CUDA(cudaMemcpy(c.max(), &mx, 4, cudaMemcpyHostToDevice));
+                HGA_CUDA(cudaMemcpy(c.files(), &nf, 4, cudaMemcpyHostToDevice));
+                continue;
+            }
             if (packed)
                 count_emit_packed_kernel<true><<<grid((n_bases + COUNT_PACKED_SPAN - 1) / COUNT_PACKED_SPAN), 256, 0, st>>>(d_words, sub, d_off, n_reads, d_xs, d_xe, n_exc, k, n_bases,
                                                                                                                        COUNT_PACKED_SPAN, 1, lo, hi, b.keys.as<unsigned long long>(), B,
@@ -479,14 +772,7 @@ int hga_count_run(const char *who, int device, int k, const char *bases, const u
                         if (n_bins) hist[std::min<uint64_t>(m, n_bins) - 1]++;
                         continue;
                     }
-                    if (m > 0xFFFFFFFFull) {                                 // the counts are 32-bit: refuse rather than clip
-                        char s[33];
-                        for (int i = 0; i < k; i++) s[i] = "ACGT"[(lo >> (2 * (k - 1 - i))) & 3];
-                        s[k] = '\0';
-                        hga_set_error("%s: k-mer %s occurs %llu times, more than a 32-bit count holds (2^32 - 1); hga_count_spectrum gives its exact count",
-                                      who, s, m);
-                        return HGA_E_OVERFLOW;
-                    }
+                    if (m > 0xFFFFFFFFull) { count_too_many(who, k, lo, m); return HGA_E_OVERFLOW; }      // the counts are 32-bit: refuse rather than clip
                     if (m >= min_count) { res_k.push_back(lo); res_c.push_back((uint32_t) m); }
                     continue;
                 }
@@ -508,6 +794,7 @@ int hga_count_run(const char *who, int device, int k, const char *bases, const u
         for (uint32_t i = 0; i < spec_bins; i++) hist[i] += h[3 + i];
         return HGA_OK;
     }
+    if (files) return HGA_OK;
     const uint64_t n_out = res_k.size();
     uint64_t *hk = (uint64_t *) std::malloc((n_out + 1) * 8);
     uint32_t *hc = (uint32_t *) std::malloc((n_out + 1) * 4);
@@ -539,4 +826,191 @@ extern "C" void hga_free_kmer_counts(hga_kmer_counts_t *c) {
     if (!c) return;
     std::free((void *) c->kmer); std::free((void *) c->count);
     c->kmer = nullptr; c->count = nullptr; c->n = 0;
+}
+
+// ---- SDK selection handle -----------------------------------------------------------------------------------------------------------
+extern "C" void hga_sdk_free(hga_sdk *s) {
+    if (!s) return;
+    if (!s->chunks.empty()) cudaSetDevice(s->device);
+    for (const hga_sdk::Chunk &c : s->chunks) cudaFree(c.p);
+    delete s;
+}
+
+// the device half of hga_sdk_count_packed (hga_capi.cu checks the arguments): on failure nothing is left on the device
+int hga_sdk_run(const char *who, int device, int k, const uint8_t *packed, uint64_t first_base, const uint64_t *read_off, uint64_t n_reads,
+                const uint64_t *exc_start, const uint64_t *exc_end, uint64_t n_exc, int n_files, const uint64_t *file_first, uint32_t min_count, hga_sdk **out) {
+    hga_sdk *s = new hga_sdk;
+    s->device = device;
+    const SdkFiles files{n_files, file_first};
+    const int rc = count_run(who, device, k, nullptr, packed, first_base, read_off, n_reads, exc_start, exc_end, n_exc, min_count, nullptr, nullptr, 0, nullptr, &files, s);
+    if (rc != HGA_OK) { hga_sdk_free(s); return rc; }
+    *out = s;
+    return HGA_OK;
+}
+
+extern "C" int hga_sdk_size(const hga_sdk *s, uint64_t *n_kmers) {
+    if (!s || !n_kmers) { hga_set_error("hga_sdk_size: NULL argument"); return HGA_E_ARG; }
+    *n_kmers = s->n;
+    return HGA_OK;
+}
+
+// Bins of hga_host_sdk_specificity on the device: totals below dense_lim in a dense [bin][total] table, larger totals as a sorted list
+// of (bin, total) keys run-length encoded; rows in (threshold, total) order, as the reference's nested std::map gives them.
+extern "C" int hga_sdk_specificity(const hga_sdk *s, const double *thresholds, int n_thresholds, double *out_threshold, uint32_t *out_occurrences,
+                                   uint64_t *out_unique, uint64_t capacity, uint64_t *out_n) {
+    if (!s || !out_n || n_thresholds < 1 || !thresholds) { hga_set_error("hga_sdk_specificity: bad argument"); return HGA_E_ARG; }
+    for (int i = 0; i < n_thresholds; i++)
+        if (thresholds[i] != thresholds[i]) { hga_set_error("hga_sdk_specificity: threshold %d is NaN", i); return HGA_E_ARG; }
+    std::vector<double> thr(thresholds, thresholds + n_thresholds);         // ascending, without repeats: the bins of the table
+    std::sort(thr.begin(), thr.end());
+    thr.erase(std::unique(thr.begin(), thr.end()), thr.end());
+    *out_n = 0;
+    if (s->n == 0) return HGA_OK;
+    HGA_CUDA(cudaSetDevice(s->device));
+    cudaStream_t st = nullptr;
+    const uint32_t n_thr = (uint32_t) thr.size(), dense_lim = n_thr <= 64 ? 65536u : 256u;
+    int sm = 148;
+    cudaDeviceGetAttribute(&sm, cudaDevAttrMultiProcessorCount, s->device);
+    auto grid = [&](uint64_t n) { return (int) std::max<uint64_t>(1, std::min<uint64_t>((n + 255) / 256, (uint64_t) sm * 16)); };
+    Bufs b;
+    HGA_TRY(b.acc_key2.ensure(n_thr * 8ull)); HGA_TRY(b.spectrum.ensure((uint64_t) n_thr * dense_lim * 8)); HGA_TRY(b.scalars.ensure(64));
+    const double *d_thr = b.acc_key2.as<double>();
+    unsigned long long *d_dense = b.spectrum.as<unsigned long long>(), *d_scal = b.scalars.as<unsigned long long>();
+    HGA_CUDA(cudaMemcpy(b.acc_key2.p, thr.data(), n_thr * 8ull, cudaMemcpyHostToDevice));
+    HGA_CUDA(cudaMemsetAsync(d_dense, 0, (uint64_t) n_thr * dense_lim * 8, st));
+    HGA_CUDA(cudaMemsetAsync(d_scal, 0, 8, st));
+    HGA_CUDA(cudaMemsetAsync(d_scal + 1, 0xFF, 8, st));
+    uint64_t base = 0;
+    for (const hga_sdk::Chunk &c : s->chunks) {
+        sdk_spec_kernel<false><<<grid(c.n), 256, 0, st>>>(c.total(), c.max(), c.n, d_thr, n_thr, dense_lim, d_dense, nullptr, 0, d_scal, d_scal + 1, base);
+        base += c.n;
+    }
+    HGA_CUDA(cudaGetLastError());
+    unsigned long long h[2] = {0, 0};
+    HGA_CUDA(cudaMemcpyAsync(h, d_scal, 16, cudaMemcpyDeviceToHost, st));
+    HGA_CUDA(cudaStreamSynchronize(st));
+    if (h[1] != ~0ull) {                                                     // the first k-mer without a bin, as the host loop meets it
+        uint64_t i = h[1];
+        for (const hga_sdk::Chunk &c : s->chunks) {
+            if (i >= c.n) { i -= c.n; continue; }
+            uint32_t t = 0, m = 0;
+            HGA_CUDA(cudaMemcpy(&t, c.total() + i, 4, cudaMemcpyDeviceToHost));
+            HGA_CUDA(cudaMemcpy(&m, c.max() + i, 4, cudaMemcpyDeviceToHost));
+            const double v = ((double) m / (double) t) * 100;
+            hga_set_error("hga_sdk_specificity: no threshold above %.4f (the reference dereferences end() here)", v);
+            return HGA_E_ARG;
+        }
+    }
+    // the totals of dense_lim and more: (bin, total) keys, exactly as many as counted, sorted and run-length encoded
+    const unsigned long long n_tail = h[0];
+    std::vector<unsigned long long> t_key, t_len;
+    if (n_tail) {
+        HGA_TRY(b.keys.ensure(n_tail * 8)); HGA_TRY(b.sorted.ensure(n_tail * 8)); HGA_TRY(b.run_key.ensure(n_tail * 8)); HGA_TRY(b.run_len.ensure(n_tail * 4));
+        unsigned long long *d_keys = b.keys.as<unsigned long long>(), *d_sorted = b.sorted.as<unsigned long long>(), *d_rk = b.run_key.as<unsigned long long>();
+        uint32_t *d_rl = b.run_len.as<uint32_t>();
+        HGA_CUDA(cudaMemsetAsync(d_scal, 0, 8, st));
+        for (const hga_sdk::Chunk &c : s->chunks)
+            sdk_spec_kernel<true><<<grid(c.n), 256, 0, st>>>(c.total(), c.max(), c.n, d_thr, n_thr, dense_lim, d_dense, d_keys, n_tail, d_scal, d_scal + 1, 0);
+        HGA_CUDA(cudaGetLastError());
+        size_t t1 = 0, t2 = 0;
+        HGA_CUDA(cub::DeviceRadixSort::SortKeys(nullptr, t1, d_keys, d_sorted, n_tail, 0, 64, st));
+        HGA_CUDA(cub::DeviceRunLengthEncode::Encode(nullptr, t2, d_sorted, d_rk, d_rl, d_scal + 2, n_tail, st));
+        HGA_TRY(b.tmp.ensure(std::max(t1, t2) + 16));
+        HGA_CUDA(cub::DeviceRadixSort::SortKeys(b.tmp.p, t1, d_keys, d_sorted, n_tail, 0, 64, st));
+        HGA_CUDA(cub::DeviceRunLengthEncode::Encode(b.tmp.p, t2, d_sorted, d_rk, d_rl, d_scal + 2, n_tail, st));
+        HGA_CUDA(cudaGetLastError());
+        unsigned long long nr = 0;
+        HGA_CUDA(cudaMemcpyAsync(&nr, d_scal + 2, 8, cudaMemcpyDeviceToHost, st));
+        HGA_CUDA(cudaStreamSynchronize(st));
+        t_key.resize(nr);
+        std::vector<uint32_t> l32(nr);
+        if (nr) {
+            HGA_CUDA(cudaMemcpy(t_key.data(), d_rk, nr * 8, cudaMemcpyDeviceToHost));
+            HGA_CUDA(cudaMemcpy(l32.data(), d_rl, nr * 4, cudaMemcpyDeviceToHost));
+        }
+        t_len.assign(l32.begin(), l32.end());     // a (bin, total) run holds k-mers seen dense_lim times or more: far fewer than 2^32 of them
+    }
+    std::vector<unsigned long long> dense((uint64_t) n_thr * dense_lim);
+    HGA_CUDA(cudaMemcpy(dense.data(), d_dense, dense.size() * 8, cudaMemcpyDeviceToHost));
+    uint64_t m = 0, j = 0;
+    auto row = [&](double t, uint32_t occ, uint64_t cnt) {
+        if (m < capacity && out_threshold && out_occurrences && out_unique) { out_threshold[m] = t; out_occurrences[m] = occ; out_unique[m] = cnt; }
+        m++;
+    };
+    for (uint32_t bin = 0; bin < n_thr; bin++) {
+        for (uint32_t t = 0; t < dense_lim; t++)
+            if (dense[(uint64_t) bin * dense_lim + t]) row(thr[bin], t, dense[(uint64_t) bin * dense_lim + t]);
+        for (; j < t_key.size() && (t_key[j] >> 32) == bin; j++) row(thr[bin], (uint32_t) t_key[j], t_len[j]);
+    }
+    *out_n = m;                                                              // > capacity: call again with more room
+    return HGA_OK;
+}
+
+extern "C" int hga_sdk_range(const hga_sdk *s, uint32_t lower, uint32_t upper, hga_sdk_range_t *out) {
+    if (!out) { hga_set_error("hga_sdk_range: NULL argument"); return HGA_E_ARG; }
+    std::memset(out, 0, sizeof *out);
+    if (!s) { hga_set_error("hga_sdk_range: NULL argument"); return HGA_E_ARG; }
+    std::vector<unsigned long long> cnt(s->chunks.size() + 1, 0);
+    Bufs b;
+    cudaStream_t st = nullptr;
+    int sm = 148;
+    auto grid = [&](uint64_t n) { return (int) std::max<uint64_t>(1, std::min<uint64_t>((n + 255) / 256, (uint64_t) sm * 16)); };
+    unsigned long long n_out = 0;
+    if (lower <= upper && s->n) {
+        HGA_CUDA(cudaSetDevice(s->device));
+        cudaDeviceGetAttribute(&sm, cudaDevAttrMultiProcessorCount, s->device);
+        // count per chunk, then fill arrays of exactly that size
+        HGA_TRY(b.scalars.ensure(cnt.size() * 8 + 8));
+        unsigned long long *d_cnt = b.scalars.as<unsigned long long>();
+        HGA_CUDA(cudaMemsetAsync(d_cnt, 0, cnt.size() * 8, st));
+        uint64_t largest = 0;
+        for (size_t i = 0; i < s->chunks.size(); i++) {
+            const hga_sdk::Chunk &c = s->chunks[i];
+            sdk_range_kernel<<<grid(c.n), 256, 0, st>>>(c.total(), c.n, lower, upper, nullptr, d_cnt + i);
+            largest = std::max<uint64_t>(largest, c.n);
+        }
+        HGA_CUDA(cudaGetLastError());
+        HGA_CUDA(cudaMemcpyAsync(cnt.data(), d_cnt, s->chunks.size() * 8, cudaMemcpyDeviceToHost, st));
+        HGA_CUDA(cudaStreamSynchronize(st));
+        for (size_t i = 0; i < s->chunks.size(); i++) n_out += cnt[i];
+        if (n_out) {
+            HGA_TRY(b.flag.ensure(largest + 16)); HGA_TRY(b.keys.ensure(n_out * 8)); HGA_TRY(b.run_len.ensure(n_out * 12));
+            unsigned long long *d_k = b.keys.as<unsigned long long>();
+            uint32_t *d_t = b.run_len.as<uint32_t>(), *d_m = d_t + n_out, *d_f = d_m + n_out;
+            uint8_t *d_flag = b.flag.as<uint8_t>();
+            unsigned long long *d_ns = d_cnt + s->chunks.size();
+            uint64_t at = 0;
+            for (size_t i = 0; i < s->chunks.size(); i++) {
+                const hga_sdk::Chunk &c = s->chunks[i];
+                if (!cnt[i]) continue;
+                sdk_range_kernel<<<grid(c.n), 256, 0, st>>>(c.total(), c.n, lower, upper, d_flag, d_ns);
+                size_t t1 = 0, t2 = 0;
+                HGA_CUDA(cub::DeviceSelect::Flagged(nullptr, t1, c.kmer(), d_flag, d_k + at, d_ns, c.n, st));
+                HGA_CUDA(cub::DeviceSelect::Flagged(nullptr, t2, c.total(), d_flag, d_t + at, d_ns, c.n, st));
+                HGA_TRY(b.tmp.ensure(std::max(t1, t2) + 16));
+                HGA_CUDA(cub::DeviceSelect::Flagged(b.tmp.p, t1, c.kmer(), d_flag, d_k + at, d_ns, c.n, st));
+                HGA_CUDA(cub::DeviceSelect::Flagged(b.tmp.p, t2, c.total(), d_flag, d_t + at, d_ns, c.n, st));
+                HGA_CUDA(cub::DeviceSelect::Flagged(b.tmp.p, t2, c.max(), d_flag, d_m + at, d_ns, c.n, st));
+                HGA_CUDA(cub::DeviceSelect::Flagged(b.tmp.p, t2, c.files(), d_flag, d_f + at, d_ns, c.n, st));
+                HGA_CUDA(cudaGetLastError());
+                at += cnt[i];
+            }
+        }
+    }
+    uint64_t *hk = (uint64_t *) std::malloc((n_out + 1) * 8);
+    uint32_t *ht = (uint32_t *) std::malloc((n_out + 1) * 12);
+    if (!hk || !ht) { std::free(hk); std::free(ht); hga_set_error("hga_sdk_range: out of host memory"); return HGA_E_NOMEM; }
+    if (n_out) {
+        cudaError_t e = cudaMemcpy(hk, b.keys.p, n_out * 8, cudaMemcpyDeviceToHost);
+        for (int a = 0; a < 3 && e == cudaSuccess; a++) e = cudaMemcpy(ht + a * (n_out + 1), b.run_len.as<uint32_t>() + a * n_out, n_out * 4, cudaMemcpyDeviceToHost);
+        if (e != cudaSuccess) { std::free(hk); std::free(ht); hga_set_error("hga_sdk_range: copy to the host failed: %s", cudaGetErrorString(e)); return HGA_E_CUDA; }
+    }
+    out->n = n_out; out->kmer = hk; out->total = ht; out->max = ht + n_out + 1; out->files = ht + 2 * (n_out + 1);
+    return HGA_OK;
+}
+
+extern "C" void hga_free_sdk_range(hga_sdk_range_t *r) {
+    if (!r) return;
+    std::free((void *) r->kmer); std::free((void *) r->total);      // total, max and files share one block
+    std::memset(r, 0, sizeof *r);
 }

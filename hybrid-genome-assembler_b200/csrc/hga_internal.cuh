@@ -369,6 +369,8 @@ int hga_scan_finish_positions(hga_handle *h);
 int hga_count_run(const char *who, int device, int k, const char *bases, const uint8_t *packed, uint64_t first_base, const uint64_t *read_off,
                   uint64_t n_reads, const uint64_t *exc_start, const uint64_t *exc_end, uint64_t n_exc, uint32_t min_count, hga_kmer_counts_t *out,
                   hga_kmer_spectrum_t *spec, uint32_t n_bins, uint64_t *hist);
+int hga_sdk_run(const char *who, int device, int k, const uint8_t *packed, uint64_t first_base, const uint64_t *read_off, uint64_t n_reads,
+                const uint64_t *exc_start, const uint64_t *exc_end, uint64_t n_exc, int n_files, const uint64_t *file_first, uint32_t min_count, hga_sdk **out);
 int hga_index_run(hga_handle *h);
 int hga_build_lists(hga_handle *h, const uint32_t *d_keys, const uint64_t *d_row_off, uint64_t n_rows, uint64_t E, uint32_t n_keys);
 int hga_pairs_run(hga_handle *h, uint32_t min_score, const uint32_t *pivots, uint64_t n_pivots);

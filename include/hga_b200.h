@@ -20,6 +20,7 @@
  *   hga_count_kmers / hga_host_sdk_* <- jellyfish + JellyfishOccurrenceReader (the --kmers file)          occurrences/ (all files), jellyfish_occurrences.cpp
  *   hga_count_kmers_packed     the same count from case-folded 2-bit packed bases (hga_host_pack_bases_folded packs on the host)
  *   hga_count_spectrum[_packed]  the k-mer spectrum of that count (distinct k-mers per count) without materialising the k-mers
+ *   hga_sdk_*            the per-file counts merged on the GPU, with the specificity table and the count-range export of hga_host_sdk_*
  *   hga_enrich_full      <- the same plus the tail / spectral block in between (second merge_components)     :764-794
  *
  * Conventions
@@ -312,6 +313,34 @@ int hga_host_sdk_specificity(uint64_t n, const uint32_t *total, const uint32_t *
                              uint32_t *out_occurrences, uint64_t *out_unique, uint64_t capacity, uint64_t *out_n);
 int hga_host_sdk_select(uint64_t n, const uint32_t *total, const uint32_t *files, uint32_t lower, uint32_t upper, double percent, uint64_t seed,
                         uint8_t *out_selected, uint64_t *out_n_selected, uint64_t *out_n_discriminative);
+/* hga_sdk_*: the merge, the specificity table and the count-range export on the GPU; the merged table stays in HBM, so host memory
+ *   does not grow with the number of distinct k-mers (only hga_sdk_range's result does).
+ *   hga_sdk_count_packed: file f = reads [file_first_read[f], file_first_read[f + 1]) of the read set of hga_count_kmers_packed
+ *     (same packing, read-set and run rules). Every file is counted with min_count (the filter applies per file, before the merge)
+ *     and the files are merged: the handle holds what hga_host_sdk_merge returns on the per-file hga_count_kmers_packed lists.
+ *     file_first_read: n_files + 1 entries, [0] == 0, non-decreasing, [n_files] == n_reads (a file without reads is allowed).
+ *     A per-file count above 2^32 - 1 fails with HGA_E_OVERFLOW and hga_count_kmers_packed's message; so does a total above
+ *     2^32 - 1. On failure *out is NULL and no device memory is held. The handle owns device memory on `device` until hga_sdk_free.
+ *   hga_sdk_size: the number of merged k-mers.
+ *   hga_sdk_specificity: the rows, row order, errors and capacity protocol of hga_host_sdk_specificity on the merged table.
+ *   hga_sdk_range: the merged entries with lower <= total <= upper, ascending (empty when lower > upper), in arrays malloc'ed by the
+ *     library (release with hga_free_sdk_range). hga_host_sdk_select on it, with the same lower, upper, percent and seed, selects the
+ *     same k-mers as on the whole merged table: it draws only for in-range k-mers. */
+typedef struct hga_sdk hga_sdk;
+typedef struct {
+    uint64_t n;
+    const uint64_t *kmer;
+    const uint32_t *total, *max, *files;
+} hga_sdk_range_t;
+int hga_sdk_count_packed(int device, int k, const uint8_t *packed, uint64_t first_base, const uint64_t *read_off, uint64_t n_reads,
+                         const uint64_t *exc_start, const uint64_t *exc_end, uint64_t n_exc, int n_files, const uint64_t *file_first_read,
+                         uint32_t min_count, hga_sdk **out);
+int hga_sdk_size(const hga_sdk *s, uint64_t *n_kmers);
+int hga_sdk_specificity(const hga_sdk *s, const double *thresholds, int n_thresholds, double *out_threshold, uint32_t *out_occurrences,
+                        uint64_t *out_unique, uint64_t capacity, uint64_t *out_n);
+int hga_sdk_range(const hga_sdk *s, uint32_t lower, uint32_t upper, hga_sdk_range_t *out);
+void hga_free_sdk_range(hga_sdk_range_t *r);
+void hga_sdk_free(hga_sdk *s);
 
 /* Per-stage device time (CUDA events on the handle's stream) and counters of the most recent run. */
 typedef struct {

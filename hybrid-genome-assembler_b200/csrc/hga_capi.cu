@@ -121,9 +121,6 @@ int hga_create(int device, int k, const uint64_t *kmers, uint64_t n_kmers, hga_h
     cudaDeviceProp prop;
     HGA_CUDA(cudaGetDeviceProperties(&prop, device));
     if (prop.major < 10) { hga_set_error("device %d is sm_%d%d; this library is built for sm_100a (B200) only", device, prop.major, prop.minor); return HGA_E_CUDA; }
-    if (const char *eg = getenv("HGA_L2_FETCH")) {       // experiment switch: DRAM fetch granularity of L2 misses (32 / 64 / 128 B), a device-wide limit
-        if (cudaDeviceSetLimit(cudaLimitMaxL2FetchGranularity, (size_t) atoi(eg)) != cudaSuccess) cudaGetLastError();
-    }
     hga_handle *h = new hga_handle();
     memset(&h->metrics, 0, sizeof(h->metrics));
     h->device = device; h->k = k; h->n_kmers = n_kmers; h->sm_count = prop.multiProcessorCount;

@@ -466,7 +466,6 @@ int hga_comm_reduce_partials_packed(hga_handle *h, uint64_t n, uint64_t *out_n, 
     const int G = h->comm->size, me = h->comm->rank;
     *reduced = false;
     const int rb = (int) std::max<uint32_t>(hga_ceil_log2(h->inc_rows + 1), 1), sb = 64 - 2 * rb;
-    if (getenv("HGA_PARTIALS_UNPACKED")) return HGA_OK;
     if (sb < 12) return HGA_OK;                         // (the same on every rank: inc_rows is global)
     const int owner_bits = (int) std::max<uint32_t>(hga_ceil_log2((uint64_t) G), 1);
     double part_ms = 0;

@@ -171,7 +171,6 @@ int hga_build_lists(hga_handle *h, const uint32_t *d_keys, const uint64_t *d_row
     // sort runs over the GROUP bits only and index_local_sort_kernel finishes the order inside the groups.
     int L = 0;
     if (end_bit > 8 && (end_bit - 1) % 8 < 5 && n_keys % 32 == 0) L = 5;
-    if (const char *e = getenv("HGA_INDEX_LOCAL")) { if (atoi(e) == 0) L = 0; }
     uint32_t *d_sorted_rows = h->d_inv_row.as<uint32_t>();
     if (L) { HGA_TRY(h->d_index_tmp.ensure((E + 1) * 4)); d_sorted_rows = h->d_index_tmp.as<uint32_t>(); }
     HGA_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, d_keys, h->d_sort_a.as<uint32_t>(), d_rows, d_sorted_rows, E, L, end_bit, h->stream));

@@ -91,7 +91,7 @@ struct PinBuf {
 // (4^m / 2 >= 3 n: unrelated loci must not share a minimizer VALUE) with W <= HGA_MIN_W; when k leaves no room for that
 // (k < HGA_MIN_K_FOR_MIN, or k - 16 + 1 > HGA_MIN_W) a mix of hb takes Mc's place (no locality, still correct).
 //
-//   filter    : blocked Bloom filter over the canonical keys; block = 32 B (8 words) selected by Mc, word + 2 bits inside the
+//   filter    : blocked Bloom filter over the canonical keys; block = 32 B (8 words) selected by Mc, word + 3 bits inside the
 //               block selected by hb. Sized to stay L2 resident: measured on B200 (profiles/r2c), a filter of <= 48 MB is served
 //               from L2 while 10 Gbases stream through, 64 MB is not (26.9 -> 37.6 -> 59.2 ms at 48 / 64 / 96 MB).
 //   key table : canonical keys, u64, buckets of 32 (256 B) selected by Mc. Inside the bucket a key starts at the 32 B SECTOR
@@ -128,8 +128,6 @@ struct KmerTable {
     uint32_t n_blocks = 0;
     uint32_t n_slots = 0;           // n_main + n_over
     uint32_t slot_bits = 0;         // ceil(log2(n_slots))
-    int sector_by_min = 0;          // hga_start_sector
-    int filter_k = 3;               // bits a key sets in its filter word (3: 9.1 % of the windows of config 4 pass the 48 MB filter, 2: 10.0 %)
     KmerGeom geom;
 };
 
@@ -190,24 +188,22 @@ __host__ __device__ __forceinline__ uint32_t hga_bits_hash(uint64_t x, const Kme
     return hga_strand_hash((uint32_t) (x >> 32), (uint32_t) x, g) + hga_strand_hash((uint32_t) (r >> 32), (uint32_t) r, g);
 }
 __host__ __device__ __forceinline__ uint32_t hga_bits_word(uint32_t h) { return h >> 29; }
-// the bit positions inside the filter word (two, or three with filter_k = 3) come from the HIGH half of hb * C2: its low bits are well
-// mixed, so a wrapping shift takes a bit position straight from the register (no mask is ever built by the scan)
+// the three bit positions a key sets inside its filter word (3 bits: 9.1 % of the windows of config 4 pass the 48 MB filter, 2 bits: 10.0 %)
+// come from the HIGH half of hb * C2: its low bits are well mixed, so a wrapping shift takes a bit position straight from the register (no
+// mask is ever built by the scan)
 __host__ __device__ __forceinline__ uint32_t hga_bits_pos(uint32_t hb) { return hga_scale(hb, HGA_C2); }
-__host__ __device__ __forceinline__ uint32_t hga_bits_mask(uint32_t hb, int filter_k) {
+__host__ __device__ __forceinline__ uint32_t hga_bits_mask(uint32_t hb) {
     const uint32_t v = hga_bits_pos(hb);
-    return (1u << (v & 31)) | (1u << ((v >> 5) & 31)) | (1u << ((filter_k == 3 ? v >> 10 : v) & 31));
+    return (1u << (v & 31)) | (1u << ((v >> 5) & 31)) | (1u << ((v >> 10) & 31));
 }
 #ifdef __CUDACC__
-__device__ __forceinline__ bool hga_bits_test(uint32_t word, uint32_t hb, int filter_k) {
+__device__ __forceinline__ bool hga_bits_test(uint32_t word, uint32_t hb) {
     const uint32_t v = hga_bits_pos(hb);
-    return (__funnelshift_r(word, 0u, v) & __funnelshift_r(word, 0u, v >> 5) & __funnelshift_r(word, 0u, filter_k == 3 ? v >> 10 : v) & 1u) != 0;
+    return (__funnelshift_r(word, 0u, v) & __funnelshift_r(word, 0u, v >> 5) & __funnelshift_r(word, 0u, v >> 10) & 1u) != 0;
 }
 #endif
-// start sector of a key inside its bucket: from the bit hash (keys spread evenly: 95 % of the lookups end in their first sector), or -
-// sector_by_min - from the minimizer (the keys of a run share a sector: fewer DRAM bursts per run of hits, more second steps)
-__host__ __device__ __forceinline__ uint32_t hga_start_sector(uint32_t B, uint32_t hb, int sector_by_min) {
-    return ((sector_by_min ? B >> 7 : hb >> 16)) & (HGA_BUCKET_SLOTS / HGA_SECTOR_SLOTS - 1);
-}
+// start sector of a key inside its bucket, from the bit hash: keys spread evenly, 95 % of the lookups end in their first sector
+__host__ __device__ __forceinline__ uint32_t hga_start_sector(uint32_t hb) { return (hb >> 16) & (HGA_BUCKET_SLOTS / HGA_SECTOR_SLOTS - 1); }
 // when there is no minimizer: the locality value is a mix of the bit hash
 __host__ __device__ __forceinline__ uint32_t hga_mix_bits(uint32_t hb) { return (hb ^ (hb >> 15)) * HGA_C3; }
 

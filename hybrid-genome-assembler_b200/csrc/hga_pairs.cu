@@ -73,7 +73,6 @@ struct PairParams {
     const uint8_t *pivot_flag;      // SUBSET mode only
     uint64_t n_pivots;
     int mode;
-    int single_pass;                // tier 1 runs once with the 1024-entry accumulator (multi-GPU)
     uint32_t min_score;
     uint64_t *out_key;
     uint32_t *out_score;
@@ -314,27 +313,29 @@ __device__ __forceinline__ void flush_table(WarpAcc<CMAX> &A, const PairParams &
     }
 }
 
-// CMAX / REDO: the kernel is latency bound and its time is inversely proportional to the number of resident warps (r3s: 1 / 2 / 3 /
-// 4 / 6 CTAs per SM -> 359 / 186 / 130 / 102 / 75 ms), and the accumulator is what limits them. The first pass therefore runs with
-// a 512-entry accumulator (17 KB per CTA: 11 CTAs = 44 warps per SM); the rows whose partner set does not fit it are listed and
-// redone by a second pass with 1024 entries (6 CTAs per SM), and only what overflows that goes on to tier 2.
-template<int CMAX, bool REDO, int MINB = 1, int EPS = 4, bool TAILONLY = false, bool CHECK = false>
-__global__ void __launch_bounds__(PW_THREADS, MINB) pair_count_warp_kernel(const __grid_constant__ PairParams p) {
+// The kernel is latency bound and its time is inversely proportional to the number of resident warps (r3s: 1 / 2 / 3 / 4 / 6 CTAs
+// per SM -> 359 / 186 / 130 / 102 / 75 ms), and the accumulator is what limits them. The first pass therefore runs with a 512-entry
+// accumulator (17 KB per CTA), registers limited for 9 CTAs per SM, and eight list entries (one 32 B sector) per step; the rows whose
+// partner set does not fit are listed and redone by pair_count_redo_kernel with 1024 entries, and only what overflows that goes on to
+// tier 2. (r3p / r3q, config 4, (CTAs per SM the registers are limited for, entries per step): (1, 4) 56 registers 55.5 ms, (1, 8) 75
+// registers 53.7, (8, 8) 59 registers 49.8, (9, 8) 48.7, (10, 8) 47 registers 48.7, (8, 16) 60.3, (6, 16) 65.0.)
+template<bool TAILONLY, bool CHECK>
+__global__ void __launch_bounds__(PW_THREADS, 9) pair_count_warp_kernel(const __grid_constant__ PairParams p) {
+    constexpr int CMAX = PW_CMAX_FIRST;
     __shared__ WarpAcc<CMAX> s_acc[PW_WARPS];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     WarpAcc<CMAX> &A = s_acc[warp];
     const bool tail = p.mode == PAIR_MODE_TAIL;
-    const unsigned long long n_items = REDO ? p.sc->redo_count : p.n_pivots;
+    const unsigned long long n_items = p.n_pivots;
 
     for (;;) {
         unsigned long long t = 0;
-        if (lane == 0) t = atomicAdd(REDO ? &p.sc->redo_ticket : &p.sc->ticket, 1ull);
+        if (lane == 0) t = atomicAdd(&p.sc->ticket, 1ull);
         t = __shfl_sync(0xFFFFFFFFu, t, 0);
         if (t >= n_items) break;
         // x: global row (what the inverted lists hold); xl: row of the by-read incidence on this GPU
-        uint32_t x, xl;
-        if (REDO) { xl = p.redo_list[t]; x = p.pivot_rows ? xl : xl * p.pivot_mul + p.pivot_add; }
-        else { x = p.pivot_rows ? p.pivot_rows[t] : (uint32_t) t * p.pivot_mul + p.pivot_add; xl = p.pivot_rows ? x : (uint32_t) t; }
+        const uint32_t x = p.pivot_rows ? p.pivot_rows[t] : (uint32_t) t * p.pivot_mul + p.pivot_add;
+        const uint32_t xl = p.pivot_rows ? x : (uint32_t) t;
         const uint64_t a = p.row_off[xl], b = p.row_off[xl + 1];
         if (a == b) continue;
 
@@ -348,16 +349,13 @@ __global__ void __launch_bounds__(PW_THREADS, MINB) pair_count_warp_kernel(const
             if (lane == 0) { A.distinct = 0; A.overflow = 0; A.n_defer = 0; }
             __syncwarp();
 
-            walk_row<CMAX, EPS, TAILONLY, CHECK>(A, p, x, a, b, tail, cmask, cshift, limit, lane);
+            walk_row<CMAX, 8, TAILONLY, CHECK>(A, p, x, a, b, tail, cmask, cshift, limit, lane);
             if (!*reinterpret_cast<volatile uint32_t *>(&A.overflow)) {
                 flush_table<CMAX>(A, p, x, C, lane);
                 break;
             }
             if (C == CMAX) {         // more partners than this accumulator holds: second pass, then tier 2
-                if (lane == 0) {
-                    if (REDO || p.single_pass) p.mid_list[atomicAdd(&p.sc->mid_count, 1ull)] = xl;
-                    else p.redo_list[atomicAdd(&p.sc->redo_count, 1ull)] = xl;
-                }
+                if (lane == 0) p.redo_list[atomicAdd(&p.sc->redo_count, 1ull)] = xl;
                 break;
             }
         }
@@ -606,29 +604,6 @@ __global__ void row_minhash_kernel(const uint64_t *__restrict__ row_off, const u
     }
 }
 
-// Pivot order, second form: label(r) = smallest row that shares a (sampled) k-mer with r. Inverted lists are ascending, so the label
-// every list hands to its rows is its first entry; one atomicMin per list entry. All reads overlapping a read m whose id is the
-// smallest in its neighbourhood get the label m: groups of ~coverage reads around one locus, whatever the error rate (the min-hash
-// order needs ONE particular k-mer to survive in both reads). Sorting the pivots by label makes the rows in flight share their
-// lists (and the inv_off sectors of those lists) in L2.
-__global__ void row_label_init_kernel(uint32_t *__restrict__ label, uint32_t *__restrict__ row, uint64_t n_rows) {
-    for (uint64_t i = blockIdx.x * (uint64_t) blockDim.x + threadIdx.x; i < n_rows; i += (uint64_t) gridDim.x * blockDim.x) { label[i] = (uint32_t) i; row[i] = (uint32_t) i; }
-}
-__global__ void row_neighbor_min_kernel(const uint32_t *__restrict__ inv_off, const uint32_t *__restrict__ inv_row, uint32_t n_keys, uint32_t stride,
-                                        uint32_t *__restrict__ label) {
-    const uint64_t n_samples = ((uint64_t) n_keys + stride - 1) / stride;
-    for (uint64_t t = blockIdx.x * (uint64_t) blockDim.x + threadIdx.x; t < n_samples; t += (uint64_t) gridDim.x * blockDim.x) {
-        const uint32_t s = (uint32_t) (t * stride);
-        const uint32_t lo = __ldg(&inv_off[s]), hi = __ldg(&inv_off[s + 1]);
-        if (hi - lo < 2) continue;
-        const uint32_t m = __ldg(&inv_row[lo]);
-        for (uint32_t i = lo + 1; i < hi; i++) {
-            const uint32_t y = __ldg(&inv_row[i]);
-            if (y != m) atomicMin(&label[y], m);
-        }
-    }
-}
-
 // largest hit count of a row: bounds every score by its square
 __global__ void max_row_hits_kernel(const uint64_t *__restrict__ row_off, uint64_t n_rows, unsigned long long *out) {
     unsigned long long m = 0;
@@ -734,11 +709,14 @@ int hga_pairs_run(hga_handle *h, uint32_t min_score, const uint32_t *pivots, uin
         p.mode = PAIR_MODE_SUBSET;
     }
 
-    // experiment hook: a pivot order read from a file (HGA_PAIR_ORDER=3 + HGA_PAIR_ORDER_FILE = u32 rows), loaded before the stage timer
+    // pivot order (a performance hint only: the pairs are sorted into canonical order afterwards): the min-hash of the row's k-mers when every
+    // row is a pivot, or - HGA_PAIR_ORDER=3 + HGA_PAIR_ORDER_FILE = u32 rows - an order read from a file, loaded before the stage timer
+    // (bench.py: the true genome order of its synthetic input, the upper bound of what an order can buy)
+    const bool ordered = !pivots && n_rows > 4096;
     const uint32_t *file_order = nullptr;
     if (const char *e = getenv("HGA_PAIR_ORDER")) {
         const char *order_file = getenv("HGA_PAIR_ORDER_FILE");
-        if (atoi(e) == 3 && order_file && !pivots && n_rows > 4096) {
+        if (atoi(e) == 3 && order_file && ordered) {
             std::vector<uint32_t> ord(n_rows);
             FILE *f = fopen(order_file, "rb");
             if (!f || fread(ord.data(), 4, n_rows, f) != n_rows) { if (f) fclose(f); hga_set_error("HGA_PAIR_ORDER_FILE: cannot read %llu rows", (unsigned long long) n_rows); return HGA_E_ARG; }
@@ -752,78 +730,36 @@ int hga_pairs_run(hga_handle *h, uint32_t min_score, const uint32_t *pivots, uin
 
     StageTimer timer(h, &h->metrics.pair_ms);
     Trace tr(h);
-    // pivot order (a performance hint only: the pairs are sorted into canonical order afterwards). 0: row order, 1: min-hash of the
-    // row's k-mers, 2: smallest neighbouring row (row_neighbor_min_kernel), 3: read from HGA_PAIR_ORDER_FILE (experiments: the true
-    // genome order of a synthetic input as the upper bound of what an order can buy)
-    int order_mode = (!pivots && n_rows > 4096) ? 1 : 0;
-    if (const char *e = getenv("HGA_PAIR_ORDER")) { if (!pivots && n_rows > 4096) order_mode = atoi(e); }
-    if (order_mode == 3) { order_mode = 0; if (file_order) p.pivot_rows = file_order; }
-    if (order_mode == 1 || order_mode == 2) {
+    if (file_order) {
+        p.pivot_rows = file_order;
+    } else if (ordered) {
         HGA_TRY(h->d_pivot_order.ensure((n_rows + 1) * 4 * 4));
         uint32_t *k_in = h->d_pivot_order.as<uint32_t>(), *r_in = k_in + (n_rows + 1), *k_out = r_in + (n_rows + 1), *r_out = k_out + (n_rows + 1);
-        if (order_mode == 1) {
-            row_minhash_kernel<<<(int) std::min<uint64_t>((n_rows * 32 + 255) / 256, (uint64_t) h->sm_count * 32), 256, 0, h->stream>>>(p.row_off, p.row_slot, n_rows, k_in, r_in);
-        } else {
-            // ~48 sampled lists per row on average
-            uint64_t stride = h->inc_entries / (48 * std::max<uint64_t>(n_rows, 1));
-            if (const char *e = getenv("HGA_PAIR_ORDER_STRIDE")) stride = (uint64_t) atoi(e);
-            stride = std::min<uint64_t>(std::max<uint64_t>(stride, 1), 256);
-            const uint64_t n_samples = ((uint64_t) h->index_keys + stride - 1) / stride;
-            row_label_init_kernel<<<(int) std::min<uint64_t>((n_rows + 255) / 256, (uint64_t) h->sm_count * 16), 256, 0, h->stream>>>(k_in, r_in, n_rows);
-            row_neighbor_min_kernel<<<(int) std::max<uint64_t>(1, std::min<uint64_t>((n_samples + 255) / 256, (uint64_t) h->sm_count * 32)), 256, 0, h->stream>>>(
-                p.inv_off, p.inv_row, h->index_keys, (uint32_t) stride, k_in);
-            h->metrics.kernel_launches++;
-        }
-        const int label_bits = order_mode == 1 ? 32 : (int) std::max<uint32_t>(hga_ceil_log2(n_rows + 1), 1);
+        row_minhash_kernel<<<(int) std::min<uint64_t>((n_rows * 32 + 255) / 256, (uint64_t) h->sm_count * 32), 256, 0, h->stream>>>(p.row_off, p.row_slot, n_rows, k_in, r_in);
         size_t tmp_bytes = 0;
-        HGA_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, k_in, k_out, r_in, r_out, n_rows, 0, label_bits, h->stream));
+        HGA_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, k_in, k_out, r_in, r_out, n_rows, 0, 32, h->stream));
         HGA_TRY(h->d_sort_tmp.ensure(tmp_bytes + 16));
-        HGA_CUDA(cub::DeviceRadixSort::SortPairs(h->d_sort_tmp.p, tmp_bytes, k_in, k_out, r_in, r_out, n_rows, 0, label_bits, h->stream));
+        HGA_CUDA(cub::DeviceRadixSort::SortPairs(h->d_sort_tmp.p, tmp_bytes, k_in, k_out, r_in, r_out, n_rows, 0, 32, h->stream));
         h->metrics.kernel_launches += 6;
         HGA_CUDA(cudaGetLastError());
         p.pivot_rows = r_out;        // all rows, TAIL mode, in that order
     }
     uint64_t capacity = std::max<uint64_t>(h->pair_capacity, std::max<uint64_t>(64 * n_rows, 1ull << 20));
-    int occ_w = 0, occ_c = 0;
-    int occ_r = 0;
-    int pair_occ = 0;                        // experiment switch, see first_pass below
-    if (const char *e = getenv("HGA_PAIR_OCC")) pair_occ = atoi(e);
-    if (const char *e = getenv("HGA_PAIR_CARVEOUT"))   // experiment switch: shared-memory carve-out of the first pass in percent (the rest of the 228 KB is L1)
-        HGA_CUDA(cudaFuncSetAttribute(pair_count_warp_kernel<PW_CMAX_FIRST, false, 9, 8, true>, cudaFuncAttributePreferredSharedMemoryCarveout, atoi(e)));
-    size_t pad_smem = 0;                     // experiment switch: cap the first pass at HGA_PAIR_CTAS CTAs per SM with unused dynamic shared memory
-    if (const char *e = getenv("HGA_PAIR_CTAS")) {
-        const int want = std::max(1, atoi(e));
-        const size_t per = (size_t) (227 * 1024) / want;
-        const size_t stat = sizeof(WarpAcc<PW_CMAX_FIRST>) * PW_WARPS + 1024;
-        if (per > stat) pad_smem = std::min<size_t>(per - stat, (size_t) 200 * 1024);
-        HGA_CUDA(cudaFuncSetAttribute(pair_count_warp_kernel<PW_CMAX_FIRST, false, 9, 8, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) pad_smem));
-    }
-    // first-pass kernel: (CTAs per SM the registers are limited for, list entries per step). Default (9, 8): 55 registers, eight entries = one 32 B sector per
-    // step. r3p / r3q, config 4: (1, 4) 56 registers 55.5 ms, (1, 8) 75 registers 53.7, (8, 8) 59 registers 49.8, (9, 8) 48.7, (10, 8) 47 registers 48.7,
-    // (8, 16) 60.3, (6, 16) 65.0. HGA_PAIR_OCC=4 selects the four-entry kernel for A/B runs.
+    int occ_w = 0, occ_c = 0, occ_r = 0;
     typedef void (*pair_kernel_t)(const PairParams);
-    pair_kernel_t first_pass = pair_count_warp_kernel<PW_CMAX_FIRST, false, 9, 8, true>;
-    if (p.mode != PAIR_MODE_TAIL) first_pass = pair_count_warp_kernel<PW_CMAX_FIRST, false, 9, 8, false>;
-    if (pair_occ == 4) first_pass = pair_count_warp_kernel<PW_CMAX_FIRST, false, 1, 4>;
-    if (pair_occ == 98) first_pass = pair_count_warp_kernel<PW_CMAX_FIRST, false, 9, 8, false>;
-    pair_kernel_t single_pass_kernel = pair_count_warp_kernel<PW_CMAX, false>;
+    pair_kernel_t first_pass = p.mode == PAIR_MODE_TAIL ? pair_count_warp_kernel<true, false> : pair_count_warp_kernel<false, false>;
     pair_kernel_t redo_kernel = pair_count_redo_kernel<false>, mid_kernel = pair_count_kernel<false>, heavy_kernel = pair_count_heavy_kernel<false>;
     if (check_scores) {
-        first_pass = p.mode == PAIR_MODE_TAIL ? pair_count_warp_kernel<PW_CMAX_FIRST, false, 9, 8, true, true> : pair_count_warp_kernel<PW_CMAX_FIRST, false, 9, 8, false, true>;
-        single_pass_kernel = pair_count_warp_kernel<PW_CMAX, false, 1, 4, false, true>;
+        first_pass = p.mode == PAIR_MODE_TAIL ? pair_count_warp_kernel<true, true> : pair_count_warp_kernel<false, true>;
         redo_kernel = pair_count_redo_kernel<true>; mid_kernel = pair_count_kernel<true>; heavy_kernel = pair_count_heavy_kernel<true>;
-        pad_smem = 0;
     }
-    HGA_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_w, first_pass, PW_THREADS, pad_smem));
+    HGA_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_w, first_pass, PW_THREADS, 0));
     HGA_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_r, redo_kernel, PW_THREADS, 0));
     if (occ_r < 1) occ_r = 1;
     HGA_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_c, mid_kernel, PC_THREADS, 0));
     if (occ_w < 1) occ_w = 1;
     if (occ_c < 1) occ_c = 1;
     const int grid_w = (int) std::max<uint64_t>(1, std::min<uint64_t>((uint64_t) h->sm_count * occ_w, (p.n_pivots + PW_WARPS - 1) / PW_WARPS));
-    p.single_pass = 0;
-    if (const char *e = getenv("HGA_PAIR_SINGLE_PASS")) p.single_pass = atoi(e) != 0;
-    const int grid_s = (int) std::max<uint64_t>(1, std::min<uint64_t>((uint64_t) h->sm_count * occ_r, (p.n_pivots + PW_WARPS - 1) / PW_WARPS));
     PairScalars sc;
     h->metrics.pair_retries = 0;
     for (int attempt = 0;; attempt++) {
@@ -832,10 +768,7 @@ int hga_pairs_run(hga_handle *h, uint32_t min_score, const uint32_t *pivots, uin
         p.out_key = h->d_pair_key.as<uint64_t>(); p.out_score = h->d_pair_score.as<uint32_t>(); p.capacity = capacity;
         HGA_CUDA(cudaMemsetAsync(d_sc, 0, sizeof(PairScalars), h->stream));
         if (p.n_pivots) {
-            // multi-GPU: the index is keyed by kmer_id there, neighbouring hits of a read do not have neighbouring lists, and the
-            // extra warps of the 512-entry pass only add random DRAM traffic (r3z, 2 GPUs: 50.6 ms against 45.2 ms single pass)
-            if (p.single_pass) single_pass_kernel<<<grid_s, PW_THREADS, 0, h->stream>>>(p);
-            else first_pass<<<grid_w, PW_THREADS, pad_smem, h->stream>>>(p);
+            first_pass<<<grid_w, PW_THREADS, 0, h->stream>>>(p);
             h->metrics.kernel_launches++;
             HGA_CUDA(cudaGetLastError());
         }

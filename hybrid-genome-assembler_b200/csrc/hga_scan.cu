@@ -10,8 +10,7 @@
 //     them into one word of forward codes (first base most significant) and one word of complement codes (first base least
 //     significant). Bytes outside {A,C,G,T} get code 0 in BOTH streams - the reference's rule (KmerIterator.cpp:56,62:
 //     unordered_map::operator[] default-inserts 0 in both tables) - and a bit in an exception bitmap (validity = one PRMT lookup
-//     of the expected byte per 4 bases); the two previous lanes' words come over with four shuffles. (The same 512 bytes as a
-//     1-D bulk copy into a double buffer, cp.async.bulk + mbarrier: template variant TMA, HGA_SCAN_TMA=1, measured slower.)
+//     of the expected byte per 4 bases); the two previous lanes' words come over with four shuffles.
 //   * phase B, lane-sequential: a lane owns SCAN_LANE (16) CONSECUTIVE window ends. With its 48 bases in registers every piece
 //     is a funnel shift with a compile-time register index: the forward and reverse strand's last 16 bases and the 16 before,
 //     the two hashed m-mers (one IMAD each: the multiplier shifts out everything above the m-mer), the sliding minimum over the
@@ -75,9 +74,7 @@ struct ScanParams {
     uint64_t tile_stride;             // > 0: sampling mode (count only, tile = tile_begin + ticket * stride)
     uint32_t chunk;                   // hit-buffer entries a warp reserves per atomic
     unsigned long long *warp_chunks;  // chunked launches: every warp's open chunk [pos, end) survives from one launch to the next (nullptr: one launch)
-    int diag;                         // HGA_SCAN_DIAG experiment: 1 = no key probes (results are WRONG), 2 = metrics.n_candidates counts sector probes
-    // packed input (hga_scan_packed*; appended so that the parameter offsets of the ASCII kernels stay as they were). frame is then 4 B aligned
-    // and lead counts bases (0..15)
+    // packed input (hga_scan_packed*): frame is then 4 B aligned and lead counts bases (0..15)
     const uint64_t *exc_start, *exc_end;  // exception runs, half-open stream positions, sorted and disjoint
     uint64_t n_exc;
     const unsigned long long *exc_dir;    // per tile: the first run that touches its staged span, ~0 = none (nullptr: no runs, never read)
@@ -213,7 +210,7 @@ __device__ __forceinline__ bool probe_sector(const uint64_t *keys, uint32_t base
     return slot != SCAN_NONE || a == HGA_EMPTY_KEY || b == HGA_EMPTY_KEY || d == HGA_EMPTY_KEY || e == HGA_EMPTY_KEY;
 }
 
-struct QueueState { uint32_t head, tail, st_count, probes; };     // warp uniform (probes: per lane, HGA_SCAN_DIAG=2 only)
+struct QueueState { uint32_t head, tail, st_count; };     // warp uniform
 
 // n (<= 32) queued candidates starting at ring position head: check the window against the read boundaries, rebuild the canonical
 // k-mer, probe the key table; hits are appended to the staging area in position order
@@ -231,7 +228,7 @@ __device__ __forceinline__ void drain_queue(QueueState &qs, uint32_t n, int lane
         const int i = (int) widx;
         uint2 en = T.tr[tr_index(i)];     // x = locality hash, y = bit hash (still there: hits are staged below index i - 32)
         const int start = read_start_of(c, i);
-        if (i < c.i_end && i - start + 1 >= k && !(p.diag & 1)) {
+        if (i < c.i_end && i - start + 1 >= k) {
             uint32_t lo, hi;
             extract_window(T.pk, i, lo, hi);
             const unsigned long long kmask = k == 32 ? ~0ull : ((1ull << (2 * k)) - 1);
@@ -245,7 +242,7 @@ __device__ __forceinline__ void drain_queue(QueueState &qs, uint32_t n, int lane
                 en.x = hga_locality_from_min(hga_minimizer(key, en.y, t.geom));
             }
             base_slot = hga_scale(en.x, t.n_buckets) * HGA_BUCKET_SLOTS;
-            sec = hga_start_sector(en.x, en.y, t.sector_by_min);
+            sec = hga_start_sector(en.y);
             open = true;
         }
     }
@@ -254,7 +251,6 @@ __device__ __forceinline__ void drain_queue(QueueState &qs, uint32_t n, int lane
     const uint64_t pol_first = l2_policy_evict_first();
     for (int step = 0; __any_sync(0xFFFFFFFFu, open); step++) {
         if (open) {
-            if (p.diag & 2) qs.probes++;
             if (probe_sector(t.keys, base_slot, sec + step, key, pol_first, slot)) open = false;
             else if (step == HGA_BUCKET_SLOTS / HGA_SECTOR_SLOTS - 1) {
                 open = false;
@@ -344,8 +340,7 @@ __device__ __forceinline__ uint32_t phase_c(const TileCtx &c, int lane, uint32_t
     const uint64_t pol_last = l2_policy_evict_last();
     const uint32_t n_blocks = p.t.n_blocks, lane_lt = (1u << lane) - 1;
     const uint32_t *filter = p.t.filter;
-    const int filter_k = p.t.filter_k;
-    QueueState qs = {0, 0, 0, 0};
+    QueueState qs = {0, 0, 0};
     #pragma unroll 1
     for (int s0 = 0; s0 <= SCAN_SPAN / 32; s0 += SCAN_UNROLL) {
         const bool last = s0 >= SCAN_SPAN / 32;                     // one more round that only empties the queue
@@ -361,7 +356,7 @@ __device__ __forceinline__ uint32_t phase_c(const TileCtx &c, int lane, uint32_t
             for (int u = 0; u < SCAN_UNROLL; u++) {
                 if (u == 0 && s0 == 0) continue;                    // the halo's windows belong to the previous tile
                 const int i = 32 * (s0 + u) + lane;
-                bool pass = hga_bits_test(fw[u], en[u].y, filter_k);
+                bool pass = hga_bits_test(fw[u], en[u].y);
                 bool exc = false;
                 if (EXC) { exc = window_exc(T.exc, i, p.t.geom.k) != 0; pass |= exc; }
                 const uint32_t bal = __ballot_sync(0xFFFFFFFFu, pass);
@@ -378,21 +373,16 @@ __device__ __forceinline__ uint32_t phase_c(const TileCtx &c, int lane, uint32_t
             __syncwarp();
         }
     }
-    n_cand += (p.diag & 2) ? __reduce_add_sync(0xFFFFFFFFu, qs.probes) : qs.tail;     // HGA_SCAN_DIAG=2: sector probes instead of candidates
+    n_cand += qs.tail;
     return qs.st_count;
 }
 
-// 32 independent warps per SM (4 CTAs of 8; 5.2 KB of shared memory per warp). The parameters are __grid_constant__ and every helper
-// is inlined so that nothing lives in local memory.
-// MINB = resident CTAs per SM the register allocation aims at (4: 64 registers = 32 warps, 5: 48 registers = 40 warps, 3: 80
-// registers = 24 warps; experiment switch HGA_SCAN_OCC)
-// TMA (experiment, HGA_SCAN_TMA=1): the tile's 512 bytes arrive by a 1-D bulk copy (cp.async.bulk, evict-first in L2) into a per-warp double buffer and
-// complete on an mbarrier; the copy of the NEXT tile is in flight while the current one is processed, so phase A never waits for HBM.
-#define SCAN_STAGE_BYTES (2 * SCAN_SPAN + 16)    // two tile buffers + two mbarriers per warp
+// 32 independent warps per SM (4 CTAs of 8 at 64 registers; 5.2 KB of shared memory per warp). The parameters are __grid_constant__ and
+// every helper is inlined so that nothing lives in local memory.
 // PACKED: the bases arrive 2-bit packed (4 per byte, first base most significant): a lane loads one 4-byte word = its 16 bases, the
 // exception runs of the tile come from the run directory. Phases B and C, the drain and the hit staging are the same code.
-template<int MINB, bool TMA, bool PACKED = false>
-__global__ void __launch_bounds__(SCAN_THREADS, MINB) scan_probe_kernel(const __grid_constant__ ScanParams p) {
+template<bool PACKED>
+__global__ void __launch_bounds__(SCAN_THREADS, 4) scan_probe_kernel(const __grid_constant__ ScanParams p) {
     extern __shared__ __align__(16) unsigned char s_raw[];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     WarpTile &T = reinterpret_cast<WarpTile *>(s_raw)[warp];
@@ -426,54 +416,12 @@ __global__ void __launch_bounds__(SCAN_THREADS, MINB) scan_probe_kernel(const __
         T.tk[0] = t + 1;
         return t;
     };
-    // TMA path: stage buffers and mbarriers of this warp, and the bulk copy of one tile into a buffer (lane 0)
-    unsigned char *stage = s_raw + SCAN_WARPS * sizeof(WarpTile) + (size_t) warp * SCAN_STAGE_BYTES;
-    const uint32_t stage_sa = (uint32_t) __cvta_generic_to_shared(stage), mbar_sa = stage_sa + 2 * SCAN_SPAN;
-    const int64_t u_end_all = (int64_t) p.lead + (int64_t) p.n_bases;
-    auto issue_tile = [&](unsigned long long t, int buf) {
-        const uint64_t tl = p.tile_begin + (p.tile_stride ? t * p.tile_stride : t);
-        const int64_t ub = (int64_t) (tl * SCAN_TILE) - 32;
-        const int64_t lo = max(ub, (int64_t) 0), hi = min(ub + SCAN_SPAN, (u_end_all + 15) & ~(int64_t) 15);
-        const uint32_t bytes = hi > lo ? (uint32_t) (hi - lo) : 0u;
-        const uint32_t mb = mbar_sa + 8 * buf;
-        if (bytes) {
-            asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" :: "r"(mb), "r"(bytes) : "memory");
-            asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1], %2, [%3], %4;"
-                         :: "r"(stage_sa + buf * SCAN_SPAN + (uint32_t) (lo - ub)), "l"(p.frame + lo), "r"(bytes), "r"(mb), "l"(pol_stream) : "memory");
-        } else {
-            asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" :: "r"(mb) : "memory");
-        }
-    };
     unsigned long long cur = 0;
-    uint32_t parity = 0;                                                // bit b: phase parity of buffer b's mbarrier
-    int buf = 0;
-    if (TMA) {
-        if (lane == 0) {
-            asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" :: "r"(mbar_sa));
-            asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" :: "r"(mbar_sa + 8));
-            asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-        }
-        __syncwarp();
-    }
-    if (lane == 0) {
-        cur = take_ticket();
-        if (TMA && cur < p.n_tiles) issue_tile(cur, 0);
-    }
+    if (lane == 0) cur = take_ticket();
     for (;;) {
         const unsigned long long ticket = __shfl_sync(0xFFFFFFFFu, cur, 0);
         if (ticket >= p.n_tiles) break;
-        const int my_buf = buf;
-        if (lane == 0) {
-            cur = take_ticket();                                        // the tile after this one: its bytes travel while this one is processed
-            if (TMA && cur < p.n_tiles) issue_tile(cur, buf ^ 1);
-        }
-        if (TMA) {
-            const uint32_t mb = mbar_sa + 8 * my_buf, ph = (parity >> my_buf) & 1u;
-            asm volatile("{\n.reg .pred p;\nSCAN_WAIT:\nmbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n@p bra SCAN_DONE;\nbra SCAN_WAIT;\nSCAN_DONE:\n}" :: "r"(mb), "r"(ph) : "memory");
-            parity ^= 1u << my_buf;
-            buf ^= 1;
-        }
-        {
+        if (lane == 0) cur = take_ticket();                            // the tile after this one
         const uint64_t tile = p.tile_begin + (p.tile_stride ? ticket * p.tile_stride : ticket);
         // frame coordinate u = stream position + lead; the tile's window ends are u in [480 tile, 480 tile + 480); staged index 0 is u = 480 tile - 32
         const int64_t ubase = (int64_t) (tile * SCAN_TILE) - 32;
@@ -513,13 +461,8 @@ __global__ void __launch_bounds__(SCAN_THREADS, MINB) scan_probe_kernel(const __
             const int64_t u = ubase + SCAN_LANE * lane;
             uint32_t v[4];
             if (u >= 0 && u < u_end) {
-                if (TMA) {
-                    const uint4 c = *reinterpret_cast<const uint4 *>(stage + my_buf * SCAN_SPAN + SCAN_LANE * lane);
-                    v[0] = c.x; v[1] = c.y; v[2] = c.z; v[3] = c.w;
-                } else {
-                    asm volatile("ld.global.L1::no_allocate.L2::cache_hint.v4.u32 {%0, %1, %2, %3}, [%4], %5;"
-                                 : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]) : "l"(p.frame + u), "l"(pol_stream));
-                }
+                asm volatile("ld.global.L1::no_allocate.L2::cache_hint.v4.u32 {%0, %1, %2, %3}, [%4], %5;"
+                             : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]) : "l"(p.frame + u), "l"(pol_stream));
             } else {
                 #pragma unroll
                 for (int i = 0; i < 4; i++) v[i] = 0x41414141u;                        // outside the stream: 'A' (never inside a valid window)
@@ -614,7 +557,6 @@ __global__ void __launch_bounds__(SCAN_THREADS, MINB) scan_probe_kernel(const __
             }
         }
         __syncwarp();
-      }
     }
     if (lane == 0 && p.warp_chunks) {
         const size_t warp_id = (size_t) blockIdx.x * SCAN_WARPS + warp;
@@ -709,17 +651,6 @@ __global__ void scan_fix_rows_kernel(const uint64_t *__restrict__ read_off, uint
     }
 }
 
-int scan_occ_variant() {
-    static int v = 0;
-    if (!v) { const char *e = getenv("HGA_SCAN_OCC"); v = e ? atoi(e) : 4; if (v != 3 && v != 5) v = 4; }
-    return v;
-}
-bool scan_tma_variant() {
-    static int v = -1;
-    if (v < 0) { const char *e = getenv("HGA_SCAN_TMA"); v = e && atoi(e) != 0 ? 1 : 0; }
-    return v != 0;
-}
-
 // what a scan reads back at its synchronisation: the scalars and, for a device entry, the flags of scan_input_check_kernel
 struct ScanReadback {
     ScanScalars sc;
@@ -728,17 +659,11 @@ struct ScanReadback {
 };
 
 typedef void (*scan_kernel_t)(const ScanParams);
-scan_kernel_t scan_kernel(bool packed) {
-    if (packed) return scan_probe_kernel<4, false, true>;          // the experiment switches apply to ASCII input only
-    if (scan_tma_variant()) return scan_probe_kernel<4, true>;
-    if (scan_occ_variant() == 3) return scan_probe_kernel<3, false>;
-    if (scan_occ_variant() == 5) return scan_probe_kernel<5, false>;
-    return scan_probe_kernel<4, false>;
-}
-size_t scan_smem_bytes(bool packed) { return SCAN_WARPS * sizeof(WarpTile) + (!packed && scan_tma_variant() ? (size_t) SCAN_WARPS * SCAN_STAGE_BYTES : 0); }
+scan_kernel_t scan_kernel(bool packed) { return packed ? scan_probe_kernel<true> : scan_probe_kernel<false>; }
+constexpr size_t SCAN_SMEM_BYTES = SCAN_WARPS * sizeof(WarpTile);
 
 int launch_scan(hga_handle *h, const ScanParams &p, int grid, bool packed) {
-    scan_kernel(packed)<<<grid, SCAN_THREADS, scan_smem_bytes(packed), h->stream>>>(p);
+    scan_kernel(packed)<<<grid, SCAN_THREADS, SCAN_SMEM_BYTES, h->stream>>>(p);
     HGA_CUDA(cudaGetLastError());
     h->metrics.kernel_launches++;
     return HGA_OK;
@@ -779,7 +704,6 @@ int hga_scan_run(hga_handle *h, const char *d_bases, const uint64_t *d_read_off,
     p.tile_dir = h->d_tile_dir.as<uint2>();
     p.tile_tmp_off = tile_tmp_off; p.tile_cnt = tile_cnt;
     p.scalars = d_sc;
-    if (const char *e = getenv("HGA_SCAN_DIAG")) p.diag = atoi(e);
     unsigned long long *exc_dir = nullptr;
     if (n_exc) {                                                                   // run directory: n_tiles entries
         HGA_TRY(h->d_exc_dir.ensure((n_tiles + 1) * 8));
@@ -788,8 +712,8 @@ int hga_scan_run(hga_handle *h, const char *d_bases, const uint64_t *d_read_off,
     }
 
     int occ = 0;
-    HGA_CUDA(cudaFuncSetAttribute(scan_kernel(pk), cudaFuncAttributeMaxDynamicSharedMemorySize, (int) scan_smem_bytes(pk)));
-    HGA_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, scan_kernel(pk), SCAN_THREADS, scan_smem_bytes(pk)));
+    HGA_CUDA(cudaFuncSetAttribute(scan_kernel(pk), cudaFuncAttributeMaxDynamicSharedMemorySize, (int) SCAN_SMEM_BYTES));
+    HGA_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, scan_kernel(pk), SCAN_THREADS, SCAN_SMEM_BYTES));
     if (occ < 1) occ = 1;
     const int grid_full = (int) std::min<uint64_t>((uint64_t) h->sm_count * occ, std::max<uint64_t>((n_tiles + SCAN_WARPS - 1) / SCAN_WARPS, 1));
 

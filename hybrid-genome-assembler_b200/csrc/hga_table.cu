@@ -26,7 +26,7 @@ __global__ void table_bucket_kernel(const uint64_t *__restrict__ kmers, uint64_t
         if (key == HGA_EMPTY_KEY) { atomicOr(flags, 2); bucket_of[i] = t.n_buckets; continue; }   // never a canonical k-mer
         const uint32_t hb = hga_bits_hash(key, t.geom);
         const uint32_t B = hga_locality_from_min(hga_minimizer(key, hb, t.geom));
-        atomicOr(&t.filter[(size_t) hga_scale(B, t.n_blocks) * 8 + hga_bits_word(hb)], hga_bits_mask(hb, t.filter_k));
+        atomicOr(&t.filter[(size_t) hga_scale(B, t.n_blocks) * 8 + hga_bits_word(hb)], hga_bits_mask(hb));
         bucket_of[i] = hga_scale(B, t.n_buckets);
     }
 }
@@ -50,9 +50,7 @@ __global__ void table_place_kernel(const uint64_t *__restrict__ kmers, const uin
         for (uint32_t p = boff[b]; p < boff[b + 1]; p++) {
             const uint32_t i = sorted_idx[p];
             const unsigned long long key = kmers[i];
-            const uint32_t hb = hga_bits_hash(key, t.geom);
-            const uint32_t B = t.sector_by_min ? hga_locality_from_min(hga_minimizer(key, hb, t.geom)) : 0u;
-            const uint32_t start = hga_start_sector(B, hb, t.sector_by_min) * HGA_SECTOR_SLOTS;
+            const uint32_t start = hga_start_sector(hga_bits_hash(key, t.geom)) * HGA_SECTOR_SLOTS;
             bool done = false;
             for (uint32_t j = 0; j < HGA_BUCKET_SLOTS && !done; j++) {
                 const uint32_t slot = home + ((start + j) & (HGA_BUCKET_SLOTS - 1));
@@ -87,10 +85,10 @@ __global__ void table_slot_kid_kernel(const uint32_t *__restrict__ kid_slot, uin
 int hga_table_build(hga_handle *h, const uint64_t *host_kmers) {
     const uint64_t n = h->n_kmers;
     if (n >= (1ull << 29)) { hga_set_error("too many k-mers (%llu): the slot id space is 32 bit", (unsigned long long) n); return HGA_E_ARG; }
-    // filter: sized to stay L2 resident (<= 48 MB, see hga_internal.cuh); HGA_FILTER_* / HGA_TABLE_LOAD are experiment switches
-    double bits_per_key = 16.0, max_mb = 48.0, load = 0.25;
-    if (const char *e = getenv("HGA_FILTER_BITS_PER_KEY")) bits_per_key = atof(e);
-    if (const char *e = getenv("HGA_FILTER_MAX_MB")) max_mb = atof(e);
+    // filter: 16 bits per key, at most 48 MB so that it stays L2 resident (see hga_internal.cuh). HGA_TABLE_LOAD sets the key table's load
+    // factor (0.25) so that tests can fill buckets and reach the overflow region with small sets
+    const double bits_per_key = 16.0, max_mb = 48.0;
+    double load = 0.25;
     if (const char *e = getenv("HGA_TABLE_LOAD")) load = std::min(0.9, std::max(0.05, atof(e)));
     uint64_t n_blocks = (uint64_t) (n * bits_per_key / 256.0) + 64;
     const uint64_t max_blocks = (uint64_t) (max_mb * 1024 * 1024 / 32);
@@ -102,8 +100,6 @@ int hga_table_build(hga_handle *h, const uint64_t *host_kmers) {
     t.n_main = t.n_buckets * HGA_BUCKET_SLOTS;
     t.n_over = 0;
     t.n_blocks = (uint32_t) n_blocks;
-    if (const char *e = getenv("HGA_SECTOR_BY_MIN")) t.sector_by_min = atoi(e) != 0;
-    if (const char *e = getenv("HGA_FILTER_K")) t.filter_k = atoi(e) == 2 ? 2 : 3;
     HGA_TRY(h->d_keys.ensure((size_t) t.n_main * 8));
     HGA_TRY(h->d_kid_slot.ensure((size_t) (n + 1) * 4));
     HGA_TRY(h->d_filter.ensure((size_t) n_blocks * 32));

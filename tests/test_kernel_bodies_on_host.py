@@ -656,8 +656,8 @@ extern "C" int emu_table(int k, const uint64_t *kmers, uint64_t n, double load, 
         if (s >= t.n_slots || t.keys[s] != key || t.slot_kid[s] != (uint32_t) i) { bad |= 1; continue; }
         const uint32_t hb = hga_bits_hash(key, t.geom);
         const uint32_t B = hga_locality_from_min(hga_minimizer(key, hb, t.geom));
-        if ((t.filter[(size_t) hga_scale(B, t.n_blocks) * 8 + hga_bits_word(hb)] & hga_bits_mask(hb, t.filter_k)) != hga_bits_mask(hb, t.filter_k)) bad |= 2;
-        const uint32_t home = hga_scale(B, t.n_buckets) * HGA_BUCKET_SLOTS, start_sec = hga_start_sector(B, hb, t.sector_by_min);
+        if ((t.filter[(size_t) hga_scale(B, t.n_blocks) * 8 + hga_bits_word(hb)] & hga_bits_mask(hb)) != hga_bits_mask(hb)) bad |= 2;
+        const uint32_t home = hga_scale(B, t.n_buckets) * HGA_BUCKET_SLOTS, start_sec = hga_start_sector(hb);
         const uint32_t n_sec = HGA_BUCKET_SLOTS / HGA_SECTOR_SLOTS;
         if (s < t.n_main) {
             in_main++;
@@ -713,7 +713,7 @@ static inline unsigned atomicAdd(unsigned *p, unsigned v) { unsigned o = *p; *p 
 
 
 @pytest.mark.parametrize("k,load", [(19, 0.0), (19, 0.9), (15, 0.9), (31, 0.9), (8, 0.0)])
-def test_table_layout_invariants_on_host(host_table, k, load):
+def test_table_layout_and_filter_invariants_on_host(host_table, k, load):
     """load 0.9 (HGA_TABLE_LOAD) fills buckets, so that start sectors wrap round, sectors fill up and keys spill into the overflow region"""
     g1 = datagen.random_genome(60000, 600 + k)
     g2 = datagen.mutate(g1, 0.03, 700 + k)
